@@ -3,6 +3,7 @@
     python bench.py --gpus N --steps K --warmup W                  # our sm_100a path (one rank per GPU)
     python bench.py --config {c2,c3,c4,c5} ...                     # another BASELINE configuration as the main line
     python bench.py --impl reference --steps K --warmup W          # the reference algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's latents to DIR/*.npy
 
 A "step" is one whole trajectory over one batch of synthetic latents.  BASELINE.json configs:
 
@@ -83,6 +84,27 @@ def workload_config(cfg, n_gpus, global_batch, dtype):
         "nfe": nfe_of(cfg), "compute_dtype": dtype, "parallelism": f"batch-shard x{n_gpus} + final all-gather",
         "l2": "256 MiB memset between steps (inside the timed region)",
     }
+
+
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` to out_dir/<name>.npy in float32, within DUMP_MAX_BYTES in all (headers included), so
+    that two builds can be compared output for output.  A tensor over its share of the budget keeps a fixed, seeded sample
+    of its rows (dim 0), in ascending order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_MAX_BYTES // len(arrays) - 4096                  # room for the .npy header
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        if 4 * t.numel() > share:
+            n_rows = share // (4 * t[0].numel())
+            if n_rows == 0:
+                raise ValueError(f"{name}: one row of {tuple(t.shape)} exceeds the {share}-byte dump share")
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:n_rows]
+            t = t[rows.sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.contiguous().numpy())
 
 
 def seeded_state_dict(n_classes):
@@ -331,16 +353,19 @@ def run_gpu_arm(args):
             torch.cuda.synchronize()
 
     step_ms = {}
+    kept = {}                            # keep=True: what the region's last timed step returned (--dump-outputs)
 
-    def timed(fn, steps, tag):
+    def timed(fn, steps, tag, keep=False):
         barrier()
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
         ev[0].record()
         for i in range(steps):
             if not os.environ.get("FLO_BENCH_NOFLUSH"):
                 flush.zero_()
-            fn()
+            out = fn()
             ev[i + 1].record()
+        if keep:
+            kept[tag] = out
         barrier()
         step_ms[tag] = [round(ev[i].elapsed_time(ev[i + 1]), 3) for i in range(steps)]
         ms = torch.tensor([ev[0].elapsed_time(ev[steps])], device=dev)
@@ -360,10 +385,13 @@ def run_gpu_arm(args):
     torch.cuda.synchronize()
     clocks.samples.clear(); clocks.reasons.clear()
     l0 = eng.launch_count()
-    ms = timed(main.step_resident, args.steps, "resident")
+    ms = timed(main.step_resident, args.steps, "resident", keep=bool(args.dump_outputs))
     launches = eng.launch_count() - l0
     clk = clocks.stop() if rank == 0 else {}
     value = main.global_batch * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"latents": kept["resident"]})
+    kept.clear()
 
     for _ in range(2):
         flush.zero_()
@@ -605,7 +633,14 @@ def main():
     ap.add_argument("--no-other", action="store_true", help="skip the other_configs sub-records")
     ap.add_argument("--cfg", type=float, default=0.0,
                     help="class-conditional sampling with this classifier-free-guidance strength (weak RK4 configs: 2 evaluations per stage)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents the last timed step returned to DIR/latents.npy (float32; a seeded row sample "
+                         "above 64 MB); the inputs are seeded, so runs with the same arguments see the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU arm's latents; the reference arm times partial trajectories")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,8 +1,8 @@
 """Freeze outputs of the UNMODIFIED reference into ``tests/golden/*.pt``.
 
-TEST INFRASTRUCTURE ONLY.  Run in the build container (needs ``/root/reference``):
+TEST INFRASTRUCTURE ONLY.  Needs a checkout of the unmodified reference:
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden      # the checkout at oracle/_ref, or FLOCODER_REFERENCE=/path/to/flocoder
 
 For each of the three U-Nets the BASELINE configs name (n_classes = 102 flowers_sd,
 0 midi_vqgan, 10 stl_sd; SURVEY.md section 8) it seeds torch with 1234, builds the

@@ -1,9 +1,11 @@
-"""Import the UNMODIFIED reference (``/root/reference``) in the build container.
+"""Import the UNMODIFIED reference: a drscotthawley/flocoder checkout named by ``FLOCODER_REFERENCE``, else one
+placed (git-ignored) at ``oracle/_ref``.
 
-TEST INFRASTRUCTURE ONLY.  ``/root/reference`` does not exist on the GPU box, so
-nothing that runs there (``-m gpu`` tests, ``smoke()``, ``bench.py``) may call
-this; it is used to (a) prove the restatement in ``oracle/`` equal to the real
-thing and (b) generate the frozen vectors under ``tests/golden/``.
+TEST INFRASTRUCTURE ONLY.  The reference is not part of this repository, so
+nothing that must run from the repository alone (``-m gpu`` tests, ``smoke()``,
+``bench.py``) may call this; it is used to (a) prove the restatement in
+``oracle/`` equal to the real thing and (b) generate the frozen vectors under
+``tests/golden/``.  Without a checkout the tests that import it skip.
 
 The reference's ``flocoder.sampling`` imports plotting/metrics/codec packages at
 module level that are not installed here (SURVEY.md section 8c).  They carry no
@@ -17,7 +19,7 @@ import sys
 import types
 import warnings
 
-REFERENCE_ROOT = os.environ.get("FLOCODER_REFERENCE", "/root/reference")
+REFERENCE_ROOT = os.environ.get("FLOCODER_REFERENCE") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:
@@ -41,7 +43,7 @@ def _stub(name: str, **attrs):
 def load():
     """Returns (flocoder.unet, flocoder.sampling) of the reference checkout."""
     if not available():
-        raise RuntimeError(f"reference checkout not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference checkout not found at {REFERENCE_ROOT} (set FLOCODER_REFERENCE or place one at oracle/_ref)")
     _stub("omegaconf", OmegaConf=object)
     _stub("matplotlib")
     _stub("matplotlib.pyplot")

@@ -1,6 +1,6 @@
 """The CPU oracle pinned against the reference: (1) frozen outputs of the unmodified reference
-(tests/golden, made by oracle/make_golden.py) and (2), where /root/reference exists, the imported
-reference itself on fresh inputs, fp32 and fp64."""
+(tests/golden, made by oracle/make_golden.py) and (2), where a reference checkout exists (oracle/_ref or FLOCODER_REFERENCE), the
+imported reference itself on fresh inputs, fp32 and fp64."""
 import pytest
 import torch
 
@@ -97,7 +97,7 @@ def test_bf16_matched_policy_is_close_but_not_equal():
     assert 1e-4 < e < 2e-2, e      # SURVEY 8c: ~5e-3 per forward for bf16 GEMM operands
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not ref_shim.available(), reason="needs a flocoder reference checkout (oracle/_ref or FLOCODER_REFERENCE)")
 @pytest.mark.parametrize("n_classes", [102, 0])
 def test_restatement_equals_imported_reference(n_classes):
     ref_unet, ref_sampling = ref_shim.load()
@@ -122,7 +122,7 @@ def test_restatement_equals_imported_reference(n_classes):
     assert nfe == nfe_ref and rel_l2(x1, x1_ref) < 2e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not ref_shim.available(), reason="needs a flocoder reference checkout (oracle/_ref or FLOCODER_REFERENCE)")
 def test_generic_dims_equal_reference():
     """A non-default shape (dim=32, 3 levels, 8 groups, 3 channels) to pin the wiring, not just one config."""
     ref_unet, _ = ref_shim.load()

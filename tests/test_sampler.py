@@ -1,5 +1,5 @@
 """sampler() / decode_latents() / g2rgb() (SURVEY.md section 8(f) N1): host logic checked on CPU with a toy velocity
-model and a toy codec; against the unmodified reference's sampler when /root/reference is present."""
+model and a toy codec; against the unmodified reference's sampler where a checkout exists (oracle/_ref or FLOCODER_REFERENCE)."""
 import pytest
 import torch
 from torch import nn
@@ -84,7 +84,7 @@ def test_sampler_semantics():
     assert torch.allclose(lat2, ref2, atol=1e-6) and nfe2 == 28        # n_steps -> int(10 * (1 - 0.3)) = 7 (sampling.py:106)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="needs /root/reference (golden-generation container only)")
+@pytest.mark.skipif(not ref_shim.available(), reason="needs a flocoder reference checkout (oracle/_ref or FLOCODER_REFERENCE)")
 def test_sampler_matches_unmodified_reference():
     _, ref_sampling = ref_shim.load()
     torch.manual_seed(2)

@@ -891,7 +891,7 @@ static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
         ce = cudaGraphInstantiate(&pl->graph, g, 0);
         cudaGraphDestroy(g);
         if (ce != cudaSuccess) { set_error("graph instantiate failed: %s", cudaGetErrorString(ce)); destroy_plan(*pl); return FLO_ERR_CUDA; }
-        if (s.fused && !getenv("FLO_NO_GRAPH4")) {     // the stage kernels find their ODE stage in the device-side control block
+        if (s.fused) {     // the stage kernels find their ODE stage in the device-side control block
             g = nullptr;
             CUDA_TRY(cudaStreamBeginCapture(h.capture_stream, cudaStreamCaptureModeThreadLocal));
             for (int k = 0; k < 4 && rc == FLO_OK; ++k)

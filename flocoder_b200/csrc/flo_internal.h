@@ -264,17 +264,11 @@ struct ChainParams {
     int zero_off, zero_bytes;               // shared-memory range to clear at start (epilogue-written slots)
     int ones_off;                           // 4 KB constant A tile [1,0,...] that multiplies the bias slice
     int fast;                               // 1: the stage runs the warp-shuffle GroupNorm variant of k_chain (one sample per CTA, one
-                                            // accumulator chunk per thread in every step); FLO_NO_FAST_GN=1 forces the generic variant
+                                            // accumulator chunk per thread in every step)
     int max_c;                              // largest per-step channel count (sizes gpar and the tables of the warp-shuffle GroupNorm path)
     int g_max, coef_n, cpar_n;              // stats region layout: rowstat[rows*g_max] | coef[coef_n] (float2) | cpar[cpar_n] (float) |
                                             // gpar[C] (float2)
-    int prod_lanes;                         // lanes of the producer warp that issue weight chunks (chunk cc -> lane cc % prod_lanes)
     int wide;                               // 1: the grid leaves at most one CTA per SM: launch the instance without the register cap
-    int no_fast2;                           // 1: N-split stages keep the generic row-statistics GroupNorm epilogue (FLO_NO_FAST2=1)
-    int tx_handoff;                         // N-split stages: 1 = the step hand-off rides on the output stores themselves (st.async +
-                                            // mbarrier transaction bytes); 0 = stores, proxy fence, CTA barrier, release-arrive on every CTA
-    int early_pdl;                          // 1: griddepcontrol.launch_dependents at kernel start (this grid leaves SMs idle: the next
-                                            // stage's CTAs become resident there and run their prologue / weight prefetch meanwhile)
     int ring_off, ring_slot_bytes, n_ring, n_ring_deep;   // n_ring_deep: depth when one CTA owns the SM (chosen per plan)
     int stats_off, bar_off, smem_bytes, tmem_cols;
     int tab_off, tab_n;                     // per-K16-slice A operand start addresses (>>4), built at kernel start
@@ -296,15 +290,13 @@ struct ChainParams {
 // linear-attention block  Residual(PreNorm(dim, LinearAttention(dim)))  (unet.py:33-39,125-161) and the
 // mid-block full attention (unet.py:99-122), one kernel, `nb` samples per CTA
 struct AttnFusedParams {
-    int epi_warps;                          // 4, or 8 when a sample spans two M tiles (one tile per warp group)
-    int early_pdl;                          // 1: launch_dependents at kernel start (see ChainParams)
+    int epi_warps;                          // 4 for mid attention; linear attention: 8 for one M tile, 16 for two (a sample spans two tiles)
     int B, H, W, C, nb, n, n_pad, n_mtiles; // n = H*W; n_pad = max(n,16) rows per sample in the P/V/Q slots;
                                             // n_mtiles = 128-row tiles of the dense rows (s*n + p)
     int full;                               // 1: softmax(QK^T)V mid attention (no GroupNorm after to_out)
     int ktrans;                             // 1: K and V are projected TRANSPOSED (weights as the A operand, the CTA's pixels as N): tensor-
                                             // memory lanes = channels, columns = pixels, so the softmax over pixels is a loop per thread
     int small;                              // 1: k_attn_small (n = 4 or 16 pixels: 128 / n samples per CTA, attention core on CUDA cores)
-    int hc, hsplit;                         // heads per CTA (4, or 2 with the head split) and CTAs per sample (cluster size 1 / 2)
     int fmt;
     unsigned wq_off, wk_off, wv_off, wo_off; // 16-bit weight streams in wblob (N = 128,128,128,C)
     int qkv_chunks, qkv_S, o_chunks, o_S;   // ring chunking of those streams
@@ -323,7 +315,6 @@ struct AttnFusedParams {
 
 cudaError_t fused_configure();
 int fused_max_active_clusters(int nsplit, int smem_bytes);
-void fused_set_pdl(bool on);     // programmatic dependent launch between the fused stage kernels (default on; FLO_NO_PDL=1 disables)
 cudaError_t launch_chain(const ChainParams& p, const CUtensorMap* maps, int grid, cudaStream_t s);
 cudaError_t launch_attn_fused(const AttnFusedParams& p, const CUtensorMap& xh_map, int grid, cudaStream_t s);
 

@@ -179,7 +179,6 @@ template <int N> struct IntTag { static constexpr int value = N; };
 // `gpar[c]` = (gamma, beta); with `has_film`, coef[s*C+c] holds (1+scale, shift) on entry.
 struct XChg {                    // cross-CTA (cluster) reduction of per-sample statistics; nsplit == 1: unused
     int nsplit; uint32_t rank, smem_base, bar_x; int xpart_off; uint32_t* phase; uint8_t* smem;
-    bool tx;                     // the partial sums travel as st.async stores that complete transaction bytes on bar_x
 };
 __device__ __forceinline__ void stats_to_coef(const Geo& g, int R, const float2* rowstat, float2* coef, const float2* gpar, int G, int pm,
                                               int C, int HW, bool has_film, int et, const XChg* xc = nullptr) {
@@ -220,22 +219,12 @@ __device__ __forceinline__ void stats_to_coef(const Geo& g, int R, const float2*
         // G == 1 here: every CTA of the cluster holds the sums over ITS channels; publish them to all CTAs, then
         // add the parts in rank order (deterministic, identical in every CTA)
         n_parts = xc->nsplit;
-        if (xc->tx) {
-            // every CTA receives nsplit x nb (sum, sumsq) pairs of 8 bytes; one thread posts the expectation, the stores signal
-            if (et == 0) mbar_expect_tx(xc->bar_x, (uint32_t)(n_parts * g.nb * 8));
-            if (active && li == 0)
-                for (int q = 0; q < n_parts; ++q)
-                    st_async_f2(mapa_shared(xc->smem_base + (uint32_t)xc->xpart_off + (uint32_t)((int)xc->rank * g.nb + s) * 8u, (uint32_t)q),
-                                make_float2(sx, sq), mapa_shared(xc->bar_x, (uint32_t)q));
-        } else {
-            if (active && li == 0)
-                for (int q = 0; q < n_parts; ++q)
-                    st_cluster_f2(mapa_shared(xc->smem_base + (uint32_t)xc->xpart_off + (uint32_t)((int)xc->rank * g.nb + s) * 8u, (uint32_t)q),
-                                  make_float2(sx, sq));
-            epi_sync();                      // the publishing lanes' remote stores are ordered before the release-arrives below
-            if (et == 0)
-                for (int q = 0; q < n_parts; ++q) mbar_arrive_cluster(mapa_shared(xc->bar_x, (uint32_t)q));
-        }
+        // every CTA receives nsplit x nb (sum, sumsq) pairs of 8 bytes; one thread posts the expectation, the stores signal
+        if (et == 0) mbar_expect_tx(xc->bar_x, (uint32_t)(n_parts * g.nb * 8));
+        if (active && li == 0)
+            for (int q = 0; q < n_parts; ++q)
+                st_async_f2(mapa_shared(xc->smem_base + (uint32_t)xc->xpart_off + (uint32_t)((int)xc->rank * g.nb + s) * 8u, (uint32_t)q),
+                            make_float2(sx, sq), mapa_shared(xc->bar_x, (uint32_t)q));
         mbar_wait_cluster(xc->bar_x, *xc->phase & 1u);
         ++*xc->phase;
         if (active) {
@@ -320,8 +309,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
     const uint32_t bar_epi = bar_mma + 8;
     const uint32_t tmem_slot = bar_epi + 8;
     const uint32_t bar_x = tmem_slot + 8;
-    const uint32_t bar_epi2 = bar_x + 8;         // transaction hand-off: steps alternate between bar_epi and bar_epi2
-    const bool txh = SPLIT && (ENDS == 0 ? true : p.tx_handoff != 0);      // (the lean N-split instance is only launched with it)
+    const uint32_t bar_epi2 = bar_x + 8;         // N-split step hand-off: steps alternate between bar_epi and bar_epi2
     volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem + bar_off + 16 * MAX_WSTAGES + 24);
     const Geo geo = make_geo(p);
     // N-split: the Q CTAs of a cluster own the same samples and 1/Q of every step's output channels
@@ -334,18 +322,15 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
     const int ones_off = p.ones_off;
     long long* dbg = (blockIdx.x == 0) ? p.dbg : nullptr;
     if (p.dbg && tid == 0 && blockIdx.x == 0) p.dbg[100] = global_ns();
-    // a grid that leaves SMs idle lets the next stage become resident at once: its prologue, TMEM allocation and weight
-    // prefetch run beside this kernel instead of after its last epilogue (every read of our output is behind its griddep_wait)
-    if (p.early_pdl) griddep_launch();
 
     if (warp == W_PROD && lane == 0) {
         for (int i = 0; i < n_ring; ++i) { mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, 1); }
         mbar_init(bar_load, 1);
         mbar_init(bar_mma, 1);
-        // N-split: one elected thread per CTA arrives (after a CTA-local barrier) on the barriers of every CTA of the cluster
-        mbar_init(bar_epi, txh ? 1 : (SPLIT ? Q : EPI_THREADS));
+        // N-split: the stores of every CTA of the cluster complete transaction bytes on these (one arrival: the expectation)
+        mbar_init(bar_epi, SPLIT ? 1 : EPI_THREADS);
         mbar_init(bar_epi2, 1);
-        mbar_init(bar_x, txh ? 1 : (SPLIT ? Q : EPI_THREADS));
+        mbar_init(bar_x, SPLIT ? 1 : EPI_THREADS);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == W_MMA) tmem_alloc(tmem_slot, (uint32_t)tmem_cols);
@@ -390,7 +375,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                 if (cc >= 8) dbg[104 + (cc - 8) * 3] = clock64();
             }
         }
-        const int NL = p.prod_lanes;
+        constexpr int NL = 2;
         if (lane < NL) {
             const uint32_t ring_base = smem_base + p.ring_off, ring_slot_bytes = p.ring_slot_bytes;
             const uint2* wtab = reinterpret_cast<const uint2*>(smem + p.wtab_off);
@@ -437,8 +422,8 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
         for (int i = 0; i < n_steps; ++i) {
             if (i > 0) {
                 // epilogue -> MMA hand-off: inside one CTA a named barrier the 256 epilogue threads arrive on (no 256
-                // serialised mbarrier arrivals); across a cluster the mbarrier with cluster-scope release / acquire
-                if (txh) {
+                // serialised mbarrier arrivals); across a cluster the output stores themselves
+                if (SPLIT) {
                     // every CTA of the cluster stores step i-1's 16-bit outputs into our slot with st.async: the barrier completes when
                     // all of them have landed -- (live rows) x (channel blocks of the step) x 16 bytes; steps alternate between two
                     // barriers, so a peer that is one step ahead signals the other one
@@ -448,8 +433,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                     __syncwarp();
                     mbar_wait_cluster(bar, ((i - 1) >> 1) & 1);
                     fence_proxy_async_all();
-                } else if (Q > 1) { mbar_wait_cluster(bar_epi, (i - 1) & 1); fence_proxy_async_all(); }
-                else named_bar_sync(2, EPI_THREADS + 32);
+                } else {
+                    named_bar_sync(2, EPI_THREADS + 32);
+                }
             }
             tc_fence_after();
             if (dbg && lane == 0) dbg[i * 8 + 0] = clock64();
@@ -504,7 +490,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
         uint32_t xphase = 0;
         XChg xc;
         xc.nsplit = Q; xc.rank = qrank; xc.smem_base = smem_base; xc.bar_x = bar_x; xc.xpart_off = p.xpart_off; xc.phase = &xphase;
-        xc.smem = smem; xc.tx = txh;
+        xc.smem = smem;
 
         for (int i = 0; i < n_steps; ++i) {
             // ---- step parameters into registers
@@ -528,8 +514,6 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                 if (out_slot_off >= 0) {
                     const uint32_t soff = (uint32_t)out_slot_off + (uint32_t)cb * plane_bytes + (uint32_t)R.pp * 16u;
                     if (!SPLIT) *reinterpret_cast<uint4*>(smem + soff) = u;
-                    else if (!txh)
-                        for (int q = 0; q < Q; ++q) st_cluster_v4(mapa_shared(smem_base + soff, (uint32_t)q), u);
                     else if (i + 1 < n_steps) {
                         const uint32_t bar = (i & 1) ? bar_epi2 : bar_epi;
                         for (int q = 0; q < Q; ++q) st_async_v4(mapa_shared(smem_base + soff, (uint32_t)q), u, mapa_shared(bar, (uint32_t)q));
@@ -896,7 +880,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                             const float4 ab = gc[j >> 1];
                             float ya = fmaf(y[j], ab.x, ab.y);
                             float yb = fmaf(y[j + 1], ab.z, ab.w);
-                            ya = fast_silu_t<FMT>(ya); yb = fast_silu_t<FMT>(yb);          // every GroupNorm step of the U-Net is followed by SiLU (unet.py:67)
+                            ya = fast_silu(ya); yb = fast_silu(yb);          // every GroupNorm step of the U-Net is followed by SiLU (unet.py:67)
                             ya += rr[j]; yb += rr[j + 1];
                             y[j] = ya; y[j + 1] = yb;
                             sxa += ya; sqa = fmaf(ya, ya, sqa); sxb += yb; sqb = fmaf(yb, yb, sqb);
@@ -972,11 +956,11 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                 // shared memory, no coefficient table, no second tensor-memory load.
                 bool fast2 = false;
                 if constexpr (SPLIT && MT == 1)
-                    fast2 = G == 1 && geo.PP == 16 && !is_final && (cend - cbeg == 8 || cend - cbeg == 16) && !p.no_fast2;
+                    fast2 = G == 1 && geo.PP == 16 && !is_final && (cend - cbeg == 8 || cend - cbeg == 16);
                 bool fast3 = false;
                 if constexpr (!SPLIT && MT == 1 && WIDE)
                     fast3 = geo.H == 4 && geo.W == 4 && geo.nb <= 3 && !is_final && (cpg == 8 || cpg == 16) && ((cend - cbeg) & 15) == 0 &&
-                            cend > cbeg && !p.no_fast2;
+                            cend > cbeg;
                 if (fast2) {
                     if (dbg && et == 0) dbg[i * 8 + 3] = clock64();
                     auto body = [&](auto cw_tag) {
@@ -1035,7 +1019,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                             a0 *= f.x; b0 = fmaf(b0, f.x, f.y); a1 *= f.z; b1 = fmaf(b1, f.z, f.w);
                             float ya = fmaf(__uint_as_float(av[j]), a0, b0);
                             float yb = fmaf(__uint_as_float(av[j + 1]), a1, b1);
-                            ya = fast_silu_t<FMT>(ya); yb = fast_silu_t<FMT>(yb);
+                            ya = fast_silu(ya); yb = fast_silu(yb);
                             ya += rr[j]; yb += rr[j + 1];
                             v[j] = ya; v[j + 1] = yb;
                             sxa += ya; sqa = fmaf(ya, ya, sqa); sxb += yb; sqb = fmaf(yb, yb, sqb);
@@ -1099,7 +1083,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                             a0 *= f.x; b0 = fmaf(b0, f.x, f.y); a1 *= f.z; b1 = fmaf(b1, f.z, f.w);
                             float ya = fmaf(__uint_as_float(av[j]), a0, b0);
                             float yb = fmaf(__uint_as_float(av[j + 1]), a1, b1);
-                            ya = fast_silu_t<FMT>(ya); yb = fast_silu_t<FMT>(yb);
+                            ya = fast_silu(ya); yb = fast_silu(yb);
                             ya += rr[j]; yb += rr[j + 1];
                             v[j] = ya; v[j + 1] = yb;
                             sxa += ya; sqa = fmaf(ya, ya, sqa); sxb += yb; sqb = fmaf(yb, yb, sqb);
@@ -1189,7 +1173,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
                         const float4 ab = cf[j >> 1];
                         float ya = fmaf(__uint_as_float(av[j]), ab.x, ab.y);
                         float yb = fmaf(__uint_as_float(av[j + 1]), ab.z, ab.w);
-                        ya = fast_silu_t<FMT>(ya); yb = fast_silu_t<FMT>(yb);          // every GroupNorm step of the U-Net is followed by SiLU (unet.py:67)
+                        ya = fast_silu(ya); yb = fast_silu(yb);          // every GroupNorm step of the U-Net is followed by SiLU (unet.py:67)
                         ya += rr[j]; yb += rr[j + 1];
                         v[j] = ya; v[j + 1] = yb;
                         sxa += ya; sqa = fmaf(ya, ya, sqa); sxb += yb; sqb = fmaf(yb, yb, sqb);
@@ -1265,14 +1249,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
             }
             if (dbg && et == 0) dbg[i * 8 + 5] = clock64();
             tc_fence_before();
-            if (SPLIT && txh) {
-                // nothing: the stores of write8 complete the consumers' barriers as they land
-            } else if (SPLIT) {
-                fence_proxy_async_all();     // local and remote shared-memory results -> visible to every CTA's next tcgen05.mma
-                epi_sync();                  // every thread's stores are ordered before the elected thread's release-arrives
-                if (et == 0)
-                    for (int q = 0; q < Q; ++q) mbar_arrive_cluster(mapa_shared(bar_epi, (uint32_t)q));
-            } else {
+            if (!SPLIT) {                 // (N-split: the stores of write8 complete the consumers' barriers as they land)
                 fence_proxy_async();      // shared-memory results -> visible to the next step's tcgen05.mma
                 if (i + 1 < n_steps) named_bar_arrive(2, EPI_THREADS + 32);
             }
@@ -1305,8 +1282,6 @@ cudaError_t fused_configure() {
     if (e == cudaSuccess) e = chain_attr<2, false, false>();
     if (e == cudaSuccess) e = chain_attr<3, false, false>();
     if (e == cudaSuccess) e = chain_attr<4, false, false>();
-    if (e == cudaSuccess) e = chain_attr<1, false, true>();
-    if (e == cudaSuccess) e = chain_attr<2, false, true>();
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain<1, true, 0, false, false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain<1, true, 1, false, false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_chain<1, false, 0, false, true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -1323,19 +1298,15 @@ cudaError_t fused_configure() {
     return attn_configure();
 }
 
-static bool g_pdl = true;
-void fused_set_pdl(bool on) { g_pdl = on; }
 cudaError_t launch_pdl(const void* fn, int grid, int block, size_t smem, cudaStream_t s, void** args, int cluster) {
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = smem; cfg.stream = s;
     cudaLaunchAttribute at[2];
     int n = 0;
-    if (g_pdl) {
-        at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
+    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // programmatic dependent launch between the stage kernels
+    at[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
     if (cluster > 1) {
         at[n].id = cudaLaunchAttributeClusterDimension;
         at[n].val.clusterDim.x = (unsigned)cluster; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
@@ -1363,9 +1334,9 @@ int fused_max_active_clusters(int nsplit, int smem_bytes) {
 }
 
 template <int FMT>
-static const void* chain_fn(int mt, bool split, bool fast, bool wide, int ends, bool txh) {
+static const void* chain_fn(int mt, bool split, bool fast, bool wide, int ends) {
     if (ends == 0 && !fast && mt == 1) {
-        if (split && txh) return (const void*)k_chain<1, true, FMT, false, false, 0>;
+        if (split) return (const void*)k_chain<1, true, FMT, false, false, 0>;
         if (!split && wide) return (const void*)k_chain<1, false, FMT, false, true, 0>;
     }
     if (wide && !fast && !split && mt == 1) return (const void*)k_chain<1, false, FMT, false, true>;
@@ -1374,7 +1345,7 @@ static const void* chain_fn(int mt, bool split, bool fast, bool wide, int ends, 
         if (ends == 0) return mt == 1 ? (const void*)k_chain<1, false, FMT, true, false, 0> : (const void*)k_chain<2, false, FMT, true, false, 0>;
         if (ends == 1) return mt == 1 ? (const void*)k_chain<1, false, FMT, true, false, 1> : (const void*)k_chain<2, false, FMT, true, false, 1>;
         if (ends == 2) return mt == 1 ? (const void*)k_chain<1, false, FMT, true, false, 2> : (const void*)k_chain<2, false, FMT, true, false, 2>;
-        return mt == 1 ? (const void*)k_chain<1, false, FMT, true> : (const void*)k_chain<2, false, FMT, true>;
+        return nullptr;          // no stage holds both the init conv and the final conv (fused_plan.inc)
     }
     switch (mt) {
         case 1: return split ? (const void*)k_chain<1, true, FMT, false> : (const void*)k_chain<1, false, FMT, false>;
@@ -1388,8 +1359,8 @@ cudaError_t launch_chain(const ChainParams& p, const CUtensorMap* maps, int grid
     if (p.nsplit > 1 && p.n_mtiles != 1) return cudaErrorInvalidValue;
     int ends = 0;
     for (int i = 0; i < p.n_steps; ++i) ends |= (p.st[i].epi == CE_INIT ? 1 : 0) | (p.st[i].final != 0 ? 2 : 0);
-    const void* fn = p.fmt ? chain_fn<1>(p.n_mtiles, p.nsplit > 1, p.fast != 0, p.wide != 0, ends, p.tx_handoff != 0)
-                           : chain_fn<0>(p.n_mtiles, p.nsplit > 1, p.fast != 0, p.wide != 0, ends, p.tx_handoff != 0);
+    const void* fn = p.fmt ? chain_fn<1>(p.n_mtiles, p.nsplit > 1, p.fast != 0, p.wide != 0, ends)
+                           : chain_fn<0>(p.n_mtiles, p.nsplit > 1, p.fast != 0, p.wide != 0, ends);
     if (!fn) return cudaErrorInvalidValue;
     void* args[5] = {(void*)&maps[0], (void*)&maps[1], (void*)&maps[2], (void*)&maps[3], (void*)&p};
     return launch_pdl(fn, grid * p.nsplit, FUSED_THREADS, (size_t)p.smem_bytes, s, args, p.nsplit);

@@ -30,13 +30,13 @@ constexpr int ATTN_RING = 4;       // weight ring depth of k_attn (the planner s
 
 // weight chunk g of the stage: K, V, Q projections (qkv_chunks each), then to_out (o_chunks)
 __device__ __forceinline__ void attn_issue_chunk(const AttnFusedParams& p, uint32_t smem_base, uint32_t bar_full, uint32_t bar_empty,
-                                                 int g, int qkv_bytes, int o_bytes, int wo_rank_elems) {
+                                                 int g, int qkv_bytes, int o_bytes) {
     const int qc = p.qkv_chunks;
     const uint16_t* w; int ci, bytes;
     if (g < qc) { w = p.wblob + p.wk_off; ci = g; bytes = qkv_bytes; }
     else if (g < 2 * qc) { w = p.wblob + p.wv_off; ci = g - qc; bytes = qkv_bytes; }
     else if (g < 3 * qc) { w = p.wblob + p.wq_off; ci = g - 2 * qc; bytes = qkv_bytes; }
-    else { w = p.wblob + p.wo_off + wo_rank_elems; ci = g - 3 * qc; bytes = o_bytes; }   // head split: this CTA's K slices of to_out
+    else { w = p.wblob + p.wo_off; ci = g - 3 * qc; bytes = o_bytes; }
     const int slot = g & (ATTN_RING - 1);
     if (g >= ATTN_RING) mbar_wait(bar_empty + 8 * slot, ((g / ATTN_RING) - 1) & 1);
     mbar_expect_tx(bar_full + 8 * slot, (uint32_t)bytes);
@@ -44,11 +44,10 @@ __device__ __forceinline__ void attn_issue_chunk(const AttnFusedParams& p, uint3
                  (uint32_t)bytes, bar_full + 8 * slot);
 }
 // 1x1 conv over a K-major operand slot: A rows = tile t rows [128t, 128t+128), planes at `a_plane` stride.
-// The weight stream holds tiles of `n_tile` output channels per K16 slice; the MMA uses `n` of them starting at byte
-// offset `b_off` inside the tile (head split: a CTA's 64 of the 128 q/k/v channels), so only descriptors change.
+// The weight stream holds tiles of `n_tile` output channels per K16 slice; the MMA uses the first `n` of them.
 __device__ __forceinline__ void attn_conv(const AttnFusedParams& p, uint32_t smem_base, uint32_t tmem_base, uint32_t bar_full,
                                           uint32_t bar_empty, RingA& rs, uint32_t a_off, uint32_t a_plane, int n, int n_tile,
-                                          uint32_t b_off, int col, int n_chunks, int S) {
+                                          int col, int n_chunks, int S) {
     const uint32_t idesc = make_idesc16(128, n, p.fmt, 0, 0);
     const int n_mtiles = p.n_mtiles;
     const uint32_t ring_off = p.ring_off, ring_slot_bytes = p.ring_slot_bytes;
@@ -62,7 +61,7 @@ __device__ __forceinline__ void attn_conv(const AttnFusedParams& p, uint32_t sme
         mbar_wait(bar_full + 8 * slot, (rs.cc / ATTN_RING) & 1);
         tc_fence_after();
         if (elect_one()) {
-            uint32_t b_lo = (((smem_base + ring_off + slot * ring_slot_bytes + b_off) >> 4) & 0x3FFFu) | b_lbo;
+            uint32_t b_lo = (((smem_base + ring_off + slot * ring_slot_bytes) >> 4) & 0x3FFFu) | b_lbo;
             uint32_t a_lo = a_lo0 + (uint32_t)(ci * S) * a_step;
             for (int s = 0; s < S; ++s) {
                 const uint64_t bdesc = desc64(b_lo, hi);
@@ -171,25 +170,26 @@ __device__ __forceinline__ int colmax16(float (&v)[16], int lane) {
     return chan;
 }
 
-// HC: heads per CTA (4; 2 = the head split), a template parameter so that the channel loops keep compile-time bounds
-// LEAN: the instance the default plan launches (linear attention, transposed K / V projections): `full` and `ktrans` are
-// compile-time there, so the mid-attention path, the row-form first epilogue and their helpers are not part of its code
-// (200 KB -> the kernels are latency chains that stall on instruction fetch as much as on memory)
 // NT: M tiles per CTA as a compile-time constant (1: the 8x8 level with 8 epilogue warps, 2: 16x16 with 16; 0: run time)
+// NT > 0 is the LEAN instance the default plan launches (linear attention, transposed K / V projections): `full` and `ktrans` are
+// compile-time there, so the mid-attention path, the row-form first epilogue and their helpers are not part of its code
+// (200 KB -> the kernels are latency chains that stall on instruction fetch as much as on memory).  NT = 0 is the generic
+// instance: full attention, and linear attention with the row-form projections.
 // FMTK: the 16-bit operand format as a compile-time constant (0 fp16, 1 bf16; -1: run time)
-template <int HC, bool LEAN = false, int NT = 0, int FMTK = -1>
+template <int NT = 0, int FMTK = -1>
 __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant__ CUtensorMap tm_xh,
                                                         const __grid_constant__ AttnFusedParams p) {
     extern __shared__ __align__(128) uint8_t smem[];
+    constexpr bool LEAN = NT > 0;
     const int fmt_k = FMTK >= 0 ? FMTK : p.fmt;
     const bool is_full = LEAN ? false : (p.full != 0);
-    const bool is_kt = LEAN ? true : (p.ktrans != 0);
+    const bool is_kt = LEAN;                            // the generic instance is launched only for the row-form projections
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
-    // Warp roles: [0, EW) epilogue (EW = 4, or 8 when a sample spans two M tiles: one tile per warp group, both groups
-    // share the TMEM lane quadrants), EW = TMA producer, EW + 1 = MMA issuer.
+    // Warp roles: [0, EW) epilogue (EW = 4 for mid attention, 8 for one M tile, 16 for two; the warp groups share the TMEM
+    // lane quadrants), EW = TMA producer, EW + 1 = MMA issuer.
     const int EW = NT == 2 ? 16 : (NT == 1 ? 8 : p.epi_warps), n_epi = EW * 32, n_thr = (int)blockDim.x;
     const int n_mtiles_k = NT ? NT : p.n_mtiles;
-    const bool n_ge32 = (LEAN && NT) ? true : (p.n >= 32);
+    const bool n_ge32 = LEAN ? true : (p.n >= 32);
     const int w_prod = EW, w_mma = EW + 1;
     const uint32_t smem_base = smem_u32(smem);
     const uint32_t bar_full = smem_base + p.bar_off;
@@ -199,17 +199,9 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
     const uint32_t bar_epi = bar_mma + 8;
     const uint32_t tmem_slot = bar_epi + 8;
     volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem + p.bar_off + 16 * MAX_WSTAGES + 24);
-    // Head split (p.hsplit == 2, 16x16 level): the two CTAs of a cluster own the same sample and two of the four heads each
-    // (64 of the 128 q/k/v channels): half the shared memory and tensor memory per CTA, so two CTAs share an SM, and every
-    // phase is half as long.  Nothing crosses the CTAs until the to_out projection, whose two K halves are added through
-    // distributed shared memory in the last epilogue (CTA r finalises pixel tile r).
-    constexpr int NCH = HC * 32;
-    const int HS = HC == 4 ? 1 : 2;
-    const uint32_t hrank = HS > 1 ? cluster_ctarank() : 0u;
-    const int b0 = (HS > 1 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x) * p.nb;
-    const uint32_t bar_r = tmem_slot + 8, bar_d = bar_r + 8, bar_s = bar_d + 8;      // head split: one-shot cluster hand-offs
+    constexpr int NCH = 128;                            // q / k / v channels: 4 heads x 32
+    const int b0 = (int)blockIdx.x * p.nb;
     if (p.dbg && tid == 0 && blockIdx.x == 0) p.dbg[100] = global_ns();
-    if (p.early_pdl) griddep_launch();      // see k_chain
     const int n = p.n, n_pad = p.n_pad, C = p.C;
     const uint32_t plane = (uint32_t)p.plane_bytes;
     const uint32_t xh_plane = (uint32_t)(p.nb * n) * 16u;
@@ -221,7 +213,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
         mbar_init(bar_load, 1);
         mbar_init(bar_mma, 1);
         mbar_init(bar_epi, n_epi);
-        mbar_init(bar_r, 1); mbar_init(bar_d, 4); mbar_init(bar_s, 8);     // head split (see the last epilogue)
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == w_mma) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
@@ -229,14 +220,13 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
     // end of the batch, rows past the last sample of a partly filled M tile.  A CTA whose rows are all live skips the clear
     // (152 KB of shared-memory stores at the 16x16 level, on the critical path of every CTA that is not in the first wave):
     // every contraction runs over the rows of ONE sample, and what the unwritten planes feed are accumulator columns nobody loads.
-    const bool all_live = !is_full && HS == 1 && p.n_pad == p.n && ((p.nb * p.n) & 127) == 0 && b0 + p.nb <= p.B;
+    const bool all_live = !is_full && p.n_pad == p.n && ((p.nb * p.n) & 127) == 0 && b0 + p.nb <= p.B;
     if (!all_live)
         for (int i = tid * 16; i < p.zero_bytes; i += n_thr * 16)
             *reinterpret_cast<uint4*>(smem + p.zero_off + i) = make_uint4(0, 0, 0, 0);
     fence_proxy_async();
     tc_fence_before();
-    if (HS > 1) cluster_sync_all();          // the peer's barriers are initialised before any remote arrive
-    else __syncthreads();
+    __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot_ptr;
     long long* dbg = (blockIdx.x == 0) ? p.dbg : nullptr;
@@ -247,12 +237,11 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
     if (warp == w_prod) {
         if (lane == 0) {
             const int total = 3 * p.qkv_chunks + p.o_chunks, pre = min(ATTN_RING, total);
-            const int wo_rank = (int)hrank * (NCH / 16) * C * 16;          // elements: this CTA's K16 slices of the to_out stream
-            for (int g = 0; g < pre; ++g) attn_issue_chunk(p, smem_base, bar_full, bar_empty, g, qkv_bytes, o_bytes, wo_rank);
+            for (int g = 0; g < pre; ++g) attn_issue_chunk(p, smem_base, bar_full, bar_empty, g, qkv_bytes, o_bytes);
             griddep_wait();          // weights are constants; the activations come from the previous kernel
             mbar_expect_tx(bar_load, (uint32_t)(C >> 3) * xh_plane);
             tma_load_5d(smem_base + p.xh_off, &tm_xh, bar_load, 0, 0, 0, b0, 0);
-            for (int g = pre; g < total; ++g) attn_issue_chunk(p, smem_base, bar_full, bar_empty, g, qkv_bytes, o_bytes, wo_rank);
+            for (int g = pre; g < total; ++g) attn_issue_chunk(p, smem_base, bar_full, bar_empty, g, qkv_bytes, o_bytes);
         }
     } else if (warp == w_mma) {
         {   // whole warp, warp-uniform; one elected lane issues the tcgen05 instructions
@@ -261,7 +250,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
             tc_fence_after();
             if (dbg && lane == 0) dbg[0] = clock64();
             // ---- phase 0: K and V convolutions (and Q for the mid attention)
-            const uint32_t wb_off = hrank * (uint32_t)NCH * 16u;      // this CTA's channels inside every 128-channel weight tile
             const bool tr = is_kt != 0;
             // transposed projection D[channel lanes][pixel columns] = W (A operand: the K-major weight tile, 128 rows x 16 B per K half)
             // x x^ (B operand: the CTA's nb * n pixel rows of the input tile, planes of 8 channels)
@@ -288,10 +276,10 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
                 conv_T(p.col_k);
                 conv_T(p.col_v);
             } else {
-            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, wb_off, p.col_k, p.qkv_chunks, p.qkv_S);
-            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, wb_off, p.col_v, p.qkv_chunks, p.qkv_S);
+            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, p.col_k, p.qkv_chunks, p.qkv_S);
+            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, p.col_v, p.qkv_chunks, p.qkv_S);
             }
-            if (is_full) attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, wb_off, p.col_q, p.qkv_chunks, p.qkv_S);
+            if (is_full) attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, p.col_q, p.qkv_chunks, p.qkv_S);
             if (dbg && lane == 0) dbg[1] = clock64();
             if (elect_one()) umma_commit(bar_mma);
             __syncwarp();
@@ -301,8 +289,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
                 named_bar_sync(2, n_epi + 32); ++ph;
                 tc_fence_after();
                 if (dbg && lane == 0) dbg[8] = clock64();
-                // M = 128 channel rows are always read (with two heads per CTA rows 64..127 are whatever follows the P slot:
-                // their accumulator lanes are never loaded), N = this CTA's (h, e) channels + the ones block
+                // M = the 128 (h, d) channel rows, N = the 128 (h, e) channels + the ones block
                 const uint32_t idesc_ctx = make_idesc16(128, NCH + 16, fmt_k, 1, 1);
                 {
                     const int nb = p.nb, col_ctx = p.col_ctx;
@@ -327,7 +314,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
                             }
                     __syncwarp();
                 }
-                attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, wb_off, p.col_q, p.qkv_chunks, p.qkv_S);
+                attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, p.xh_off, xh_plane, NCH, 128, p.col_q, p.qkv_chunks, p.qkv_S);
                 if (dbg && lane == 0) dbg[9] = clock64();
                 if (elect_one()) umma_commit(bar_mma);
                 __syncwarp();
@@ -342,11 +329,11 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
                     if (elect_one()) {
                         for (int s = 0; s < nb; ++s)
                             for (int t = 0; t < mtS; ++t)
-                                for (int h = 0; h < HC; ++h)
+                                for (int h = 0; h < 4; ++h)
                                     for (int k = 0; k < 2; ++k) {
                                         const uint32_t a_addr = smem_base + p_off + (uint32_t)(4 * h + 2 * k) * plane +
                                                                 (uint32_t)(s * n_pad + t * 128) * 16u;
-                                        const uint32_t b_addr = smem_base + ct_off + (uint32_t)(s * HC + h) * 2048u + (uint32_t)k * 1024u;
+                                        const uint32_t b_addr = smem_base + ct_off + (uint32_t)(s * 4 + h) * 2048u + (uint32_t)k * 1024u;
                                         umma_bf16(tmem_base + (uint32_t)(col_out + (s * mtS + t) * NCH + h * 32),
                                                   make_smem_desc(a_addr, plane, 128u), make_smem_desc(b_addr, 512u, 128u), idesc_out,
                                                   k > 0 ? 1u : 0u);
@@ -360,7 +347,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
             named_bar_sync(2, n_epi + 32); ++ph;
             tc_fence_after();
             if (dbg && lane == 0) dbg[24] = clock64();
-            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, is_full ? p.p_off : p.v_off, plane, C, C, 0u, p.col_proj,
+            attn_conv(p, smem_base, tmem_base, bar_full, bar_empty, rs, is_full ? p.p_off : p.v_off, plane, C, C, p.col_proj,
                       p.o_chunks, p.o_S);
             if (elect_one()) umma_commit(bar_mma);
             __syncwarp();
@@ -369,15 +356,14 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
         const int quad = warp & 3, grp = warp >> 2;            // TMEM lane quadrant; which warp group
         const int r = quad * 32 + lane;                        // row inside an M tile == TMEM lane
         const int et = grp * 128 + r;                          // epilogue thread index
-        // EW = 4: one warp group does everything; EW = 8: M tiles / samples are dealt round-robin to two warp groups; EW = 16 (a
-        // sample spans two M tiles): tile = grp & 1 and the two groups of a tile split the q/k/v channels (cpart = grp >> 1) --
-        // the softmax epilogues are chains of TMEM loads, shuffles and MUFU ops, and four warps per scheduler hide what two cannot
-        // One M tile per CTA (8x8 level, two samples) with EW = 8: both groups work on tile 0 and split the channels the same way
+        // EW = 4 (mid attention): one warp group does everything; EW = 16 (a sample spans two M tiles): tile = grp & 1 and the two
+        // groups of a tile split the q/k/v channels (cpart = grp >> 1) -- the softmax epilogues are chains of TMEM loads, shuffles
+        // and MUFU ops, and four warps per scheduler hide what two cannot
+        // EW = 8 (one M tile per CTA, 8x8 level, two samples): both groups work on tile 0 and split the channels the same way
         // (four warps per SM left every scheduler idle most of the time: 6 k-cycle softmax epilogues on 16 k exponentials).
-        const bool one_tile_split = EW == 8 && n_mtiles_k == 1;
-        const int half = (EW >= 8 && !one_tile_split) ? (grp & 1) : 0;
-        const int t0 = half, tstep = (EW >= 8 && !one_tile_split) ? 2 : 1;
-        const int cpart = EW == 16 ? (grp >> 1) : (one_tile_split ? grp : 0), ncp = (EW == 16 || one_tile_split) ? 2 : 1;
+        const int half = EW == 16 ? (grp & 1) : 0;
+        const int t0 = half, tstep = EW == 16 ? 2 : 1;
+        const int cpart = EW == 16 ? (grp >> 1) : (EW == 8 ? grp : 0), ncp = EW >= 8 ? 2 : 1;
         const int ch_lo = cpart * (NCH / ncp), ch_hi = ch_lo + NCH / ncp;      // this thread's q/k/v channels in the softmax epilogues
         const uint32_t tlane = tmem_base + ((uint32_t)(quad * 32) << 16);
         auto esync = [&]() { named_bar_sync(1, n_epi); };
@@ -561,7 +547,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
             {
                 const int h = quad, d = lane;                // TMEM row r = (h, d)
                 for (int s = t0; s < p.nb; s += tstep) {
-                    if (h >= HC) break;                      // head split: rows 64..127 of the context accumulator are not ours (warp-uniform)
                     uint32_t u0[16], u1[16], us[16];
                     // (with two channel groups per tile each takes 16 of the row's 32 context columns)
                     tmem_ld16_issue(tlane + (uint32_t)(p.col_ctx + s * (NCH + 16) + h * 32), u0);
@@ -573,7 +558,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
 #pragma unroll
                     for (int j = 0; j < 16; ++j) { c0[j] = __uint_as_float(u0[j]); c1[j] = __uint_as_float(u1[j]); }
                     const float inv = 0.17677669529663687f * fast_rcp(__uint_as_float(us[0]));      // 32^-0.5 / sum_n exp(k - max)
-                    uint8_t* base = smem + p.ct_off + (uint32_t)(s * HC + h) * 2048u + (uint32_t)(d >> 3) * 512u + (uint32_t)(d & 7) * 2u;
+                    uint8_t* base = smem + p.ct_off + (uint32_t)(s * 4 + h) * 2048u + (uint32_t)(d >> 3) * 512u + (uint32_t)(d & 7) * 2u;
 #pragma unroll
                     for (int e = 0; e < 32; ++e) {
                         if (e < e_lo || e >= e_hi) continue;
@@ -589,7 +574,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
                 const uint32_t row_off = (uint32_t)(s * n_pad + px) * 16u;
                 // two heads per iteration (four TMEM loads in flight, two independent softmax chains); max and sum as
                 // 4-way trees instead of 32-long dependent chains
-                for (int h2 = cpart * (HC / ncp); h2 < (cpart + 1) * (HC / ncp); h2 += 2) {
+                for (int h2 = cpart * (4 / ncp); h2 < (cpart + 1) * (4 / ncp); h2 += 2) {
                     uint32_t qu[2][32];
 #pragma unroll
                     for (int k = 0; k < 2; ++k) {
@@ -629,7 +614,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
             if (dbg && r == 0) dbg[18] = clock64();
             for (int s = 0; s < p.nb; ++s)
                 for (int t = (mtS > 1 ? t0 : 0); t < mtS; t += (mtS > 1 ? tstep : 1)) {
-                    if (mtS == 1 && half != (s & (tstep - 1))) continue;      // one-tile samples: round-robin over the warp groups
                     const int px = t * 128 + r;
                     const bool valid = px < n && b0 + s < p.B;
                     const uint32_t row_off = (uint32_t)(s * n + px) * 16u;
@@ -650,9 +634,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
             fence_proxy_async();
             tc_fence_before();
             named_bar_arrive(2, n_epi + 32);
-            // head split: the out MMAs (the last readers of this CTA's P slot) completed before this epilogue began, so the peer
-            // may use it as its exchange buffer from here on: tell it now, long before it asks
-            if (HS > 1 && et == 0) mbar_arrive_cluster(mapa_shared(bar_r, hrank ^ 1u));
         } else {
             // ================= mid attention: softmax(q k^T) v on CUDA cores (unet.py:99-122) =================
             // A CTA owns nb = 32/n samples = 32 rows (TMEM lane quadrant 0).  Warp 0 moves K, V (16-bit) and Q (fp32)
@@ -757,7 +738,7 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
         // the residual rows of this thread's first tile are requested BEFORE waiting for the to_out MMAs: their L2 round trip
         // (~800 cycles) otherwise sits on the critical path between the statistics barrier and the stores
         uint4 pre_xa = make_uint4(0, 0, 0, 0), pre_xb = pre_xa;
-        if (!is_full && HS == 1 && t0 < n_mtiles_k && cpart == 0) {
+        if (!is_full && t0 < n_mtiles_k && cpart == 0) {
             const int rd = t0 * 128 + r, s = rd >> lgn, px = rd & (n - 1);
             if (s < p.nb && b0 + s < p.B) {
                 const uint4* xsrc = reinterpret_cast<const uint4*>(p.x2);
@@ -770,100 +751,6 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
         if (dbg && r == 0) dbg[26] = clock64();
         griddep_launch();            // PDL: the next stage kernel may become resident during the last epilogue
         const float* bias = par;
-        if (HS > 1) {
-            // ================= head split: add the two K halves of the to_out projection across the CTA pair =================
-            // Warp group g holds pixel tile g of this CTA's partial projection; CTA r finalises tile r.  Three one-shot
-            // cluster-scope mbarriers, all arrived on per WARP (lane 0 after __syncwarp; no CTA-wide barrier on this path):
-            //   bar_r (1 arrival, sent by the peer at the end of ITS epilogue 2): the peer's P slot is dead, so the exchange
-            //          buffer that aliases it may be written;
-            //   bar_d (4 arrivals: the peer's four sending warps): the partial rows have been delivered;
-            //   bar_s (8 arrivals: four finalising warps of each CTA): the GroupNorm partial sums have been delivered.
-            const int t = half;                           // this warp group's pixel tile (EW == 8, two M tiles)
-            const bool mine = (uint32_t)t == hrank;
-            const uint32_t peer = hrank ^ 1u;
-            float* xbuf = reinterpret_cast<float*>(smem + p.p_off);           // [128 rows][C] fp32, written by the peer
-            float2* xstat = stat + 64;                                        // [2 CTAs][4 warps] (sum, sumsq) of the finalised tiles
-            const int rd = t * 128 + r, px = rd & (n - 1);
-            if (!mine) {
-                mbar_wait_cluster(bar_r, 0);
-                const uint32_t dst0 = mapa_shared(smem_base + p.p_off + (uint32_t)r * (uint32_t)C * 4u, peer);
-                for (int c16 = 0; c16 < C; c16 += 16) {
-                    float v[16];
-                    tmem_ld16(tlane + (uint32_t)(p.col_proj + t * C + c16), v);
-#pragma unroll
-                    for (int k4 = 0; k4 < 4; ++k4)
-                        st_cluster_v4(dst0 + (uint32_t)(c16 + 4 * k4) * 4u,
-                                      make_uint4(__float_as_uint(v[4 * k4]), __float_as_uint(v[4 * k4 + 1]), __float_as_uint(v[4 * k4 + 2]),
-                                                 __float_as_uint(v[4 * k4 + 3])));
-                }
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(mapa_shared(bar_d, peer));
-            } else {
-                // the residual rows of this tile are requested before the wait (an exposed L2 round trip otherwise)
-                const uint4* xsrc = reinterpret_cast<const uint4*>(p.x2);
-                uint4 xres[8];
-#pragma unroll
-                for (int cb = 0; cb < 8; ++cb)
-                    xres[cb] = cb < (C >> 3) ? xsrc[(size_t)(cb * p.B + b0) * n + px] : make_uint4(0, 0, 0, 0);
-                mbar_wait_cluster(bar_d, 0);
-                float sx = 0.f, sq = 0.f;
-                for (int c16 = 0; c16 < C; c16 += 16) {
-                    float v[16];
-                    tmem_ld16(tlane + (uint32_t)(p.col_proj + t * C + c16), v);
-                    const float4* xb = reinterpret_cast<const float4*>(xbuf + r * C + c16);
-#pragma unroll
-                    for (int k4 = 0; k4 < 4; ++k4) {
-                        const float4 o = xb[k4];
-                        const float oo[4] = {o.x, o.y, o.z, o.w};
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const int j = 4 * k4 + e;
-                            // fixed order: (heads 0,1) + (heads 2,3)
-                            const float x = (hrank == 0 ? v[j] + oo[e] : oo[e] + v[j]) + bias[c16 + j];
-                            sx += x; sq = fmaf(x, x, sq);
-                        }
-                    }
-                }
-                for (int o = 16; o > 0; o >>= 1) { sx += __shfl_xor_sync(0xffffffffu, sx, o); sq += __shfl_xor_sync(0xffffffffu, sq, o); }
-                if (lane == 0) {
-                    const uint32_t off = (uint32_t)((uint8_t*)(xstat + hrank * 4 + quad) - smem);
-                    st_cluster_f2(mapa_shared(smem_base + off, 0u), make_float2(sx, sq));
-                    st_cluster_f2(mapa_shared(smem_base + off, 1u), make_float2(sx, sq));
-                    mbar_arrive_cluster(mapa_shared(bar_s, 0u));
-                    mbar_arrive_cluster(mapa_shared(bar_s, 1u));
-                }
-                mbar_wait_cluster(bar_s, 0);
-                float tx = 0.f, tq = 0.f;
-#pragma unroll
-                for (int k = 0; k < 8; ++k) { tx += xstat[k].x; tq += xstat[k].y; }          // fixed order, identical in both CTAs
-                const float icnt = fast_rcp((float)(C * n));
-                const float mean = tx * icnt;
-                const float rstd = rsqrtf(fmaxf(tq * icnt - mean * mean, 0.f) + 1e-5f);
-                const float* gamma = par + 128;
-                const float* beta = par + 256;
-                for (int c16 = 0; c16 < C; c16 += 16) {
-                    float v[16], x2[16];
-                    tmem_ld16(tlane + (uint32_t)(p.col_proj + t * C + c16), v);
-                    const float4* xb = reinterpret_cast<const float4*>(xbuf + r * C + c16);
-#pragma unroll
-                    for (int cb = 0; cb < 8; ++cb)
-                        if (cb == (c16 >> 3)) { unpack8(xres[cb], x2, fmt_k); unpack8(xres[cb + (cb < 7 ? 1 : 0)], x2 + 8, fmt_k); }
-#pragma unroll
-                    for (int k4 = 0; k4 < 4; ++k4) {
-                        const float4 o = xb[k4];
-                        const float oo[4] = {o.x, o.y, o.z, o.w};
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const int j = 4 * k4 + e;
-                            const float a = hrank == 0 ? v[j] + oo[e] : oo[e] + v[j];
-                            const float y = (a + bias[c16 + j] - mean) * rstd * gamma[c16 + j] + beta[c16 + j];
-                            v[j] = y + x2[j];
-                        }
-                    }
-                    attn_write_out(p, b0, px, c16, v, fmt_k);
-                }
-            }
-        } else {
         if (!is_full) {
             // (the C output channels are not split: with 16 epilogue warps the second channel group only keeps the barriers)
             for (int t = t0; t < n_mtiles_k && cpart == 0; t += tstep) {
@@ -1007,10 +894,8 @@ __global__ void __launch_bounds__(ATTN_MAX_THREADS) k_attn(const __grid_constant
         }
         if (dbg && et == 0) dbg[29] = clock64();
     }
-    }
     tc_fence_before();
     __syncthreads();
-    if (HS > 1) cluster_sync_all();          // no CTA of the pair may exit while the other can still store into its shared memory
     if (dbg && tid == 0) dbg[65] = clock64();
     if (p.dbg && tid == 0) { if (blockIdx.x == 0) p.dbg[102] = global_ns(); atomicMax(reinterpret_cast<unsigned long long*>(p.dbg + 103), (unsigned long long)global_ns()); }
     if (warp == w_mma) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
@@ -1091,7 +976,6 @@ __global__ void __launch_bounds__(SMALL_THREADS, 1) k_attn_small(const __grid_co
     const int live_rows = p.nb * NPX;
     long long* dbg = (blockIdx.x == 0) ? p.dbg : nullptr;
     if (dbg && tid == 0) dbg[100] = global_ns();
-    if (p.early_pdl) griddep_launch();                 // see k_chain
     if (warp == w_prod && lane == 0) {
         for (int i = 0; i < p.n_ring; ++i) { mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, 1); }
         mbar_init(bar_load, 1);
@@ -1552,13 +1436,11 @@ __global__ void __launch_bounds__(SMALL_THREADS, 1) k_attn_small(const __grid_co
 }
 
 cudaError_t attn_configure() {
-    cudaError_t e = cudaFuncSetAttribute(k_attn<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<4, true, 1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<4, true, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<4, true, 2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<4, true, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(k_attn<>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn_small<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn_small<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_attn_small<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -1581,12 +1463,13 @@ cudaError_t launch_attn_fused(const AttnFusedParams& p, const CUtensorMap& xh_ma
                                              : (qt ? (const void*)k_attn_small<4, true, true> : (const void*)k_attn_small<4, true>));
         return launch_pdl(fn, grid, SMALL_THREADS, (size_t)p.smem_bytes, s, args, 1);
     }
-    const void* fn = p.hc == 2 ? (const void*)k_attn<2> : ((p.ktrans && !p.full) ? (const void*)k_attn<4, true> : (const void*)k_attn<4>);
-    if (p.hc == 4 && p.ktrans && !p.full && p.n >= 64) {
-        if (p.n_mtiles == 2 && p.epi_warps == 16) fn = p.fmt ? (const void*)k_attn<4, true, 2, 1> : (const void*)k_attn<4, true, 2, 0>;
-        if (p.n_mtiles == 1 && p.epi_warps == 8) fn = p.fmt ? (const void*)k_attn<4, true, 1, 1> : (const void*)k_attn<4, true, 1, 0>;
-    }
-    return launch_pdl(fn, grid * p.hsplit, (p.epi_warps + 2) * 32, (size_t)p.smem_bytes, s, args, p.hsplit);
+    // transposed K / V projections (linear attention): the planner sets them only for one M tile with 8 epilogue warps or two
+    // with 16, the two LEAN instances
+    const void* fn = (const void*)k_attn<>;
+    if (p.ktrans && !p.full)
+        fn = p.n_mtiles == 2 ? (p.fmt ? (const void*)k_attn<2, 1> : (const void*)k_attn<2, 0>)
+                             : (p.fmt ? (const void*)k_attn<1, 1> : (const void*)k_attn<1, 0>);
+    return launch_pdl(fn, grid, (p.epi_warps + 2) * 32, (size_t)p.smem_bytes, s, args, 1);
 }
 
 }  // namespace flo

@@ -77,28 +77,6 @@ __device__ __forceinline__ float fast_rcp(float x) {
     float r; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r;
 }
 // SiLU (unet.py:67 nn.SiLU): y * sigmoid(y)
-#ifdef FLO_SILU_TANH
-// one MUFU instead of two: sigmoid(y) = 0.5 + 0.5 tanh(y/2)
-__device__ __forceinline__ float fast_silu(float y) {
-    float t; asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * y));
-    return y * fmaf(0.5f, t, 0.5f);
-}
-#else
 __device__ __forceinline__ float fast_silu(float y) { return y * fast_rcp(1.0f + fast_exp(-y)); }
-#endif
-
-// Format-aware SiLU of the fused epilogues: bf16 results are rounded to 8 mantissa bits right afterwards, so the
-// one-MUFU form  y * (0.5 + 0.5 tanh(y/2))  (tanh.approx: 2^-11) is below the rounding; fp16 keeps ex2 + rcp.
-template <int FMT>
-__device__ __forceinline__ float fast_silu_t(float y) {
-#ifdef FLO_SILU_TANH_BF16
-    if constexpr (FMT != 0) {
-        float t; asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * y));
-        const float h = 0.5f * y;
-        return fmaf(h, t, h);
-    }
-#endif
-    return y * fast_rcp(1.0f + fast_exp(-y));
-}
 
 }  // namespace flo

@@ -163,9 +163,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile
 __device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
     uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank)); return r;
 }
-__device__ __forceinline__ void st_cluster_v4(uint32_t raddr, uint4 v) {
-    asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(raddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
 // 16-byte store into the shared memory of a CTA of the cluster that, when it lands, completes 16 transaction bytes on an mbarrier
 // of the SAME CTA: data and signal travel together (no fence + release-arrive round trip behind the stores)
 __device__ __forceinline__ void st_async_v4(uint32_t raddr, uint4 v, uint32_t rbar) {
@@ -178,13 +175,7 @@ __device__ __forceinline__ void st_async_f2(uint32_t raddr, float2 v, uint32_t r
                  "r"(__float_as_uint(v.x)), "r"(__float_as_uint(v.y)), "r"(rbar)
                  : "memory");
 }
-__device__ __forceinline__ void st_cluster_f2(uint32_t raddr, float2 v) {
-    asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(raddr), "f"(v.x), "f"(v.y) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t raddr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-// wait with cluster-scope acquire: the phase is completed by arrivals from other CTAs of the cluster whose
+// wait with cluster-scope acquire: the phase is completed by the st.async stores of other CTAs of the cluster, whose
 // distributed-shared-memory writes must be visible afterwards
 __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;

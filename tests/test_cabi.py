@@ -121,3 +121,24 @@ def test_fused_plan_decisions_round2():
     assert "nb=2 " in by_name["downs.2.2"] and "ctas=128" in by_name["downs.2.2"]      # 4x4: 32 live rows per CTA
     assert "nb=8 " in by_name["downs.3.2"] and "ctas=32" in by_name["downs.3.2"]       # 2x2
     assert "nb=8 " in by_name["mid_attn"] and "full=1" in by_name["mid_attn"]
+
+
+def test_environment_switches_are_the_ones_the_tests_use():
+    """The library reads a FLO_* environment variable only to force a path that the planner also selects from the input, so that
+    a test can compare the two on one input (FLO_TIMELINE: the clock64 instrumentation behind tools/gpu_timeline.py).  A losing
+    A/B alternative goes together with its switch; a new switch comes with a test that uses it."""
+    csrc = os.path.join(ROOT, "flocoder_b200", "csrc")
+    read = set()
+    for name in os.listdir(csrc):
+        with open(os.path.join(csrc, name)) as f:
+            read |= set(re.findall(r'getenv\("(FLO_\w+)"\)', f.read()))
+    kept = {"FLO_SMALL_DIV", "FLO_ATTN_NO_KTRANS", "FLO_CFG_TWO_PASS", "FLO_GN_NO_TMA", "FLO_GN_CTA", "FLO_TIMELINE"}
+    assert read == kept
+    tests = os.path.join(ROOT, "tests")
+    text = ""
+    for name in os.listdir(tests):
+        if name.endswith(".py") and name != os.path.basename(__file__):
+            with open(os.path.join(tests, name)) as f:
+                text += f.read()
+    for switch in sorted(kept - {"FLO_TIMELINE"}):
+        assert switch in text, f"{switch} is read by the library, but no test uses it"

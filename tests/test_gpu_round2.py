@@ -368,9 +368,8 @@ def test_three_channel_latents_midi_vqgan_3d_gray(compute_dtype, tol):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# the small-batch plan (quarter-filled k_attn_small tiles with four threads per (row, head); st.async hand-off of the N-split
-# stages; transposed K / V projections in k_attn) against the full-tile / fence-and-arrive / row forms of the same kernels:
-# the arithmetic is the same in the same order
+# the small-batch plan (quarter-filled k_attn_small tiles with four threads per (row, head); transposed K / V projections in
+# k_attn) against the full-tile / row forms of the same kernels: the arithmetic is the same in the same order
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("B", [37, 256])
 def test_plan_switches_are_bit_identical(B, monkeypatch):
@@ -395,5 +394,22 @@ def test_plan_switches_are_bit_identical(B, monkeypatch):
     assert torch.isfinite(base).all()
     assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "1"}))        # full k_attn_small tiles, one thread per (row, head)
     assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "2"}))        # half tiles
-    assert torch.equal(base, forward_with({"FLO_TX_HANDOFF": "0"}))       # stores -> fence -> barrier -> release-arrive hand-off
     assert torch.equal(base, forward_with({"FLO_ATTN_NO_KTRANS": "1"}))   # K / V projected with pixels as lanes (shuffle softmax)
+
+
+def test_generic_attention_instance_on_16x8_latents():
+    """16x8 latents with dim_mults=[1, 2, 4]: linear attention at 8x4 (n = 32, row-form projections) and the full mid attention at
+    4x2 (n = 8) run the generic k_attn instance, which the default 16x16 configs never launch.  fp16 against the fp32 CUDA path on
+    the same weights."""
+    from flocoder_b200.unet import Unet
+    torch.manual_seed(7)
+    m32 = Unet(dim=16, channels=4, dim_mults=[1, 2, 4], n_classes=0, compute_dtype="fp32").cuda().eval()
+    m16 = Unet(dim=16, channels=4, dim_mults=[1, 2, 4], n_classes=0, compute_dtype="fp16").cuda().eval()
+    m16.load_state_dict(m32.state_dict())
+    gen = torch.Generator().manual_seed(8)
+    x = torch.randn(5, 4, 16, 8, generator=gen).cuda()
+    t = (torch.rand(5, generator=gen) * 999).cuda()
+    with torch.no_grad():
+        v32, v16 = m32(x, t), m16(x, t)
+    assert torch.isfinite(v16).all()
+    assert rel_l2(v16, v32) <= 3e-3

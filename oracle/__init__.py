@@ -12,7 +12,7 @@ build container by ``oracle/ref_shim.py`` and frozen into ``tests/golden/`` by
 ``oracle/make_golden.py``.
 """
 from .unet_oracle import (UnetSpec, Precision, unet_forward, FP32, BF16_MATCHED, FUSED_BF16,  # noqa: F401
-                          FUSED_FP16)
+                          FUSED_FP16, trained_like)
 from .sampling_oracle import (  # noqa: F401
     warp_time, rk4_step, v_func_cfg, generate_latents_rk4, generate_latents, euler_sampler,
     rk4_stage_times,

@@ -86,6 +86,34 @@ FUSED_BF16 = Precision("fused_bf16", gemm_operands_bf16=True, stream_16=True)
 FUSED_FP16 = Precision("fused_fp16", gemm_operands_bf16=True, stream_16=True, dtype16=torch.float16)
 
 
+def trained_like(sd: Dict[str, Tensor], seed: int = 3, qkv_scale: float = 4.0) -> Dict[str, Tensor]:
+    """New weights with statistics a trained checkpoint has and default init lacks.  Not a model of any real checkpoint.
+
+    Default init leaves every GroupNorm at gamma = 1, beta = 0, so a kernel that drops beta or reads gamma at the wrong
+    channel computes the same numbers, and it gives q / k logits with a standard deviation of ~0.5, so the softmaxes are
+    nearly uniform and pairing values with the wrong pixel barely moves the output.  Here:
+
+    * every GroupNorm affine (``*.norm`` and the linear attention's ``*.to_out.1``) gets gamma = 1 + 0.3 N(0, 1) and
+      beta = 0.3 N(0, 1), per channel;
+    * every ``*.to_qkv.weight`` is multiplied by ``qkv_scale`` (x4 puts the logit std at ~2: sharp softmaxes);
+    * every other tensor is returned unchanged (as a copy).
+
+    Deterministic in ``seed``: values are drawn in fp32 in sorted key order and cast to each tensor's dtype, so an fp32
+    state dict and its fp64 copy give the same weights."""
+    gen = torch.Generator().manual_seed(seed)
+    out = {}
+    for k in sorted(sd):
+        v = sd[k]
+        affine = k.endswith((".norm.weight", ".norm.bias", ".to_out.1.weight", ".to_out.1.bias"))
+        if affine:
+            z = 0.3 * torch.randn(v.shape, generator=gen, dtype=torch.float32)
+            v = (1 + z if k.endswith(".weight") else z).to(dtype=v.dtype, device=v.device)
+        elif k.endswith(".to_qkv.weight"):
+            v = v * qkv_scale
+        out[k] = v.detach().clone()
+    return {k: out[k] for k in sd}
+
+
 def key_usable(d, key) -> bool:
     """general.py:18-20."""
     return (d is not None) and isinstance(d, dict) and (d.get(key) is not None)

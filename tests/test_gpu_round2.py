@@ -373,13 +373,17 @@ def test_three_channel_latents_midi_vqgan_3d_gray(compute_dtype, tol):
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("B", [37, 256])
 def test_plan_switches_are_bit_identical(B, monkeypatch):
+    """With default-init weights and with oracle.trained_like ones, whose sharp softmaxes make a value paired with the wrong key
+    visible."""
     from flocoder_b200.unet import Unet
+    from oracle.unet_oracle import trained_like
 
-    def forward_with(env):
+    def forward_with(env, sd):
         for k, v in env.items():
             monkeypatch.setenv(k, v)
-        torch.manual_seed(1234)
-        m = Unet(dim=16, channels=4, dim_mults=[1, 2, 4, 8], n_classes=10, compute_dtype="bf16").cuda().eval()   # a fresh engine reads the switches
+        m = Unet(dim=16, channels=4, dim_mults=[1, 2, 4, 8], n_classes=10, compute_dtype="bf16")
+        m.load_state_dict(sd)
+        m = m.cuda().eval()                                                 # a fresh engine reads the switches
         x = torch.randn(B, 4, 16, 16, generator=torch.Generator().manual_seed(7)).cuda()
         t = torch.linspace(10.0, 900.0, B).cuda()
         cls = (torch.arange(B) % 10).cuda()
@@ -390,11 +394,14 @@ def test_plan_switches_are_bit_identical(B, monkeypatch):
             monkeypatch.delenv(k)
         return v
 
-    base = forward_with({})
-    assert torch.isfinite(base).all()
-    assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "1"}))        # full k_attn_small tiles, one thread per (row, head)
-    assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "2"}))        # half tiles
-    assert torch.equal(base, forward_with({"FLO_ATTN_NO_KTRANS": "1"}))   # K / V projected with pixels as lanes (shuffle softmax)
+    torch.manual_seed(1234)
+    sd0 = {k: v.detach().clone() for k, v in Unet(dim=16, channels=4, dim_mults=[1, 2, 4, 8], n_classes=10).state_dict().items()}
+    for sd in (sd0, trained_like(sd0)):
+        base = forward_with({}, sd)
+        assert torch.isfinite(base).all()
+        assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "1"}, sd))        # full k_attn_small tiles, one thread per (row, head)
+        assert torch.equal(base, forward_with({"FLO_SMALL_DIV": "2"}, sd))        # half tiles
+        assert torch.equal(base, forward_with({"FLO_ATTN_NO_KTRANS": "1"}, sd))   # K / V projected with pixels as lanes (shuffle softmax)
 
 
 def test_generic_attention_instance_on_16x8_latents():

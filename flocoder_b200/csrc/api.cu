@@ -631,6 +631,34 @@ struct Builder {
     }
 };
 
+// ---- kernels of the layer-by-layer program ----------------------------------------------------
+// launch_op runs each op with one kernel, chosen from the op's shape alone: refuse at plan time an op no kernel can run, so
+// that a forward never starts on it.  The fused path runs its own stage kernels; its planner (fused_plan.inc) checks them.
+static int check_op_kernels(const Handle& h) {
+    const Spec& s = h.spec;
+    if (s.fused) return FLO_OK;
+    const char* path = s.bf16 ? "the layer-wise 16-bit path" : "the fp32 path";
+    for (const Op& op : h.ops) {
+        if (op.kind == OP_GN && gn_variant(op.C, op.H, op.W, op.groups, s.bf16) == GN_NONE) {
+            set_error("GroupNorm '%s' (C=%d, %dx%d, groups=%d) has no kernel on %s: its 16-bit kernels need W, H*W and the "
+                      "groups (or channel-block pairs of 4-channel groups) per sample to be powers of two, and at most 8192 "
+                      "elements per group", op.name.c_str(), op.C, op.H, op.W, op.groups, path);
+            return FLO_ERR_UNSUPPORTED;
+        }
+        if (op.kind == OP_MIDATTN && !midattn_supported(op.n)) {
+            set_error("mid attention '%s' at %dx%d (n=%d) has no kernel on %s: it holds at most 64 pixels", op.name.c_str(), op.H,
+                      op.W, op.n, path);
+            return FLO_ERR_UNSUPPORTED;
+        }
+        if (op.kind == OP_LINATTN && !linattn_supported(op.n, s.bf16)) {
+            set_error("linear attention '%s' at %dx%d (n=%d) has no kernel on %s: more than 256 pixels need fp32 and a multiple "
+                      "of 256", op.name.c_str(), op.H, op.W, op.n, path);
+            return FLO_ERR_UNSUPPORTED;
+        }
+    }
+    return FLO_OK;
+}
+
 // ---- activation arena: linear-scan allocation over buffer live ranges ---------------------------
 static void allocate_arena(Handle& h) {
     const bool reuse = !(h.spec.flags & FLO_FLAG_NO_BUFFER_REUSE);
@@ -1036,14 +1064,8 @@ int flo_unet_create(flo_unet_t** out, const flo_unet_cfg* cfg, const void* const
     Builder b(*h);
     rc = b.build();
     if (rc) return rc;
-    // the layer-wise GroupNorm kernel (fp32 path, FLO_FLAG_LAYERWISE) keeps one (sample, group) unit in the registers of a CTA
-    if (!h->spec.fused && h->spec.bf16)
-        for (const Op& op : h->ops)
-            if (op.kind == OP_GN && (op.C / op.groups) * op.H * op.W > 8192) {
-                set_error("GroupNorm '%s' normalises %d elements per (sample, group); the layer-wise path holds at most 8192 "
-                          "(use a 16-bit compute_dtype for this dim / latent size)", op.name.c_str(), (op.C / op.groups) * op.H * op.W);
-                return FLO_ERR_UNSUPPORTED;
-            }
+    rc = check_op_kernels(*h);
+    if (rc) return rc;
     allocate_arena(*h);
     if (h->spec.fused) {
         FusedBuilder fb(*h, h->ftensors, h->fstages, 4);
@@ -1380,6 +1402,8 @@ int flo_describe_plan(const flo_unet_cfg* cfg, int B, char* out, int cap) {
     Builder b(h);
     rc = b.build();
     if (rc) return rc;
+    rc = check_op_kernels(h);
+    if (rc) return rc;
     allocate_arena(h);
     std::string t;
     char line[512];
@@ -1409,10 +1433,13 @@ int flo_describe_plan(const flo_unet_cfg* cfg, int B, char* out, int cap) {
             }
             t += "\n";
         } else if (op.kind == OP_GN) {
-            snprintf(line, sizeof(line), "%3zu gn      %-28s C=%d %dx%d groups=%d film=%d silu=%d in=%s res=%s out_m=%s out_o=%s un=%s up=%s\n", i,
+            snprintf(line, sizeof(line), "%3zu gn      %-28s C=%d %dx%d groups=%d film=%d silu=%d in=%s res=%s out_m=%s out_o=%s un=%s up=%s", i,
                      op.name.c_str(), op.C, op.H, op.W, op.groups, op.film_off, op.silu, bn(op.gn_in), bn(op.res), bn(op.out_m),
                      bn(op.out_o), bn(op.out_un), bn(op.out_up));
             t += line;
+            // the kernel launch_gn runs; the fused stage kernels normalise in their own epilogues and never launch it
+            if (!h.spec.fused) t += std::string(" gn=") + gn_variant_name(gn_variant(op.C, op.H, op.W, op.groups, h.spec.bf16));
+            t += "\n";
         } else if (op.kind == OP_LINATTN || op.kind == OP_MIDATTN) {
             snprintf(line, sizeof(line), "%3zu %-7s %-28s n=%d qkv=%s out=%s\n", i, kinds[op.kind], op.name.c_str(), op.n, bn(op.qkv),
                      bn(op.attn_out));

@@ -191,6 +191,14 @@ cudaError_t launch_temb(const TembParams& p, cudaStream_t s);
 cudaError_t launch_final(const FinalParams& p, cudaStream_t s);
 cudaError_t launch_mask_prep(const MaskPrepParams& p, cudaStream_t s);   // p.mask == null: *mode = 0 only
 cudaError_t launch_gn_any(const GnParams& p, cudaStream_t s);            // any channels-per-group (fp32 path)
+
+// Host-side kernel choices of the layer-by-layer program: the launchers above follow them, and the planner refuses an op
+// they give no kernel for before anything is launched.
+enum GnVariant { GN_TMA, GN_WARP, GN_CTA, GN_ANY, GN_NONE };
+GnVariant gn_variant(int C, int H, int W, int groups, bool bf16);       // the GroupNorm kernel launch_gn runs
+const char* gn_variant_name(GnVariant v);                               // "tma", "warp", "cta", "any", "none"
+bool linattn_supported(int n, bool bf16);                               // launch_linattn has a kernel for n pixels
+bool midattn_supported(int n);                                          // launch_midattn has a kernel for n pixels
 cudaError_t launch_conv_umma(const ConvUmmaParams& p, const CUtensorMap& a0, const CUtensorMap& a1,
                              cudaStream_t s);
 cudaError_t conv_umma_configure();   // one-time cudaFuncSetAttribute calls

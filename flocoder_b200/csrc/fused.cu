@@ -77,7 +77,7 @@ struct RingPos {               // ring slot and mbarrier phase, advanced without
     __device__ __forceinline__ void next(int n_ring) { if (++slot == n_ring) { slot = 0; phase ^= 1u; } }
 };
 struct ConvIssue {
-    const int32_t* tab;        // per-slice A start address (>>4, tile row offset not included); entries [0, slices)
+    const int32_t* tab;        // per-slice A start address (>>4, tap shift + Wp + 1; IssueCtx::row0 adds the tile's rest)
     int n, col, slices, S;
 };
 template <int MT>
@@ -417,7 +417,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, (MT <= 2 && !SPLIT && !WIDE) ? 
         x.desc_hi_ones = (128u >> 4) | (1u << 14);
         x.n_ring = n_ring; x.cc = 0; x.rp.slot = 0; x.rp.phase = 0; x.dbg = dbg;
 #pragma unroll
-        for (int t = 0; t < MT; ++t) x.row0[t] = (uint32_t)tile_row0(geo, t);
+        for (int t = 0; t < MT; ++t) x.row0[t] = (uint32_t)(tile_row0(geo, t) - (geo.Wp + 1));   // atab holds tile 0's Wp + 1
         if (n_loads > 0) mbar_wait(bar_load, 0);
         for (int i = 0; i < n_steps; ++i) {
             if (i > 0) {

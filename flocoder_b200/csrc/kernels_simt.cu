@@ -229,7 +229,7 @@ template <typename TO>
 __global__ void __launch_bounds__(256) k_gn(GnParams p) {
     __shared__ float red[32];
     const int G = p.groups, cpg = p.C / G, HW = p.H * p.W;
-    // H, W, groups are powers of two on every supported shape (checked at plan time): shifts, not integer divisions
+    // shifts, not integer divisions: gn_variant picks this kernel only when W, H*W and groups are powers of two
     const int lgG = 31 - __clz(G), lgW = 31 - __clz(p.W), lgPC = 31 - __clz(HW * 2);
     const int b = blockIdx.x >> lgG, g = blockIdx.x & (G - 1);
     const int nvec = cpg * HW / 4;
@@ -683,32 +683,65 @@ static void launch_gn_warp(const GnParams& p, int nvec, int pair, cudaStream_t s
         default: k_gn_warp<TO, 32><<<grid, GNW_THREADS, 0, s>>>(p, T, pair, n_units); break;
     }
 }
-cudaError_t launch_gn(const GnParams& p, cudaStream_t s) {
-    const int cpg = p.C / p.groups, HW = p.H * p.W;
-    if (cpg != 4 && (cpg & 7)) return launch_gn_any(p, s);
-    const int pair = cpg == 4 ? 1 : 0;
+static bool is_pow2(int x) { return x > 0 && (x & (x - 1)) == 0; }
+constexpr int GN_CTA_THREADS = 256;
+// k_gn_tma, k_gn_warp and k_gn locate pixels, channel blocks and samples with shifts and masks: each runs only where W, H*W
+// and its units per sample are powers of two.  A unit is one (sample, group), or for 4-channel groups (pair) the two groups
+// that share a channel block in k_gn_tma / k_gn_warp; k_gn always takes one group.  The order tma > warp > cta is the
+// fastest first; FLO_GN_NO_TMA skips k_gn_tma and FLO_GN_CTA both, so that tests can compare the kernels on one input.
+// Every other shape runs k_gn_any on the fp32 path and has no kernel on the 16-bit layer-wise path.
+GnVariant gn_variant(int C, int H, int W, int groups, bool bf16) {
+    const GnVariant generic = bf16 ? GN_NONE : GN_ANY;
+    if (groups < 1 || C % groups) return GN_NONE;
+    const int cpg = C / groups, HW = H * W;
+    if (cpg != 4 && (cpg & 7)) return generic;                           // the three fast kernels read whole channel quads
+    const bool pair = cpg == 4, shifts = is_pow2(W) && is_pow2(HW);
+    const int upb = pair ? C / 8 : groups;                               // k_gn_tma / k_gn_warp units per sample
     const int nvec_w = pair ? HW * 2 : cpg * HW / 4;                     // float4 per warp-team unit
-    const int n_chunks = pair ? 1 : cpg / 8, unit_bytes = n_chunks * HW * 32;
-    if (!getenv("FLO_GN_CTA") && !getenv("FLO_GN_NO_TMA") && (pair || (cpg & 7) == 0) && unit_bytes >= 2048 &&
-        unit_bytes <= 16384 && HW >= 16 && (HW & (HW - 1)) == 0 && (unit_bytes & (unit_bytes - 1)) == 0) {
-        if (p.o_is_bf16) launch_gn_tma<__nv_bfloat16>(p, pair, n_chunks, s);
-        else launch_gn_tma<float>(p, pair, n_chunks, s);
-        return cudaGetLastError();
+    const int unit_bytes = (pair ? 1 : cpg / 8) * HW * 32;
+    const bool cta_only = getenv("FLO_GN_CTA") != nullptr;
+    if (!cta_only && !getenv("FLO_GN_NO_TMA") && shifts && is_pow2(upb) && HW >= 16 && unit_bytes >= 2048 &&
+        unit_bytes <= 16384 && is_pow2(unit_bytes))
+        return GN_TMA;
+    if (!cta_only && shifts && is_pow2(upb) && nvec_w >= 2 && nvec_w <= 1024 && is_pow2(nvec_w)) return GN_WARP;
+    if (shifts && is_pow2(groups) && cpg * HW / 4 <= GN_CTA_THREADS * GN_VPT) return GN_CTA;   // the unit fits a CTA's registers
+    return generic;
+}
+const char* gn_variant_name(GnVariant v) {
+    switch (v) {
+        case GN_TMA: return "tma";
+        case GN_WARP: return "warp";
+        case GN_CTA: return "cta";
+        case GN_ANY: return "any";
+        default: return "none";
     }
-    if (!getenv("FLO_GN_CTA") && nvec_w >= 2 && nvec_w <= 1024 && (nvec_w & (nvec_w - 1)) == 0 && (pair || (cpg & 7) == 0)) {
-        if (p.o_is_bf16) launch_gn_warp<__nv_bfloat16>(p, nvec_w, pair, s);
-        else launch_gn_warp<float>(p, nvec_w, pair, s);
-        return cudaGetLastError();
+}
+cudaError_t launch_gn(const GnParams& p, cudaStream_t s) {
+    const int cpg = p.C / p.groups, HW = p.H * p.W, pair = cpg == 4 ? 1 : 0;
+    switch (gn_variant(p.C, p.H, p.W, p.groups, p.o_is_bf16)) {
+        case GN_TMA: {
+            const int n_chunks = pair ? 1 : cpg / 8;
+            if (p.o_is_bf16) launch_gn_tma<__nv_bfloat16>(p, pair, n_chunks, s);
+            else launch_gn_tma<float>(p, pair, n_chunks, s);
+        } break;
+        case GN_WARP: {
+            const int nvec_w = pair ? HW * 2 : cpg * HW / 4;
+            if (p.o_is_bf16) launch_gn_warp<__nv_bfloat16>(p, nvec_w, pair, s);
+            else launch_gn_warp<float>(p, nvec_w, pair, s);
+        } break;
+        case GN_CTA: {
+            const int nvec = cpg * HW / 4;
+            int nt = 32;
+            while (nt < GN_CTA_THREADS && nt * GN_VPT < nvec) nt <<= 1;
+            // prefer ~4 vectors per thread when the unit is big enough to fill more warps
+            while (nt < GN_CTA_THREADS && nvec / nt > 4) nt <<= 1;
+            const int grid = p.B * p.groups;
+            if (p.o_is_bf16) k_gn<__nv_bfloat16><<<grid, nt, 0, s>>>(p);
+            else k_gn<float><<<grid, nt, 0, s>>>(p);
+        } break;
+        case GN_ANY: return launch_gn_any(p, s);
+        default: return cudaErrorInvalidValue;
     }
-    const int nvec = (p.C / p.groups) * p.H * p.W / 4;
-    int nt = 32;
-    while (nt < 256 && nt * GN_VPT < nvec) nt <<= 1;
-    // prefer ~4 vectors per thread when the unit is big enough to fill more warps
-    while (nt < 256 && nvec / nt > 4) nt <<= 1;
-    if (nt * GN_VPT < nvec) return p.o_is_bf16 ? cudaErrorInvalidValue : launch_gn_any(p, s);   // unit larger than a CTA's registers
-    const int grid = p.B * p.groups;
-    if (p.o_is_bf16) k_gn<__nv_bfloat16><<<grid, nt, 0, s>>>(p);
-    else k_gn<float><<<grid, nt, 0, s>>>(p);
     return cudaGetLastError();
 }
 
@@ -1035,9 +1068,11 @@ cudaError_t simt_configure() {
     return cudaFuncSetAttribute(k_linattn<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)linattn_smem(256));
 }
+// up to 256 pixels: one CTA holds q, k, v of a (sample, head); beyond, the fp32 tiled kernel takes whole LA_TILE tiles
+bool linattn_supported(int n, bool bf16) { return n >= 1 && (n <= 256 || (!bf16 && n % LA_TILE == 0)); }
 cudaError_t launch_linattn(const AttnParams& p, cudaStream_t s) {
+    if (!linattn_supported(p.n, p.is_bf16)) return cudaErrorInvalidValue;
     if (p.n > 256) {
-        if (p.is_bf16 || p.n % LA_TILE) return cudaErrorInvalidValue;
         k_linattn_big<<<p.B * 4, LA_THREADS, linattn_big_smem(), s>>>(p);
         return cudaGetLastError();
     }
@@ -1102,8 +1137,9 @@ __global__ void __launch_bounds__(64) k_midattn(AttnParams p) {
         store8(out + ((size_t)((head * 4 + cbl) * p.B + b) * n + i) * 8, o);
     }
 }
+bool midattn_supported(int n) { return n >= 1 && n <= MA_MAXN; }
 cudaError_t launch_midattn(const AttnParams& p, cudaStream_t s) {
-    if (p.n > MA_MAXN) return cudaErrorInvalidValue;
+    if (!midattn_supported(p.n)) return cudaErrorInvalidValue;
     if (p.is_bf16) k_midattn<__nv_bfloat16><<<p.B * 4, 64, 0, s>>>(p);
     else k_midattn<float><<<p.B * 4, 64, 0, s>>>(p);
     return cudaGetLastError();

@@ -68,6 +68,13 @@ def test_unsupported_configs_are_explicit_errors():
     cfg = _lib.make_cfg(24, 4, (1, 2), 4, 0, 16, 16, "bf16", 0)       # bf16 path needs dim % 16 == 0
     with pytest.raises(NotImplementedError):
         _lib.check(L.flo_param_count(ctypes.byref(cfg)))
+    # the layer-wise 16-bit GroupNorm kernels index by shifts: 6 groups per sample and 12x12 planes have no kernel there.  The
+    # manifest exists (the module can hold such weights); planning the forward refuses, naming the GroupNorm.
+    for dim, groups, mults, hw in ((48, 6, (1, 2, 4, 8), 16), (16, 4, (1, 2, 4), 12)):
+        cfg = _lib.make_cfg(dim, 8, mults, groups, 0, hw, hw, "bf16", 0, _lib.FLO_FLAG_LAYERWISE)
+        _lib.check(L.flo_param_count(ctypes.byref(cfg)))
+        with pytest.raises(NotImplementedError, match=r"GroupNorm 'downs\.0\.0\.block1' .* has no kernel"):
+            _lib.describe_plan(cfg, 8)
 
 
 def test_inpainting_manifest_matches_the_module():

@@ -18,7 +18,7 @@ import torch
 
 LIB_PATH = os.environ.get("FLO_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_C", "libflocoder_b200.so")   # FLO_LIB: A/B-test another build of the same ABI
 
-FLO_OK, FLO_ERR_INVALID, FLO_ERR_UNSUPPORTED, FLO_ERR_CUDA, FLO_ERR_NOMEM = 0, -1, -2, -3, -4
+FLO_OK, FLO_ERR_INVALID, FLO_ERR_UNSUPPORTED, FLO_ERR_CUDA, FLO_ERR_NOMEM, FLO_ERR_STEP = 0, -1, -2, -3, -4, -5
 FLO_F32, FLO_BF16, FLO_F16 = 0, 1, 2
 FLO_RK4, FLO_EULER_LEGACY, FLO_EULER_GRID = 0, 1, 2
 FLO_FLAG_NO_BUFFER_REUSE, FLO_FLAG_NO_GRAPH, FLO_FLAG_LAYERWISE = 1, 2, 4
@@ -30,6 +30,7 @@ EXPORTS = (
     "flo_integrate_nfe", "flo_unet_num_ops", "flo_unet_op_name", "flo_unet_launches_per_forward",
     "flo_unet_launch_count", "flo_unet_read_activation", "flo_selftest_umma", "flo_describe_plan",
     "flo_unet_op_info", "flo_unet_profile_ops", "flo_unet_read_timeline", "flo_unet_set_mask",
+    "flo_integrate_rk45", "flo_integrate_rk45_timing",
 )
 
 
@@ -70,6 +71,9 @@ def lib() -> ctypes.CDLL:
     L.flo_integrate_host.argtypes = [c_void_p, c_void_p, c_void_p, POINTER(c_float), c_int, c_int, c_float,
                                      c_float, c_void_p, c_float, c_int, c_void_p]
     L.flo_unet_set_mask.argtypes = [c_void_p, c_void_p, c_int, c_void_p]
+    L.flo_integrate_rk45.argtypes = [c_void_p, c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_double,
+                                     ctypes.c_double, c_float, c_void_p, c_float, c_int, POINTER(c_int), c_int, c_void_p]
+    L.flo_integrate_rk45_timing.argtypes = [c_void_p, POINTER(ctypes.c_double)]
     L.flo_integrate_nfe.argtypes = [c_int, c_int]
     L.flo_unet_num_ops.argtypes = [c_void_p]
     L.flo_unet_op_name.argtypes = [c_void_p, c_int, c_char_p, c_int]
@@ -251,6 +255,27 @@ class Engine:
                                        None if v_trace is None else v_trace.data_ptr(), b,
                                        _stream_ptr(self.device)), "flo_integrate")
         return y
+
+    def integrate_rk45(self, y: torch.Tensor, t0: float, t1: float = 1.0, rtol: float = 1e-5, atol: float = 1e-5,
+                       t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0, max_steps: int = 10000):
+        """Adaptive Dormand-Prince 5(4) from ``t0`` to ``t1`` in place on ``y`` (``flo_integrate_rk45``: scipy's RK45 step
+        control on the device, one host wait per attempt).  Returns ``(nfev, accepted, rejected)``; raises RuntimeError
+        when the step size collapses or ``max_steps`` attempts do not reach ``t1``."""
+        assert y.dtype == torch.float32 and y.is_contiguous() and y.device == self.device
+        b = y.shape[0]
+        keep, cptr = self._cls_ptr(class_ids, b)
+        counts = (c_int * 3)()
+        with torch.cuda.device(self.device):
+            check(self.L.flo_integrate_rk45(self.handle, y.data_ptr(), float(t0), float(t1), float(rtol), float(atol),
+                                            float(t_scale), cptr, float(cfg_strength), int(max_steps), counts, b,
+                                            _stream_ptr(self.device)), "flo_integrate_rk45")
+        return counts[0], counts[1], counts[2]
+
+    def rk45_timing(self):
+        """(attempts, host wall ms, attempt-graph device ms) of the last :meth:`integrate_rk45` call."""
+        out = (ctypes.c_double * 3)()
+        check(self.L.flo_integrate_rk45_timing(self.handle, out), "flo_integrate_rk45_timing")
+        return int(out[0]), out[1], out[2]
 
     def integrate_host(self, x0: torch.Tensor, x1: torch.Tensor, ts: Sequence[float], method: int,
                        dt: float = 0.0, t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0):

@@ -27,7 +27,8 @@ enum StageKind : int {
     ST_RK3 = 3,       // acc += 2k;      xs = y + dt*k                     (sampling.py:46,47)
     ST_RK4 = 4,       // acc += k;       y += (dt/6)*acc; xs = y           (sampling.py:48)
     ST_EULER = 5,     // y = y + k*dt;   xs = y                            (legacy/train_sd_flowers.py:64)
-    ST_CFG_COND = 6   // vcond = k (conditional pass of classifier-free guidance, sampling.py:63)
+    ST_CFG_COND = 6,  // vcond = k (conditional pass of classifier-free guidance, sampling.py:63)
+    ST_STORE = 7      // only vtrace[eval_idx] = k: the RK45 stage slot; k_rk45_stage forms the next input (rk45.cu)
 };
 enum StageFlags : int {
     SF_CFG_COMBINE = 1,  // this pass is the unconditional one: k = k + cfg*(vcond - k)  (sampling.py:74)
@@ -320,6 +321,45 @@ struct AttnFusedParams {
     void* out; void* out_un; void* out_up;  // outputs (16-bit blocked); un/up may be null
     long long* dbg;                         // optional clock64 timeline of CTA 0 (null in production)
 };
+
+// ---------------------------------------------------------------------------------------------
+// adaptive Dormand-Prince 5(4) with scipy's step-size control (rk45.cu, flo_integrate_rk45)
+// ---------------------------------------------------------------------------------------------
+enum Rk45State : int { RK_RUNNING = 0, RK_DONE = 1, RK_TOO_SMALL = 2, RK_TOO_MANY = 3 };
+enum Rk45EndMode : int { RK_END_NORM0 = 0, RK_END_NORM1 = 1, RK_END_STEP = 2 };
+
+struct Rk45Status {           // what the host reads back after every attempt
+    double t, h_abs;
+    int accepted, rejected, nfev, state;
+    int y_idx, pad;           // which half of Rk45Params::ybuf holds the current y
+};
+
+struct Rk45Ctl {              // device-resident controller state (scipy RungeKutta._step_impl, fp64)
+    double t, t_new, t1, h, h_abs, min_step, max_step, rtol, atol, h0, d1, interval;
+    float t_scale;
+    int max_steps, attempts, step_rejected;
+    int k0;                   // physical K slot holding K[0] (0 or 6); K[6] is in 6 - k0
+    int two_pass;             // 1: conditional + combining pass per evaluation (12 stage entries per attempt)
+    int flags;                // Stage::flags of the evaluation's (last) pass: 0, SF_CFG_2B or SF_CFG_COMBINE
+    unsigned arrive;          // k_rk45_end arrival counter (zero between launches)
+    Rk45Status status;
+};
+
+struct Rk45Params {
+    Rk45Ctl* rc;
+    Ctrl* ctrl;
+    float* k;                 // [7][n] stage velocities (Ctrl::vtrace of the attempt)
+    float* ybuf;              // [2][n] y | y_new, swapped by index on accept
+    float* xs;                // forward input [n] ...
+    float* xs2;               // ... and its unconditional half on the 2B route, or null
+    double* part;             // [rk45_end_grid(n)][2] per-CTA partial sums
+    int n;                    // B*C*H*W
+};
+
+int rk45_end_grid(int n);
+cudaError_t launch_rk45_setup(Rk45Ctl* dst, const Rk45Ctl& value, Ctrl* ctrl, cudaStream_t s);   // + stage entry of f0
+cudaError_t launch_rk45_stage(const Rk45Params& p, int stage, cudaStream_t s);   // 0: xs = y; -1: first-step trial; 1..6
+cudaError_t launch_rk45_end(const Rk45Params& p, int mode, cudaStream_t s);
 
 cudaError_t fused_configure();
 int fused_max_active_clusters(int nsplit, int smem_bytes);

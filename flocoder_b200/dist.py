@@ -13,7 +13,7 @@ from typing import Callable, Optional, Tuple
 import torch
 import torch.distributed as dist
 
-from .sampling import generate_latents_rk4
+from .sampling import generate_latents_rk4, generate_latents_rk45
 
 
 def shard_bounds(batch: int, world_size: int, rank: int) -> Tuple[int, int]:
@@ -45,7 +45,12 @@ def generate_latents_sharded(model, shape, n_steps=50, cond=None, cfg_strength=3
     Returns ``(latents, nfe)``; ``latents`` is the full ``[B,...]`` tensor on every rank when
     ``gather`` is true, else this rank's slice.  With uneven slices the gather pads to the
     largest slice and trims.
+
+    RK45 is not offered here: its step size is chosen from an error norm over the whole batch, so a
+    shard's own step control would integrate each slice differently from the unsharded batch.
     """
+    if sampler is generate_latents_rk45:
+        raise ValueError("generate_latents_sharded does not offer RK45: per-shard step control would change the result")
     if not dist.is_initialized():
         return sampler(model, shape, n_steps, cond, cfg_strength, source=source, **sampler_kwargs)
     world, rank = dist.get_world_size(group), dist.get_rank(group)

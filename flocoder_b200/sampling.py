@@ -2,7 +2,8 @@
 
 Same function names, argument order, defaults and return values as the reference:
 ``warp_time``, ``rk4_step``, ``v_func_cfg``, ``generate_latents_rk4``, ``generate_latents``
-(+ the legacy ``euler_sampler``, ``legacy/train_sd_flowers.py:50-67``).
+(+ the legacy ``euler_sampler``, ``legacy/train_sd_flowers.py:50-67``, and ``generate_latents_rk45``, the adaptive
+Dormand-Prince sampler the reference's ``method='rk45'`` dispatch names, with scipy's ``solve_ivp`` semantics).
 
 When ``model`` is a :class:`flocoder_b200.unet.Unet` the whole trajectory runs inside the
 C-ABI call ``flo_integrate``: stage times, the four U-Net evaluations per interval, the
@@ -26,7 +27,7 @@ import torch
 from . import _lib
 from .unet import Unet
 
-__all__ = ["warp_time", "rk4_step", "v_func_cfg", "generate_latents_rk4", "generate_latents",
+__all__ = ["warp_time", "rk4_step", "v_func_cfg", "generate_latents_rk4", "generate_latents_rk45", "generate_latents",
            "euler_sampler", "time_grid", "g2rgb", "decode_latents", "sampler"]
 
 
@@ -134,16 +135,92 @@ def generate_latents_rk4(model, shape, n_steps=50, cond=None, cfg_strength=3.0, 
     return state.to(out_dtype), nfe
 
 
+def _rk45_t0(init_latents, init_strength):
+    """First point of the grid :func:`generate_latents_rk4` would use: ``warp_time(0) = 0``, or the fp32
+    ``warp_time(init_strength)`` with ``init_latents``."""
+    if init_latents is None:
+        return 0.0
+    return float(warp_time(torch.tensor(float(init_strength), dtype=torch.float32)))
+
+
+@torch.no_grad()
+def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None, init_latents=None, init_strength=0.0,
+                          rtol=1e-5, atol=1e-5, max_steps=10000):
+    """Adaptive Dormand-Prince 5(4) from ``t0`` to ``t1 = 1``: ``scipy.integrate.solve_ivp(fun, (t0, 1), y0.ravel(),
+    method='RK45', rtol=rtol, atol=atol)`` as the legacy RK45 samplers call it.  Returns ``(latents, nfe)`` with
+    ``nfe`` = scipy's ``nfev`` (``2 + 6 * attempts``).
+
+    * ``t0`` is the first point of the warped grid :func:`generate_latents_rk4` would use: 0, or
+      ``warp_time(init_strength)`` after the same ``y = (1-s)*noise + s*init_latents`` mix.
+    * The model sees ``torch.ones(B) * t * 999`` in fp32 at every stage time ``t``; class conditioning and
+      classifier-free guidance follow :func:`v_func_cfg`, the inpainting mask applies to every evaluation.
+    * The whole batch is ONE ODE system with one step size, and the error norm is the RMS over all ``B*C*H*W``
+      elements, so a sample's trajectory (and the step count) depends on the rest of its batch -- the legacy
+      behaviour of calling ``solve_ivp`` on the flattened batch.
+
+    For a :class:`~flocoder_b200.unet.Unet` the integration runs on the device (``flo_integrate_rk45``: stage inputs,
+    error norm and step-size control are kernels; the host waits once per attempt of six evaluations).  Any other
+    callable keeps the legacy composition: ``solve_ivp`` on the host, calling the model once per stage.  A step size
+    below scipy's minimum step, or more than ``max_steps`` attempts, raises RuntimeError."""
+    if not rtol > 0:
+        raise ValueError(f"rtol must be > 0, got {rtol}")
+    if not atol >= 0:
+        raise ValueError(f"atol must be >= 0, got {atol}")
+    if int(max_steps) != max_steps or max_steps < 1:
+        raise ValueError(f"max_steps must be a positive integer, got {max_steps}")
+    if init_latents is not None and not 0.0 <= init_strength < 1.0:
+        raise ValueError(f"init_strength must be in [0, 1) with init_latents (t0 = warp_time(init_strength) < 1), "
+                         f"got {init_strength}")
+    device, dtype = _device_dtype(model)
+    y = source if source is not None else torch.randn(shape, device=device, dtype=dtype)
+    if init_latents is not None:
+        y = (1 - init_strength) * y + init_strength * init_latents
+    t0 = _rk45_t0(init_latents, init_strength)
+
+    if not isinstance(model, Unet):
+        # foreign model: the legacy composition -- scipy on the host, one model call per stage
+        import numpy as np
+        from scipy.integrate import solve_ivp
+        t_vec = torch.zeros(y.shape[0], device=y.device, dtype=y.dtype)
+        calls = [0]
+
+        def fun(t, yf):
+            calls[0] += 1
+            if calls[0] > 2 + 6 * max_steps:
+                raise RuntimeError(f"RK45 used max_steps={max_steps} attempts and stopped at t={t}")
+            x = torch.from_numpy(np.ascontiguousarray(yf)).to(device=y.device, dtype=y.dtype).reshape(y.shape)
+            return v_func_cfg(model, cond, cfg_strength, t_vec, x, t).double().cpu().numpy().ravel()
+
+        sol = solve_ivp(fun, (t0, 1.0), y.double().cpu().numpy().ravel(), method="RK45", rtol=rtol, atol=atol)
+        if sol.status != 0:
+            raise RuntimeError(f"RK45 failed at t={sol.t[-1]}: {sol.message}")
+        out = torch.from_numpy(sol.y[:, -1]).reshape(y.shape).to(device=y.device, dtype=y.dtype)
+        return out, int(sol.nfev)
+
+    b, c, h, w = y.shape
+    eng = model.engine(h, w)
+    out_dtype = y.dtype
+    state = y.to(device=eng.device, dtype=torch.float32).contiguous()
+    if state.data_ptr() == y.data_ptr():
+        state = state.clone()                      # never integrate in place on the caller's tensor
+    cls = _class_ids(model, cond)
+    cfg = float(cfg_strength) if (cls is not None and cfg_strength) else 0.0
+    eng.set_mask(model.mask_of(cond), b)
+    nfe, _, _ = eng.integrate_rk45(state, t0, 1.0, rtol=rtol, atol=atol, class_ids=cls, cfg_strength=cfg,
+                                   max_steps=int(max_steps))
+    return state.to(out_dtype), nfe
+
+
 @torch.no_grad()
 def generate_latents(model, shape, method="rk4", n_steps=50, cond=None, cfg_strength=3.0, device=None,
                      source=None, init_latents=None, init_strength=0.0, debug=False):
-    """Dispatch (``sampling.py:128-146``).  ``method='rk45'`` is a NameError in the reference
-    (``generate_latents_rk45`` was removed, ``sampling.py:142-143``); here it is an explicit error."""
+    """Dispatch (``sampling.py:128-146``).  ``method='rk45'`` runs :func:`generate_latents_rk45` (the reference's
+    branch calls that name, which it no longer defines) with its default tolerances; ``n_steps`` is then ignored."""
     if device is None:
         device = next(model.parameters()).device
     if method == "rk45":
-        raise NotImplementedError("method='rk45' was removed from the reference (sampling.py:142-143 calls an "
-                                  "undefined function); use method='rk4'")
+        return generate_latents_rk45(model, shape, cond, cfg_strength, source=source, init_latents=init_latents,
+                                     init_strength=init_strength)
     return generate_latents_rk4(model, shape, n_steps, cond, cfg_strength, source=source,
                                 init_latents=init_latents, init_strength=init_strength)
 

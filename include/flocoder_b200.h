@@ -46,7 +46,8 @@ typedef enum flo_status {
     FLO_ERR_INVALID = -1,     /* bad argument (ValueError in Python) */
     FLO_ERR_UNSUPPORTED = -2, /* feature outside the built path, e.g. mask_cond with a 16-bit compute type (NotImplementedError) */
     FLO_ERR_CUDA = -3,        /* CUDA runtime / driver failure (RuntimeError) */
-    FLO_ERR_NOMEM = -4
+    FLO_ERR_NOMEM = -4,
+    FLO_ERR_STEP = -5         /* adaptive integrator: step size below the minimum step, or max_steps used up (RuntimeError) */
 } flo_status;
 
 typedef enum flo_dtype { FLO_F32 = 0, FLO_BF16 = 1, FLO_F16 = 2 } flo_dtype;
@@ -140,6 +141,21 @@ FLO_API int flo_integrate_host(flo_unet_t* h, const float* x0, float* x1, const 
                        float dt, float t_scale, const int64_t* class_ids, float cfg_strength, int B,
                        void* stream);
 
+/* Adaptive Dormand-Prince 5(4) from t0 to t1 with scipy.integrate.solve_ivp(method='RK45')'s step-size control
+ * (scipy/integrate/_ivp/rk.py, common.py): select_initial_step, SAFETY 0.9, factors in [0.2, 10], exponent -1/5,
+ * min_step = 10*|nextafter(t, inf) - t|, the last step clipped to land on t1, max_step = inf.
+ * ONE ODE system for the whole batch: the flattened [B,C,H,W] state has one step size and the error norm is the RMS over
+ * all B*C*H*W elements of err/(atol + rtol*max(|y|,|y_new|)), so a sample's trajectory depends on the rest of its batch.
+ * y: [B,C,H,W] fp32 device, in = state at t0, out = state at t1.  The U-Net sees fl32(fl32(t)*t_scale) at stage time t;
+ * class_ids / cfg_strength as flo_integrate; the flo_unet_set_mask state applies.  Stage times, stage inputs, the error
+ * norm (fp64, bit-reproducible) and the controller run on the device; the host waits once per attempt (6 evaluations) for
+ * a small status record, so the call is HOST-SYNCHRONISING like flo_integrate_host and returns when y holds the result.
+ * counts (HOST, may not be NULL): nfev = 2 + 6*attempts (scipy's nfev), accepted steps, rejected attempts.
+ * FLO_ERR_INVALID for rtol <= 0, atol < 0, t1 <= t0 or max_steps < 1 (checked before anything else, no device needed);
+ * FLO_ERR_STEP when the step falls below min_step or more than max_steps attempts would be needed (message gives t). */
+FLO_API int flo_integrate_rk45(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                       const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream);
+
 /* Number of function evaluations flo_integrate performs for (method, n_ts) -- the honest count,
  * not the reference's n_steps*4 over-count (sampling.py:121). */
 FLO_API int flo_integrate_nfe(int method, int n_ts);
@@ -162,6 +178,9 @@ FLO_API int flo_unet_profile_ops(flo_unet_t* h, int B, int reps, float* ms_per_o
 /* Debug: SM-clock timeline (clock64) of CTA 0 of fused stage `stage` from the last forward at batch B; needs the
  * environment variable FLO_TIMELINE=1 when the batch plan is created.  out128: HOST array of 128 int64. */
 FLO_API int flo_unet_read_timeline(flo_unet_t* h, int B, int stage, long long* out128);
+/* Last flo_integrate_rk45 call: out = {attempts, host wall ms over the attempts, device ms of the attempt graphs (CUDA
+ * events)}; wall - device is the host round trip the per-attempt wait costs. */
+FLO_API int flo_integrate_rk45_timing(flo_unet_t* h, double out[3]);
 /* Kernel launches issued per forward pass (graph nodes) and total since creation. */
 FLO_API int flo_unet_launches_per_forward(flo_unet_t* h, int B);
 FLO_API int64_t flo_unet_launch_count(flo_unet_t* h);

@@ -294,6 +294,13 @@ struct Plan {
     double* rk_part = nullptr;
     cudaGraphExec_t graph_rk = nullptr;     // one attempt: [k_rk45_stage -> k_temb -> forward] x 6 -> k_rk45_end
     int64_t graph_rk_key = -1;
+    // per-sample RK45 (flo_integrate_rk45_per_sample), allocated on first use: controllers [B] | status | stage times [B]
+    uint8_t* rkps_buf = nullptr;
+    Rk45Ctl* rkps_ctl = nullptr;
+    Rk45PsStatus* rkps_st = nullptr;
+    float* rkps_t = nullptr;
+    cudaGraphExec_t graph_rkps = nullptr;   // one attempt: [k_rk45ps_stage -> k_temb -> forward] x 6 -> k_rk45ps_end
+    int64_t graph_rkps_key = -1;
     Plan() = default;
     Plan(const Plan&) = delete;
     Plan& operator=(const Plan&) = delete;
@@ -304,6 +311,8 @@ struct Plan {
         if (graph_c4) cudaGraphExecDestroy(graph_c4);
         if (graph_rk) cudaGraphExecDestroy(graph_rk);
         if (rk_buf) cudaFree(rk_buf);
+        if (graph_rkps) cudaGraphExecDestroy(graph_rkps);
+        if (rkps_buf) cudaFree(rkps_buf);
         if (base) cudaFree(base);
         if (dbg) cudaFree(dbg);
     }
@@ -347,6 +356,7 @@ struct Handle {
     size_t farena_ps = 0;
     // RK45 host side: pinned status record, events around every attempt, timing of the last call
     Rk45Status* h_rk = nullptr;
+    Rk45PsStatus* h_rkps = nullptr;         // the per-sample call's status record
     cudaEvent_t rk_ev[3] = {nullptr, nullptr, nullptr};
     double rk_timing[3] = {0, 0, 0};        // attempts, host wall ms, graph ms (CUDA events)
     Handle() = default;
@@ -362,6 +372,7 @@ struct Handle {
             if (h_ev[i]) cudaEventDestroy(h_ev[i]);
         }
         if (h_rk) cudaFreeHost(h_rk);
+        if (h_rkps) cudaFreeHost(h_rkps);
         for (auto& e : rk_ev) if (e) cudaEventDestroy(e);
         if (capture_stream) cudaStreamDestroy(capture_stream);
     }
@@ -1419,39 +1430,52 @@ static int ensure_rk45(Handle& h, Plan& fp, cudaStream_t st) {
     return FLO_OK;
 }
 
-int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
-                       const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream) {
-    // argument checks first: they need neither a handle nor a device
+// argument checks of both RK45 entry points: they need neither a handle nor a device
+static int rk45_check_args(double t0, double t1, double rtol, double atol, int max_steps) {
     if (!(rtol > 0)) { set_error("rtol must be > 0, got %g", rtol); return FLO_ERR_INVALID; }
     if (!(atol >= 0)) { set_error("atol must be >= 0, got %g", atol); return FLO_ERR_INVALID; }
     if (!(t1 > t0) || !isfinite(t0) || !isfinite(t1)) { set_error("need finite t0 < t1, got t0=%g t1=%g", t0, t1); return FLO_ERR_INVALID; }
     if (max_steps < 1) { set_error("max_steps must be >= 1, got %d", max_steps); return FLO_ERR_INVALID; }
+    return FLO_OK;
+}
+
+// route of an RK45 evaluation: as flo_integrate -- guidance as one 2B-sample forward on the fused path when its last stage is
+// not N-split (fp = the 2B plan, flags = SF_CFG_2B), else a conditional and a combining pass per evaluation (two_pass)
+static int rk45_route(Handle& h, int B, bool use_cfg, cudaStream_t st, Plan** fp, int* flags, int* two_pass) {
+    Plan* pl = nullptr;
+    int rc = get_plan(h, B, &pl, st);
+    if (rc) return rc;
+    *fp = pl; *flags = 0; *two_pass = use_cfg ? 1 : 0;
+    if (use_cfg && h.spec.fused && !getenv("FLO_CFG_TWO_PASS")) {
+        Plan* p2 = nullptr;
+        rc = get_plan(h, 2 * B, &p2, st);
+        if (rc) return rc;
+        const FStage& last = h.stages(p2->fvar).back();
+        if (last.kind == 0 && last.cp.nsplit == 1) { *fp = p2; *flags = SF_CFG_2B; *two_pass = 0; }
+    }
+    return FLO_OK;
+}
+
+int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                       const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream) {
+    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps);
+    if (rc) return rc;
     Handle* h = reinterpret_cast<Handle*>(hh);
     if (!h || !y || !counts) { set_error("NULL argument"); return FLO_ERR_INVALID; }
     rtol = std::max(rtol, 100 * DBL_EPSILON);             // scipy's validate_tol raises a too small rtol to 100 eps
     counts[0] = counts[1] = counts[2] = 0;
     CUDA_TRY(cudaSetDevice(h->spec.device));
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = enter_stream(*h, st);
-    if (rc) return rc;
-    Plan* pl = nullptr;
-    rc = get_plan(*h, B, &pl, st);
+    rc = enter_stream(*h, st);
     if (rc) return rc;
     const Spec& s = h->spec;
     if (s.n_classes == 0) class_ids = nullptr;              // unet.py:315: no class_cond_mlp -> cond ignored
     const bool use_cls = class_ids != nullptr;
     const bool use_cfg = use_cls && cfg_strength != 0.0f;   // sampling.py:69
-    // route: as flo_integrate -- guidance as one 2B-sample forward on the fused path when its last stage is not N-split, else a
-    // conditional and a combining pass per evaluation
-    Plan* fp = pl;
-    int flags = 0, two_pass = use_cfg ? 1 : 0;
-    if (use_cfg && s.fused && !getenv("FLO_CFG_TWO_PASS")) {
-        Plan* p2 = nullptr;
-        rc = get_plan(*h, 2 * B, &p2, st);
-        if (rc) return rc;
-        const FStage& last = h->stages(p2->fvar).back();
-        if (last.kind == 0 && last.cp.nsplit == 1) { fp = p2; flags = SF_CFG_2B; two_pass = 0; }
-    }
+    Plan* fp = nullptr;
+    int flags = 0, two_pass = 0;
+    rc = rk45_route(*h, B, use_cfg, st, &fp, &flags, &two_pass);
+    if (rc) return rc;
     const size_t n = (size_t)B * s.channels * s.H * s.W;
     rc = ensure_stage_capacity(*h, 12);
     if (rc) return rc;
@@ -1562,6 +1586,169 @@ int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rt
         return FLO_ERR_STEP;
     }
     CUDA_TRY(cudaMemcpyAsync(y, rp.ybuf + (size_t)hs->y_idx * n, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return FLO_OK;
+}
+
+// ---- per-sample RK45: every sample its own controller (rk45.cu, k_rk45ps_*); the batch still shares every U-Net evaluation
+static int ensure_rk45_per_sample(Handle& h, Plan& fp, cudaStream_t st) {
+    if (!fp.rkps_buf) {
+        auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+        const size_t cbytes = al((size_t)fp.B * sizeof(Rk45Ctl)), sbytes = al(sizeof(Rk45PsStatus));
+        const size_t bytes = cbytes + sbytes + (size_t)fp.B * sizeof(float);   // fp.B >= the caller's B on every route
+        cudaError_t e = cudaMalloc((void**)&fp.rkps_buf, bytes);
+        if (e != cudaSuccess) { cudaGetLastError(); fp.rkps_buf = nullptr; set_error("cudaMalloc of %zu RK45 bytes failed", bytes); return FLO_ERR_NOMEM; }
+        fp.rkps_ctl = (Rk45Ctl*)fp.rkps_buf;
+        fp.rkps_st = (Rk45PsStatus*)(fp.rkps_buf + cbytes);
+        fp.rkps_t = (float*)(fp.rkps_buf + cbytes + sbytes);
+        CUDA_TRY(cudaMemsetAsync(fp.rkps_buf, 0, bytes, st));
+    }
+    if (!h.h_rkps) CUDA_TRY(cudaMallocHost((void**)&h.h_rkps, sizeof(Rk45PsStatus)));
+    return FLO_OK;
+}
+
+int flo_integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                                  const int64_t* class_ids, float cfg_strength, int max_steps, int32_t* counts, int B,
+                                  void* stream) {
+    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps);
+    if (rc) return rc;
+    Handle* h = reinterpret_cast<Handle*>(hh);
+    if (!h || !y || !counts) { set_error("NULL argument"); return FLO_ERR_INVALID; }
+    if (B < 1) { set_error("batch must be >= 1, got %d", B); return FLO_ERR_INVALID; }
+    rtol = std::max(rtol, 100 * DBL_EPSILON);             // scipy's validate_tol raises a too small rtol to 100 eps
+    std::fill(counts, counts + 3 * (size_t)B, 0);
+    CUDA_TRY(cudaSetDevice(h->spec.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = enter_stream(*h, st);
+    if (rc) return rc;
+    const Spec& s = h->spec;
+    if (s.n_classes == 0) class_ids = nullptr;              // unet.py:315: no class_cond_mlp -> cond ignored
+    const bool use_cls = class_ids != nullptr;
+    const bool use_cfg = use_cls && cfg_strength != 0.0f;   // sampling.py:69
+    Plan* fp = nullptr;
+    int flags = 0, two_pass = 0;
+    rc = rk45_route(*h, B, use_cfg, st, &fp, &flags, &two_pass);
+    if (rc) return rc;
+    const int per = s.channels * s.H * s.W;
+    const size_t n = (size_t)B * per;
+    rc = ensure_stage_capacity(*h, 12);
+    if (rc) return rc;
+    rc = ensure_rk45(*h, *fp, st);
+    if (rc) return rc;
+    rc = ensure_rk45_per_sample(*h, *fp, st);
+    if (rc) return rc;
+    Rk45PsParams rp{};
+    rp.rc = fp->rkps_ctl; rp.st = fp->rkps_st; rp.ctrl = fp->ctrl; rp.k = fp->rk_buf; rp.ybuf = fp->rk_buf + 7 * n;
+    rp.xs = fp->xs; rp.xs2 = (flags & SF_CFG_2B) ? fp->xs + n : nullptr; rp.tbuf = fp->rkps_t;
+    rp.n = (int)n; rp.B = B; rp.per = per; rp.two_pass = two_pass; rp.flags = flags;
+    CUDA_TRY(cudaMemcpyAsync(rp.ybuf, y, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (use_cls) CUDA_TRY(cudaMemcpyAsync(fp->cls, class_ids, (size_t)B * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    // every route runs with one FiLM row per sample (per half on the 2B route): the rows differ in time, and in class
+    Ctrl c{};
+    c.step = 0; c.done_ctr = 0; c.film_per_sample = 1; c.n_stages = two_pass ? 12 : 6; c.cfg = cfg_strength;
+    c.cfg_half = (flags & SF_CFG_2B) ? B : 0;
+    c.y = rp.ybuf;          // read (and ignored) by the ST_STORE epilogues
+    c.acc = fp->acc; c.xs = fp->xs; c.vcond = fp->vcond; c.vout = nullptr; c.vtrace = rp.k;
+    c.film = fp->film_ps; c.stages = h->d_stages; c.pair_flags = fp->pair_flags;
+    CUDA_TRY(launch_setup_ctrl(fp->ctrl, c, nullptr, nullptr, st));
+    Rk45Ctl r{};
+    r.t = t0; r.t_new = t0; r.t1 = t1; r.rtol = rtol; r.atol = atol; r.max_step = INFINITY; r.interval = fabs(t1 - t0);
+    r.t_scale = t_scale; r.max_steps = max_steps; r.k0 = 0; r.two_pass = two_pass; r.flags = flags;
+    r.status.state = RK_RUNNING; r.status.t = t0;
+    CUDA_TRY(launch_rk45ps_setup(rp, r, st));
+    h->launches += 2;
+    // time embedding inside the evaluation, one row per sample at that sample's stage time (tbuf, written by k_rk45ps_stage)
+    TembParams tp = temb_params(*h);
+    tp.ctrl = nullptr; tp.t = rp.tbuf; tp.t_stride = 1; tp.film = fp->film_ps;
+    tp.cls = use_cls ? fp->cls : nullptr; tp.n_cond = use_cls ? B : -1;
+    tp.n_rows = (flags & SF_CFG_2B) ? 2 * B : B;
+    TembParams tp_nc = tp;                                  // the unconditional pass of the two-pass route
+    tp_nc.n_cond = 0;
+    auto evaluate = [&](cudaStream_t ss) -> int {
+        for (int pass = 0; pass < (two_pass ? 2 : 1); ++pass) {
+            if (launch_temb(pass ? tp_nc : tp, ss) != cudaSuccess) { set_error("k_temb launch failed"); return FLO_ERR_CUDA; }
+            for (int i = 0; i < n_units(*h); ++i) {
+                int r2 = launch_unit(*h, *fp, i, ss);
+                if (r2) return r2;
+            }
+        }
+        return FLO_OK;
+    };
+    auto attempt = [&](cudaStream_t ss) -> int {
+        for (int e = 1; e <= 6; ++e) {
+            if (launch_rk45ps_stage(rp, e, ss) != cudaSuccess) { set_error("k_rk45ps_stage launch failed"); return FLO_ERR_CUDA; }
+            int r2 = evaluate(ss);
+            if (r2) return r2;
+        }
+        if (launch_rk45ps_end(rp, RK_END_STEP, ss) != cudaSuccess) { set_error("k_rk45ps_end launch failed"); return FLO_ERR_CUDA; }
+        return FLO_OK;
+    };
+    const int64_t per_eval = (int64_t)(two_pass ? 2 : 1) * (n_units(*h) + 1);
+    // select_initial_step per sample: f0 = fun(t0, y0), the norms d0 / d1, a trial evaluation at t0 + h0_i, d2 -> first step
+    CUDA_TRY(launch_rk45ps_stage(rp, 0, st));
+    if ((rc = evaluate(st))) return rc;
+    CUDA_TRY(launch_rk45ps_end(rp, RK_END_NORM0, st));
+    CUDA_TRY(launch_rk45ps_stage(rp, -1, st));
+    if ((rc = evaluate(st))) return rc;
+    CUDA_TRY(launch_rk45ps_end(rp, RK_END_NORM1, st));
+    h->launches += 2 * per_eval + 4;
+    const bool graphs = !(s.flags & FLO_FLAG_NO_GRAPH);
+    const int64_t key = (int64_t)B * 8 + (use_cls ? 4 : 0) + (flags ? 2 : 0) + two_pass;
+    if (graphs && (!fp->graph_rkps || fp->graph_rkps_key != key)) {
+        if (fp->graph_rkps) { cudaGraphExecDestroy(fp->graph_rkps); fp->graph_rkps = nullptr; }
+        cudaGraph_t g = nullptr;
+        CUDA_TRY(cudaStreamBeginCapture(h->capture_stream, cudaStreamCaptureModeThreadLocal));
+        int r2 = attempt(h->capture_stream);
+        cudaError_t ce = cudaStreamEndCapture(h->capture_stream, &g);
+        if (r2 == FLO_OK && ce == cudaSuccess) ce = cudaGraphInstantiate(&fp->graph_rkps, g, 0);
+        if (g) cudaGraphDestroy(g);
+        if (r2 || ce != cudaSuccess) { if (!r2) set_error("graph capture (per-sample RK45) failed: %s", cudaGetErrorString(ce)); return r2 ? r2 : FLO_ERR_CUDA; }
+        fp->graph_rkps_key = key;
+    }
+    Rk45PsStatus* hs = h->h_rkps;
+    auto read_status = [&]() -> int {
+        CUDA_TRY(cudaMemcpyAsync(hs, fp->rkps_st, sizeof(Rk45PsStatus), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaEventRecord(h->rk_ev[2], st));
+        CUDA_TRY(cudaEventSynchronize(h->rk_ev[2]));
+        return FLO_OK;
+    };
+    if ((rc = read_status())) return rc;
+    double wall_ms = 0, graph_ms = 0;
+    int attempts = 0;
+    while (hs->running > 0 && hs->failed == 0) {             // finished samples ride along, frozen, until the last one is done
+        const auto w0 = std::chrono::steady_clock::now();
+        CUDA_TRY(cudaEventRecord(h->rk_ev[0], st));
+        if (graphs) CUDA_TRY(cudaGraphLaunch(fp->graph_rkps, st));
+        else if ((rc = attempt(st))) return rc;
+        CUDA_TRY(cudaEventRecord(h->rk_ev[1], st));
+        if ((rc = read_status())) return rc;
+        const auto w1 = std::chrono::steady_clock::now();
+        float ms = 0.f;
+        CUDA_TRY(cudaEventElapsedTime(&ms, h->rk_ev[0], h->rk_ev[1]));
+        wall_ms += std::chrono::duration<double, std::milli>(w1 - w0).count();
+        graph_ms += ms;
+        ++attempts;
+        h->launches += 6 * (per_eval + 1) + 1;
+    }
+    h->rk_timing[0] = attempts; h->rk_timing[1] = wall_ms; h->rk_timing[2] = graph_ms;
+    std::vector<Rk45Ctl> ctl((size_t)B);
+    CUDA_TRY(cudaMemcpyAsync(ctl.data(), fp->rkps_ctl, (size_t)B * sizeof(Rk45Ctl), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    for (int b = 0; b < B; ++b) {
+        counts[3 * b] = ctl[b].status.nfev; counts[3 * b + 1] = ctl[b].status.accepted; counts[3 * b + 2] = ctl[b].status.rejected;
+    }
+    if (hs->failed) {
+        const Rk45Status& f = ctl[hs->first_failed].status;
+        if (f.state == RK_TOO_SMALL)
+            set_error("RK45 sample %d: step size fell below the minimum step at t=%.17g after %d accepted and %d rejected steps "
+                      "(scipy: 'Required step size is less than spacing between numbers.')", hs->first_failed, f.t, f.accepted,
+                      f.rejected);
+        else
+            set_error("RK45 sample %d used max_steps=%d attempts and stopped at t=%.17g (%d accepted, %d rejected)",
+                      hs->first_failed, max_steps, f.t, f.accepted, f.rejected);
+        return FLO_ERR_STEP;
+    }
+    CUDA_TRY(cudaMemcpyAsync(y, rp.ybuf, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return FLO_OK;
 }

@@ -356,10 +356,38 @@ struct Rk45Params {
     int n;                    // B*C*H*W
 };
 
-int rk45_end_grid(int n);
+// CTAs of k_rk45_end over n elements (the per-sample kernel sums a sample in the same chunks)
+__host__ __device__ inline int rk45_end_grid(int n) { return n / 2048 < 1 ? 1 : (n / 2048 > 1024 ? 1024 : n / 2048); }
 cudaError_t launch_rk45_setup(Rk45Ctl* dst, const Rk45Ctl& value, Ctrl* ctrl, cudaStream_t s);   // + stage entry of f0
 cudaError_t launch_rk45_stage(const Rk45Params& p, int stage, cudaStream_t s);   // 0: xs = y; -1: first-step trial; 1..6
 cudaError_t launch_rk45_end(const Rk45Params& p, int mode, cudaStream_t s);
+
+// per-sample RK45 (flo_integrate_rk45_per_sample): one controller per sample, the same kernels' arithmetic per sample.  K and
+// y keep a fixed layout (K[0] in slot 0, y in the first half of ybuf): an accepted step copies K[6] -> K[0] and y_new -> y
+// for its sample instead of swapping indices, since the ST_STORE epilogues write one batch-uniform K slot per evaluation.
+struct Rk45PsStatus {         // what the host reads back after every attempt
+    int running, done, failed;
+    int first_failed;         // lowest failed sample index, or -1
+    unsigned arrive;          // k_rk45ps_end arrival counter (zero between launches)
+    int pad;
+};
+
+struct Rk45PsParams {
+    Rk45Ctl* rc;              // [B] controllers (status.y_idx and k0 stay 0)
+    Rk45PsStatus* st;
+    Ctrl* ctrl;
+    float* k;                 // [7][n] stage velocities
+    float* ybuf;              // [2][n] y | y_new
+    float* xs;                // forward input [n] ...
+    float* xs2;               // ... and its unconditional half on the 2B route, or null
+    float* tbuf;              // [B] (2B route: [2B]) stage time fed to the U-Net per row, read by k_temb
+    int n, B, per;            // B*C*H*W, samples, C*H*W
+    int two_pass, flags;      // as Rk45Ctl: the stage-table form of one evaluation
+};
+
+cudaError_t launch_rk45ps_setup(const Rk45PsParams& p, const Rk45Ctl& value, cudaStream_t s);   // + stage entry of f0
+cudaError_t launch_rk45ps_stage(const Rk45PsParams& p, int stage, cudaStream_t s);               // stages as launch_rk45_stage
+cudaError_t launch_rk45ps_end(const Rk45PsParams& p, int mode, cudaStream_t s);
 
 cudaError_t fused_configure();
 int fused_max_active_clusters(int nsplit, int smem_bytes);

@@ -162,8 +162,6 @@ cudaError_t launch_rk45_stage(const Rk45Params& p, int stage, cudaStream_t s) {
 }
 
 // ---- norms + controller ------------------------------------------------------------------------------------------------
-int rk45_end_grid(int n) { return std::max(1, std::min(1024, n / 2048)); }
-
 __device__ __forceinline__ double block_sum_f64(double v, double* red) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -249,6 +247,184 @@ __global__ void __launch_bounds__(256) k_rk45_end(Rk45Params p, int mode) {
 }
 cudaError_t launch_rk45_end(const Rk45Params& p, int mode, cudaStream_t s) {
     k_rk45_end<<<rk45_end_grid(p.n), 256, 0, s>>>(p, mode);
+    return cudaGetLastError();
+}
+
+// ---- per-sample RK45: B controllers, each sample its own solve_ivp ------------------------------------------------------
+//
+//   k_rk45ps_setup  every controller <- the initial state; the stage entry of f0 (slot 0)
+//   k_rk45ps_stage  k_rk45_stage's arithmetic with the sample's own h (and h0), plus the sample's stage time
+//                   fl32(fl32(t + c_s*h) * t_scale) into tbuf for k_temb; a finished sample is frozen: xs = y at t1
+//   k_rk45ps_end    one CTA per sample: k_rk45_end's norm over that sample's C*H*W elements, summed in the batched kernel's
+//                   partition (so B = 1 is bit-identical to the batched mode), the controller, and on accept the copies
+//                   K[6] -> K[0] and y_new -> y; the last CTA to arrive counts running / done / failed samples
+//
+// The stage table is the same for every attempt (only times and step sizes are per sample): evaluation e writes K slot e.
+__device__ void rk45ps_write_table(const Rk45PsParams& p, int mode) {
+    Stage* stages = const_cast<Stage*>(p.ctrl->stages);
+    Rk45Ctl c{};
+    c.two_pass = p.two_pass; c.flags = p.flags;                                       // t_scaled is unused: k_temb reads tbuf
+    if (mode == RK_END_NORM0) rk45_write_eval(stages, c, 0, 0.0, 1);                   // f1 = fun(t0 + h0, y1)
+    else for (int e = 1; e <= 6; ++e) rk45_write_eval(stages, c, e - 1, 0.0, e);
+}
+
+__global__ void k_rk45ps_setup(Rk45PsParams p, Rk45Ctl value) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < p.B) p.rc[b] = value;
+    if (b == 0) {
+        Rk45Ctl c{};
+        c.two_pass = p.two_pass; c.flags = p.flags;
+        rk45_write_eval(const_cast<Stage*>(p.ctrl->stages), c, 0, 0.0, 0);          // f0 = fun(t0, y0)
+        p.ctrl->step = 0;
+        Rk45PsStatus s{};
+        s.running = p.B; s.first_failed = -1;
+        *p.st = s;
+    }
+}
+cudaError_t launch_rk45ps_setup(const Rk45PsParams& p, const Rk45Ctl& value, cudaStream_t s) {
+    k_rk45ps_setup<<<(p.B + 255) / 256, 256, 0, s>>>(p, value);
+    return cudaGetLastError();
+}
+
+__global__ void __launch_bounds__(256) k_rk45ps_stage(Rk45PsParams p, int stage) {
+    griddep_wait();
+    const int gi = blockIdx.x * blockDim.x + threadIdx.x;
+    if (gi < p.B) {                                   // the sample's stage time, as rk45_write_eval forms it
+        const Rk45Ctl& c = p.rc[gi];
+        double t;
+        if (c.status.state != RK_RUNNING) t = c.t1;
+        else if (stage == 0) t = c.t;
+        else if (stage < 0) t = c.t + c.h0;
+        else if (stage < 6) t = c.t + RK_C[stage] * c.h;
+        else t = c.t + c.h;
+        const float ts = __fmul_rn((float)t, c.t_scale);
+        p.tbuf[gi] = ts;
+        if (p.xs2) p.tbuf[p.B + gi] = ts;             // the unconditional half of the 2B route
+    }
+    const float* y = p.ybuf;
+    float* ynew = p.ybuf + p.n;
+    const float* ks[6];
+#pragma unroll
+    for (int j = 0; j < 6; ++j) ks[j] = p.k + (size_t)j * p.n;
+    for (int i = gi; i < p.n; i += gridDim.x * blockDim.x) {
+        const Rk45Ctl& c = p.rc[i / p.per];
+        const float yv = y[i];
+        float x;
+        if (stage == 0 || c.status.state != RK_RUNNING) {
+            x = yv;
+        } else if (stage < 0) {                       // select_initial_step: y1 = y0 + h0 * f0
+            x = __fadd_rn(yv, __fmul_rn((float)c.h0, ks[0][i]));
+        } else {
+            const float h = (float)c.h;
+            const float* a = stage < 6 ? RK_A[stage] : RK_B;
+            float acc = __fmul_rn(a[0], ks[0][i]);
+            for (int j = 1; j < stage; ++j) acc = __fadd_rn(acc, __fmul_rn(a[j], ks[j][i]));
+            x = __fadd_rn(yv, __fmul_rn(acc, h));   // y + dot(K[:s].T, a) * h
+            if (stage == 6) ynew[i] = x;
+        }
+        p.xs[i] = x;
+        if (p.xs2) p.xs2[i] = x;
+    }
+}
+cudaError_t launch_rk45ps_stage(const Rk45PsParams& p, int stage, cudaStream_t s) {
+    const int grid = std::max(std::min((p.n + 255) / 256, 148 * 8), (p.B + 255) / 256);
+    k_rk45ps_stage<<<grid, 256, 0, s>>>(p, stage);
+    return cudaGetLastError();
+}
+
+__global__ void __launch_bounds__(256) k_rk45ps_end(Rk45PsParams p, int mode) {
+    __shared__ double red[8];
+    __shared__ int last, accepted, cnt[3], first;
+    griddep_wait();
+    const int b = blockIdx.x;
+    Rk45Ctl* rc = p.rc + b;
+    const size_t off = (size_t)b * p.per;
+    if (rc->status.state == RK_RUNNING) {
+        const double rtol = rc->rtol, atol = rc->atol, h = rc->h;
+        const float* y = p.ybuf + off;
+        const float* yn = p.ybuf + p.n + off;
+        const float* ks[7];
+#pragma unroll
+        for (int j = 0; j < 7; ++j) ks[j] = p.k + (size_t)j * p.n + off;
+        // k_rk45_end's loops over the chunks its grid would give a lone sample, partials added in chunk order
+        const int G = rk45_end_grid(p.per), per = (p.per + G - 1) / G;
+        double a0 = 0.0, a1 = 0.0;
+        for (int g = 0; g < G; ++g) {
+            double s0 = 0.0, s1 = 0.0;
+            const int i0 = g * per, i1 = min(p.per, i0 + per);
+            if (mode == RK_END_STEP) {
+                for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+                    double e = 0.0;
+#pragma unroll
+                    for (int j = 0; j < 7; ++j) e = fma((double)ks[j][i], RK_E[j], e);
+                    const double err = e * h;                                      // dot(K.T, E) * h
+                    const double scale = atol + fmax(fabs((double)y[i]), fabs((double)yn[i])) * rtol;
+                    const double q = err / scale;
+                    s0 = fma(q, q, s0);
+                }
+            } else {
+                for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+                    const double yv = (double)y[i];
+                    const double scale = atol + fabs(yv) * rtol;
+                    if (mode == RK_END_NORM0) {
+                        const double a = yv / scale, f = (double)ks[0][i] / scale;
+                        s0 = fma(a, a, s0); s1 = fma(f, f, s1);
+                    } else {
+                        const double d = ((double)ks[1][i] - (double)ks[0][i]) / scale;
+                        s0 = fma(d, d, s0);
+                    }
+                }
+            }
+            s0 = block_sum_f64(s0, red);
+            s1 = block_sum_f64(s1, red);
+            if (threadIdx.x == 0) { a0 += s0; a1 += s1; }
+        }
+        if (threadIdx.x == 0) {
+            Rk45Ctl c = *rc;
+            const int acc0 = c.status.accepted;
+            const double rn = sqrt((double)p.per);
+            rk45_control(c, mode, sqrt(a0) / rn, sqrt(a1) / rn);           // norm(x) = ||x||_2 / sqrt(x.size)
+            accepted = c.status.accepted != acc0;
+            c.status.y_idx = 0; c.k0 = 0;             // fixed layout: the accepted step is copied below
+            *rc = c;
+        }
+        __syncthreads();
+        if (accepted) {
+            float* yw = p.ybuf + off;
+            float* k0 = p.k + off;
+            const float* k6 = p.k + (size_t)6 * p.n + off;
+            for (int i = threadIdx.x; i < p.per; i += blockDim.x) { yw[i] = yn[i]; k0[i] = k6[i]; }
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        last = atomicAdd(&p.st->arrive, 1u) == gridDim.x - 1;
+        cnt[0] = cnt[1] = cnt[2] = 0;
+        first = p.B;
+    }
+    __syncthreads();
+    if (!last) return;
+    // the last CTA to arrive: count the samples' states, publish the status record, reset the stage table position
+    __threadfence();
+    for (int i = threadIdx.x; i < p.B; i += blockDim.x) {
+        const int s = __ldcg(&p.rc[i].status.state);
+        if (s == RK_RUNNING) atomicAdd(&cnt[0], 1);
+        else if (s == RK_DONE) atomicAdd(&cnt[1], 1);
+        else { atomicAdd(&cnt[2], 1); atomicMin(&first, i); }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        Rk45PsStatus s{};
+        s.running = cnt[0]; s.done = cnt[1]; s.failed = cnt[2]; s.first_failed = cnt[2] ? first : -1; s.arrive = 0;
+        *p.st = s;
+        if (mode != RK_END_STEP) rk45ps_write_table(p, mode);
+        p.ctrl->step = 0;
+        __threadfence();
+    }
+}
+cudaError_t launch_rk45ps_end(const Rk45PsParams& p, int mode, cudaStream_t s) {
+    k_rk45ps_end<<<p.B, 256, 0, s>>>(p, mode);
     return cudaGetLastError();
 }
 

@@ -46,13 +46,24 @@ def generate_latents_sharded(model, shape, n_steps=50, cond=None, cfg_strength=3
     ``gather`` is true, else this rank's slice.  With uneven slices the gather pads to the
     largest slice and trims.
 
-    RK45 is not offered here: its step size is chosen from an error norm over the whole batch, so a
-    shard's own step control would integrate each slice differently from the unsharded batch.
+    RK45 is offered per sample only (``sampler=generate_latents_rk45, per_sample=True``; ``n_steps`` is then
+    ignored): every sample has its own step control, so a shard integrates each of its samples as the unsharded
+    batch does, and ``nfe`` is the ``[B]`` tensor of per-sample counts, gathered (or sliced) like the latents.  The
+    batched RK45 chooses its step size from an error norm over the whole batch, so a shard's own step control would
+    integrate each slice differently, and it is refused.
     """
-    if sampler is generate_latents_rk45:
-        raise ValueError("generate_latents_sharded does not offer RK45: per-shard step control would change the result")
+    rk45 = sampler is generate_latents_rk45
+    if rk45 and not sampler_kwargs.get("per_sample"):
+        raise ValueError("generate_latents_sharded does not offer batched RK45: per-shard step control would change the "
+                         "result (use per_sample=True)")
+
+    def run(shape_, cond_, source_, **kw):
+        if rk45:                                           # its third positional parameter is cond, not n_steps
+            return sampler(model, shape_, cond=cond_, cfg_strength=cfg_strength, source=source_, **kw)
+        return sampler(model, shape_, n_steps, cond_, cfg_strength, source=source_, **kw)
+
     if not dist.is_initialized():
-        return sampler(model, shape, n_steps, cond, cfg_strength, source=source, **sampler_kwargs)
+        return run(shape, cond, source, **sampler_kwargs)
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     b = shape[0]
     lo, hi = shard_bounds(b, world, rank)
@@ -70,21 +81,26 @@ def generate_latents_sharded(model, shape, n_steps=50, cond=None, cfg_strength=3
         elif torch.is_tensor(v) and v.dim() >= 1 and v.shape[0] != 1:
             raise ValueError(f"sharded sampling: tensor argument '{k}' has leading dimension {v.shape[0]}, expected the global batch {b}")
     if hi > lo:
-        local, nfe = sampler(model, local_shape, n_steps, shard_cond(cond, lo, hi), cfg_strength,
-                             source=local_src, **local_kwargs)
+        local, nfe = run(local_shape, shard_cond(cond, lo, hi), local_src, **local_kwargs)
     else:
-        local, nfe = local_src.clone(), n_steps * 4
+        local, nfe = local_src.clone(), (torch.zeros(0, dtype=torch.int64) if rk45 else n_steps * 4)
     if not gather:
         return local, nfe
-    per = -(-b // world)                                   # ceil: padded slice length
-    padded = torch.zeros((per,) + tuple(shape[1:]), device=local.device, dtype=local.dtype)
-    padded[: hi - lo] = local
-    full = torch.empty((world * per,) + tuple(shape[1:]), device=local.device, dtype=local.dtype)
-    dist.all_gather_into_tensor(full, padded, group=group)
-    if b % world == 0:
-        return full, nfe
-    pieces = []
-    for r in range(world):
-        rlo, rhi = shard_bounds(b, world, r)
-        pieces.append(full[r * per: r * per + (rhi - rlo)])
-    return torch.cat(pieces, dim=0), nfe
+
+    def all_gather(x):
+        per = -(-b // world)                               # ceil: padded slice length
+        padded = torch.zeros((per,) + tuple(x.shape[1:]), device=x.device, dtype=x.dtype)
+        padded[: hi - lo] = x
+        full = torch.empty((world * per,) + tuple(x.shape[1:]), device=x.device, dtype=x.dtype)
+        dist.all_gather_into_tensor(full, padded, group=group)
+        if b % world == 0:
+            return full
+        pieces = []
+        for r in range(world):
+            rlo, rhi = shard_bounds(b, world, r)
+            pieces.append(full[r * per: r * per + (rhi - rlo)])
+        return torch.cat(pieces, dim=0)
+
+    if rk45:                                               # the per-sample counts travel with the latents (NCCL: on the GPU)
+        nfe = all_gather(nfe.to(local.device)).cpu()
+    return all_gather(local), nfe

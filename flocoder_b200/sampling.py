@@ -143,9 +143,41 @@ def _rk45_t0(init_latents, init_strength):
     return float(warp_time(torch.tensor(float(init_strength), dtype=torch.float32)))
 
 
+def _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps, what=""):
+    """The legacy composition for a foreign model: ``solve_ivp`` on the host over ``y.ravel()``, one model call per stage.
+    Returns ``(state at t1, nfev)``; ``what`` names the problem in the errors (e.g. ``"sample 3 "``)."""
+    import numpy as np
+    from scipy.integrate import solve_ivp
+    t_vec = torch.zeros(y.shape[0], device=y.device, dtype=y.dtype)
+    calls = [0]
+
+    def fun(t, yf):
+        calls[0] += 1
+        if calls[0] > 2 + 6 * max_steps:
+            raise RuntimeError(f"RK45 {what}used max_steps={max_steps} attempts and stopped at t={t}")
+        x = torch.from_numpy(np.ascontiguousarray(yf)).to(device=y.device, dtype=y.dtype).reshape(y.shape)
+        return v_func_cfg(model, cond, cfg_strength, t_vec, x, t).double().cpu().numpy().ravel()
+
+    sol = solve_ivp(fun, (t0, 1.0), y.double().cpu().numpy().ravel(), method="RK45", rtol=rtol, atol=atol)
+    if sol.status != 0:
+        raise RuntimeError(f"RK45 {what}failed at t={sol.t[-1]}: {sol.message}")
+    return torch.from_numpy(sol.y[:, -1]).reshape(y.shape).to(device=y.device, dtype=y.dtype), int(sol.nfev)
+
+
+def _sample_cond(cond, i):
+    """``cond`` for sample ``i`` alone: the per-sample tensors (``class_cond``, ``mask_cond``) cut to ``[i:i+1]``."""
+    if cond is None:
+        return None
+    out = dict(cond)
+    for key in ("class_cond", "mask_cond"):
+        if out.get(key) is not None:
+            out[key] = out[key][i:i + 1]
+    return out
+
+
 @torch.no_grad()
 def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None, init_latents=None, init_strength=0.0,
-                          rtol=1e-5, atol=1e-5, max_steps=10000):
+                          rtol=1e-5, atol=1e-5, max_steps=10000, per_sample=False):
     """Adaptive Dormand-Prince 5(4) from ``t0`` to ``t1 = 1``: ``scipy.integrate.solve_ivp(fun, (t0, 1), y0.ravel(),
     method='RK45', rtol=rtol, atol=atol)`` as the legacy RK45 samplers call it.  Returns ``(latents, nfe)`` with
     ``nfe`` = scipy's ``nfev`` (``2 + 6 * attempts``).
@@ -158,10 +190,17 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
       elements, so a sample's trajectory (and the step count) depends on the rest of its batch -- the legacy
       behaviour of calling ``solve_ivp`` on the flattened batch.
 
-    For a :class:`~flocoder_b200.unet.Unet` the integration runs on the device (``flo_integrate_rk45``: stage inputs,
-    error norm and step-size control are kernels; the host waits once per attempt of six evaluations).  Any other
-    callable keeps the legacy composition: ``solve_ivp`` on the host, calling the model once per stage.  A step size
-    below scipy's minimum step, or more than ``max_steps`` attempts, raises RuntimeError."""
+    With ``per_sample=True`` every sample is its own problem, ``solve_ivp(fun_i, (t0, 1), y0[i].ravel(), 'RK45')``,
+    with its own step size, accept / reject decisions and error norm (the RMS over its ``C*H*W`` elements), so its result
+    does not depend on the rest of the batch; ``nfe`` is then a CPU int64 tensor ``[B]`` of each sample's ``nfev``, and
+    ``max_steps`` counts each sample's attempts.  Everything else is as above.
+
+    For a :class:`~flocoder_b200.unet.Unet` the integration runs on the device (``flo_integrate_rk45``, or
+    ``flo_integrate_rk45_per_sample`` with one controller per sample while the batch shares every evaluation: stage
+    inputs, error norms and step-size control are kernels; the host waits once per attempt of six evaluations).  Any
+    other callable keeps the legacy composition: ``solve_ivp`` on the host, calling the model once per stage (per sample,
+    on ``x[i:i+1]`` with ``cond`` cut to that sample).  A step size below scipy's minimum step, or more than ``max_steps``
+    attempts, raises RuntimeError (naming the sample with ``per_sample``)."""
     if not rtol > 0:
         raise ValueError(f"rtol must be > 0, got {rtol}")
     if not atol >= 0:
@@ -179,23 +218,14 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
 
     if not isinstance(model, Unet):
         # foreign model: the legacy composition -- scipy on the host, one model call per stage
-        import numpy as np
-        from scipy.integrate import solve_ivp
-        t_vec = torch.zeros(y.shape[0], device=y.device, dtype=y.dtype)
-        calls = [0]
-
-        def fun(t, yf):
-            calls[0] += 1
-            if calls[0] > 2 + 6 * max_steps:
-                raise RuntimeError(f"RK45 used max_steps={max_steps} attempts and stopped at t={t}")
-            x = torch.from_numpy(np.ascontiguousarray(yf)).to(device=y.device, dtype=y.dtype).reshape(y.shape)
-            return v_func_cfg(model, cond, cfg_strength, t_vec, x, t).double().cpu().numpy().ravel()
-
-        sol = solve_ivp(fun, (t0, 1.0), y.double().cpu().numpy().ravel(), method="RK45", rtol=rtol, atol=atol)
-        if sol.status != 0:
-            raise RuntimeError(f"RK45 failed at t={sol.t[-1]}: {sol.message}")
-        out = torch.from_numpy(sol.y[:, -1]).reshape(y.shape).to(device=y.device, dtype=y.dtype)
-        return out, int(sol.nfev)
+        if not per_sample:
+            return _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps)
+        outs, nfe = [], torch.zeros(y.shape[0], dtype=torch.int64)
+        for i in range(y.shape[0]):
+            out_i, nfe[i] = _solve_ivp_rk45(model, y[i:i + 1], _sample_cond(cond, i), cfg_strength, t0, rtol, atol,
+                                            max_steps, what=f"sample {i} ")
+            outs.append(out_i)
+        return torch.cat(outs, dim=0) if outs else y.clone(), nfe
 
     b, c, h, w = y.shape
     eng = model.engine(h, w)
@@ -206,6 +236,10 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
     cls = _class_ids(model, cond)
     cfg = float(cfg_strength) if (cls is not None and cfg_strength) else 0.0
     eng.set_mask(model.mask_of(cond), b)
+    if per_sample:
+        counts = eng.integrate_rk45_per_sample(state, t0, 1.0, rtol=rtol, atol=atol, class_ids=cls, cfg_strength=cfg,
+                                               max_steps=int(max_steps))
+        return state.to(out_dtype), counts[:, 0].clone()
     nfe, _, _ = eng.integrate_rk45(state, t0, 1.0, rtol=rtol, atol=atol, class_ids=cls, cfg_strength=cfg,
                                    max_steps=int(max_steps))
     return state.to(out_dtype), nfe

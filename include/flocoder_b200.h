@@ -156,6 +156,19 @@ FLO_API int flo_integrate_host(flo_unet_t* h, const float* x0, float* x1, const 
 FLO_API int flo_integrate_rk45(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol, float t_scale,
                        const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream);
 
+/* Per-sample adaptive Dormand-Prince 5(4): every sample is its own solve_ivp(fun_i, (t0, t1), y0[i].ravel(), 'RK45') with
+ * its own t, step size, accept / reject decisions and nfev; the error norm of sample i is the RMS over its C*H*W elements,
+ * so a sample's result does not depend on the rest of its batch.  The batch still shares every U-Net evaluation: a sample
+ * that reached t1 stays frozen (evaluated at t1, state unchanged) until the last one is done.  Arguments, routes, the
+ * host-synchronising wait per attempt and the error codes are those of flo_integrate_rk45; at B = 1 the result and counts
+ * equal it bit for bit.  max_steps counts attempts per sample.
+ * counts (HOST, may not be NULL): [B][3] = nfev (2 + 6*attempts_i), accepted steps, rejected attempts per sample.
+ * FLO_ERR_STEP when a sample's step falls below its min_step or it needs more than max_steps attempts: the message names
+ * the lowest failing sample index and its t, and y is left unchanged. */
+FLO_API int flo_integrate_rk45_per_sample(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol,
+                       float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps, int32_t* counts, int B,
+                       void* stream);
+
 /* Number of function evaluations flo_integrate performs for (method, n_ts) -- the honest count,
  * not the reference's n_steps*4 over-count (sampling.py:121). */
 FLO_API int flo_integrate_nfe(int method, int n_ts);
@@ -178,7 +191,7 @@ FLO_API int flo_unet_profile_ops(flo_unet_t* h, int B, int reps, float* ms_per_o
 /* Debug: SM-clock timeline (clock64) of CTA 0 of fused stage `stage` from the last forward at batch B; needs the
  * environment variable FLO_TIMELINE=1 when the batch plan is created.  out128: HOST array of 128 int64. */
 FLO_API int flo_unet_read_timeline(flo_unet_t* h, int B, int stage, long long* out128);
-/* Last flo_integrate_rk45 call: out = {attempts, host wall ms over the attempts, device ms of the attempt graphs (CUDA
+/* Last flo_integrate_rk45 or flo_integrate_rk45_per_sample call: out = {attempts (per-sample: of the whole batch), host wall ms over the attempts, device ms of the attempt graphs (CUDA
  * events)}; wall - device is the host round trip the per-attempt wait costs. */
 FLO_API int flo_integrate_rk45_timing(flo_unet_t* h, double out[3]);
 /* Kernel launches issued per forward pass (graph nodes) and total since creation. */

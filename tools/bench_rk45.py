@@ -6,7 +6,12 @@ Per configuration: samples/s of the adaptive solve (rtol = atol = 1e-5), its nfe
 CUDA events (flo_integrate_rk45_timing); and samples/s of RK4-50 (200 evaluations) from the same run.  Prints one JSON line
 per configuration, with the card name and power limit, and writes them to --out when given.
 
-    python tools/bench_rk45.py [--batches 256 1024] [--dtypes fp16 bf16] [--reps 3] [--out FILE]
+With --per-sample the per-sample RK45 (every sample its own step-size control) runs as a third arm, alternating with the
+other two on the same inputs.  Besides samples/s, attempts (the batch's, = the most any sample made) and the host gap it
+reports each sample's nfe (min / median / max) and the share of evaluated sample-forwards spent on samples that had already
+reached t = 1: 1 - sum_i nfe_i / (B * (2 + 6 * attempts)).
+
+    python tools/bench_rk45.py [--batches 256 1024] [--dtypes fp16 bf16] [--reps 3] [--per-sample] [--out FILE]
 """
 import argparse
 import json
@@ -35,6 +40,7 @@ def main():
     ap.add_argument("--batches", type=int, nargs="+", default=[256, 1024])
     ap.add_argument("--dtypes", nargs="+", default=["fp16", "bf16"])
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--per-sample", action="store_true", help="also time the per-sample RK45")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
@@ -59,12 +65,18 @@ def main():
             def rk45():
                 return sampling.generate_latents_rk45(m, (b, 4, 16, 16), source=x0)
 
+            def rk45ps():
+                return sampling.generate_latents_rk45(m, (b, 4, 16, 16), source=x0, per_sample=True)
+
             def rk4():
                 return sampling.generate_latents_rk4(m, (b, 4, 16, 16), n_steps=50, source=x0)   # the reference's RK4-50: 49 intervals
 
             rk45(); rk4(); torch.cuda.synchronize()                  # warm-up: plans, graphs, modules
+            if args.per_sample:
+                rk45ps(); torch.cuda.synchronize()
             best45, best4, timing, nfe = float("inf"), float("inf"), None, 0
-            for _ in range(args.reps):                               # alternate the two integrators
+            best_ps, timing_ps, nfe_ps = float("inf"), None, None
+            for _ in range(args.reps):                               # alternate the integrators
                 torch.cuda.synchronize()
                 t0 = time.perf_counter()
                 _, nfe = rk45()
@@ -76,6 +88,13 @@ def main():
                 rk4()
                 torch.cuda.synchronize()
                 best4 = min(best4, time.perf_counter() - t0)
+                if args.per_sample:
+                    t0 = time.perf_counter()
+                    _, nfe_ps = rk45ps()
+                    torch.cuda.synchronize()
+                    dtps = time.perf_counter() - t0
+                    if dtps < best_ps:
+                        best_ps, timing_ps = dtps, eng.rk45_timing()
             attempts, wall_ms, graph_ms = timing
             rec = {"card": name, "power_limit": power, "dtype": dt, "batch": b, "net": "flowers_sd trained_like",
                    "rk45": {"rtol": 1e-5, "atol": 1e-5, "samples_per_s": b / best45, "nfe": nfe, "attempts": attempts,
@@ -83,6 +102,16 @@ def main():
                             "host_gap_ms_per_attempt": (wall_ms - graph_ms) / attempts,
                             "host_gap_share": (wall_ms - graph_ms) / wall_ms},
                    "rk4_50": {"samples_per_s": b / best4, "nfe": 200}, "reps": args.reps, "timing": "best of reps, wall clock"}
+            if args.per_sample:
+                a_ps, wall_ps, graph_ps = timing_ps
+                evaluated = b * (2 + 6 * a_ps)                       # sample-forwards the batch ran, finished samples included
+                rec["rk45_per_sample"] = {
+                    "rtol": 1e-5, "atol": 1e-5, "samples_per_s": b / best_ps, "attempts": a_ps,
+                    "nfe_min": int(nfe_ps.min()), "nfe_median": int(nfe_ps.median()), "nfe_max": int(nfe_ps.max()),
+                    "nfe_mean": float(nfe_ps.double().mean()),
+                    "finished_forward_share": 1.0 - int(nfe_ps.sum()) / evaluated,
+                    "ms_per_attempt_wall": wall_ps / a_ps, "ms_per_attempt_graph": graph_ps / a_ps,
+                    "host_gap_ms_per_attempt": (wall_ps - graph_ps) / a_ps, "host_gap_share": (wall_ps - graph_ps) / wall_ps}
             print(json.dumps(rec), flush=True)
             lines.append(rec)
     if args.out:

@@ -63,7 +63,7 @@ struct Spec {
     bool bf16;                 // 16-bit tensor-core operand path (bf16 or fp16)
     bool f16;                  // operands are fp16 instead of bf16 (fused path only)
     bool fused;                // fused stage kernels (default for the 16-bit paths)
-    bool mask_cond;            // inpainting U-Net: mask-fusion branches (unet.py:214-235), fp32 path only
+    bool mask_cond;            // inpainting U-Net: mask-fusion branches (unet.py:214-235): fp32 path or layer-wise bf16
     int flags, device;
     std::vector<int> dims;     // [dim, dim*m0, dim*m1, ...]   (unet.py:189)
     int time_dim;              // dim*8                         (unet.py:197)
@@ -81,9 +81,10 @@ struct ParamInfo {
 
 static int make_spec(const flo_unet_cfg* c, Spec& s) {
     if (!c) { set_error("cfg is NULL"); return FLO_ERR_INVALID; }
-    if (c->mask_cond && c->compute_dtype != FLO_F32) {
-        set_error("mask_cond=1 (inpainting U-Net, unet.py:214-235) runs on the fp32 path only: its 5x5 / (dim+channels)-input "
-                  "fusion convolutions have no tcgen05 stage kernels; use compute_dtype fp32");
+    if (c->mask_cond && c->compute_dtype != FLO_F32 && !(c->compute_dtype == FLO_BF16 && (c->flags & FLO_FLAG_LAYERWISE))) {
+        set_error("mask_cond=1 (inpainting U-Net, unet.py:214-235) runs on the fp32 path, or in bf16 on the layer-wise path "
+                  "(FLO_FLAG_LAYERWISE): its 5x5 / (dim+channels)-input fusion convolutions have no fused stage kernels and no "
+                  "fp16 kernels");
         return FLO_ERR_UNSUPPORTED;
     }
     if (c->n_mults < 1 || c->n_mults > 8) { set_error("n_mults must be in 1..8"); return FLO_ERR_INVALID; }
@@ -234,7 +235,7 @@ struct Op {
     size_t w_simt = NONE, w_umma = NONE, bias = NONE;
     int n_tile = 0;
     int res = -1, out_m = -1, out_o = -1;
-    int act_silu = 0, need_mode = 0, bypass = -1;   // mask-fusion convs (fp32 path)
+    int act_silu = 0, need_mode = 0, bypass = -1;   // mask-fusion convs
     // gn
     int gn_in = -1, C = 0, groups = 0, film_off = -1, silu = 0, out_un = -1, out_up = -1;
     size_t gamma = NONE, beta = NONE;
@@ -452,7 +453,15 @@ struct Builder {
             if (n_tile) {
                 size_t off = (h.blob_bf16.size() + 63) & ~(size_t)63;     // 128-byte aligned streams
                 h.blob_bf16.resize(off);
-                pack_umma_weights(w.data(), cout, cin, ksize, perm ? perm->data() : nullptr, n_tile, s.f16, h.blob_bf16);
+                const float* wsrc = w.data();
+                std::vector<float> wpad;
+                if (cin_ref != cin) {   // [cout][C0 + c1_real][k][k] -> [cout][C0 + C1][k][k]: zero columns for the padding channels
+                    wpad.assign((size_t)cout * cin * taps, 0.f);
+                    for (int co = 0; co < cout; ++co)
+                        memcpy(&wpad[(size_t)co * cin * taps], &w[(size_t)co * cin_ref * taps], (size_t)cin_ref * taps * sizeof(float));
+                    wsrc = wpad.data();
+                }
+                pack_umma_weights(wsrc, cout, cin, ksize, perm ? perm->data() : nullptr, n_tile, s.f16, h.blob_bf16);
                 op.w_umma = off;
             }
         }
@@ -544,15 +553,18 @@ struct Builder {
             h.ops.push_back(op);
         }
         const int n_mask = s.mask_cond ? std::min(2, n) : 0;      // levels with a down / up mask fusion (unet.py:225,232)
+        // mask channels as the convolutions read them: one fp32 8-channel block, or on the 16-bit path one bf16 K16 slice
+        const int mc = s.bf16 ? 16 : 8;
         if (s.mask_cond) {
-            // per-level blocked copies of cond['mask_cond'] (8-channel block, zero padded), filled by flo_unet_set_mask;
+            // per-level blocked copies of cond['mask_cond'] (zero padded to mc channels), filled by flo_unet_set_mask;
             // never (re)defined by an op, so the arena keeps them for the whole program
-            for (int l = 0; l < n; ++l) h.mask_buf[l] = newbuf("mask_cond:" + std::to_string(l), 8, s.H >> l, s.W >> l, false);
+            for (int l = 0; l < n; ++l) h.mask_buf[l] = newbuf("mask_cond:" + std::to_string(l), mc, s.H >> l, s.W >> l, s.bf16);
             // x = mask_fusion_conv(cat(x, mask))   (unet.py:298-305; no residual; skipped when the mask is all ones)
             ConvExtra e0; e0.c1_real = s.channels; e0.silu = true; e0.need_mode = 2;
-            Val f0 = conv("mask_fusion_conv.0", "mask_fusion_conv.0", x.o, s.dim, h.mask_buf[0], 8, s.H, s.W, 2 * s.dim, 5, true, true, true, -1, nullptr, &e0);
+            // (the two inner convs feed only the next conv: no fp32 master on the 16-bit path)
+            Val f0 = conv("mask_fusion_conv.0", "mask_fusion_conv.0", x.o, s.dim, h.mask_buf[0], mc, s.H, s.W, 2 * s.dim, 5, true, false, true, -1, nullptr, &e0);
             ConvExtra e1; e1.silu = true; e1.need_mode = 2;
-            Val f1 = conv("mask_fusion_conv.2", "mask_fusion_conv.2", f0.o, 2 * s.dim, -1, 0, s.H, s.W, 2 * s.dim, 3, true, true, true, -1, nullptr, &e1);
+            Val f1 = conv("mask_fusion_conv.2", "mask_fusion_conv.2", f0.o, 2 * s.dim, -1, 0, s.H, s.W, 2 * s.dim, 3, true, false, true, -1, nullptr, &e1);
             ConvExtra e2; e2.need_mode = 2; e2.bypass = x.m;
             x = conv("mask_fusion_conv.4", "mask_fusion_conv", f1.o, 2 * s.dim, -1, 0, s.H, s.W, s.dim, 3, true, true, true, -1, nullptr, &e2);
         }
@@ -574,7 +586,7 @@ struct Builder {
                 // x = x + SiLU(conv3x3(cat(x, resize(mask))))   (unet.py:336-340); the skip above keeps the un-fused x
                 ConvExtra e; e.c1_real = s.channels; e.silu = true; e.need_mode = 1; e.bypass = x3.m; e.want_un = !last;
                 const std::string mp = "down_mask_fusions." + std::to_string(l) + ".0";
-                x3 = conv(mp, mp, x3.o, din, h.mask_buf[l], 8, H, W, din, 3, true, true, true, x3.m, nullptr, &e);
+                x3 = conv(mp, mp, x3.o, din, h.mask_buf[l], mc, H, W, din, 3, true, true, true, x3.m, nullptr, &e);
             }
             if (!last) {
                 // our unshuffled channel order is (p1 p2 c); the reference's is (c p1 p2)  (unet.py:52)
@@ -604,7 +616,7 @@ struct Builder {
                 // unet.py:360-364, at the resolution of this up level (mask level l)
                 ConvExtra e; e.c1_real = s.channels; e.silu = true; e.need_mode = 1; e.bypass = x.m; e.want_up = !last;
                 const std::string mp = "up_mask_fusions." + std::to_string(i) + ".0";
-                x = conv(mp, mp, x.o, dout, h.mask_buf[l], 8, H, W, dout, 3, true, true, true, x.m, nullptr, &e);
+                x = conv(mp, mp, x.o, dout, h.mask_buf[l], mc, H, W, dout, 3, true, true, true, x.m, nullptr, &e);
             }
             if (!last) {
                 x = conv(p + ".3.1", p + ".3", x.up, dout, -1, 0, H * 2, W * 2, din, 3, true, false, true);
@@ -682,6 +694,22 @@ static int check_op_kernels(const Handle& h) {
                       "of 256", op.name.c_str(), op.H, op.W, op.n, path);
             return FLO_ERR_UNSUPPORTED;
         }
+        if (op.kind == OP_CONV && s.bf16) {
+            // k_conv_umma: whole K16 slices, an odd window up to 5x5, TMA boxes of at most 256 per dimension, and a tiling
+            // that fits shared and tensor memory (one sample per CTA is the smallest tile any batch size can get)
+            const int pad = op.ksize / 2;
+            const bool geom = op.ksize % 2 == 1 && op.ksize <= 5 && op.ncb0 <= 256 && op.ncb1 <= 256 && op.W + 2 * pad <= 256 &&
+                              op.H + 2 * pad <= 256;
+            ConvUmmaParams p;
+            ConvShape cs{op.name.c_str(), op.H, op.W, op.ksize, op.ncb0, op.ncb1, op.cout, op.n_tile};
+            if (!geom || plan_umma(cs, 1, p) != FLO_OK) {
+                set_error("conv '%s' (%dx%d, k=%d, cin=%d+%d, cout=%d) has no kernel on %s: k_conv_umma needs whole 16-channel K "
+                          "slices, an odd window up to 5x5, at most 256 padded pixels per row / column and 256 channel blocks per "
+                          "source, and a tile within 227 KB of shared memory", op.name.c_str(), op.H, op.W, op.ksize, op.ncb0 * 8,
+                          op.ncb1 * 8, op.cout, path);
+                return FLO_ERR_UNSUPPORTED;
+            }
+        }
     }
     return FLO_OK;
 }
@@ -753,7 +781,7 @@ int plan_umma(const ConvShape& op, int B, ConvUmmaParams& p) {
         const int max_mt = std::max(1, std::min(4, 256 / op.n_tile));   // <= 256 TMEM columns: two CTAs per SM
         int best_nb = 1; double best_cost = 1e30;
         for (int nb = 1; nb <= 64; ++nb) {
-            const int rows = nb * PP - 2 * (pad ? Wp + 1 : 0);
+            const int rows = nb * PP - 2 * pad * (Wp + 1);
             const int mt = (rows + 127) / 128;
             if (mt > max_mt) break;
             const size_t a_bytes = (size_t)ncbT * nb * PP * 16;
@@ -764,9 +792,9 @@ int plan_umma(const ConvShape& op, int B, ConvUmmaParams& p) {
             if (cost <= best_cost + 1e-9) { best_cost = cost; best_nb = nb; }   // ties: more samples per weight fetch
         }
         p.nb = best_nb;
-        const int rows = p.nb * PP - 2 * (pad ? Wp + 1 : 0);
+        const int rows = p.nb * PP - 2 * pad * (Wp + 1);     // first to last valid padded pixel
         p.n_mtiles = (rows + 127) / 128;
-        p.sbo_px = 8; p.row0 = pad ? Wp + 1 : 0; p.tile_stride = 128;
+        p.sbo_px = 8; p.row0 = pad * (Wp + 1); p.tile_stride = 128;
     }
     p.plane_px = p.nb * PP;
     const int total_slices = taps * (ncbT / 2);
@@ -815,6 +843,8 @@ static int launch_op(Handle& h, Plan& pl, int i, cudaStream_t st) {
                 ConvUmmaParams p = pl.umma[i];
                 p.w = h.d_bf16 + op.w_umma; p.bias = f32c(op.bias); p.res = (const float*)ptr(op.res);
                 p.out_m = (float*)ptr(op.out_m); p.out_o = (__nv_bfloat16*)ptr(op.out_o);
+                p.act_silu = op.act_silu; p.out_un = (__nv_bfloat16*)ptr(op.out_un); p.out_up = (__nv_bfloat16*)ptr(op.out_up);
+                if (op.need_mode) { p.mask_mode = pl.mask_mode; p.need_mode = op.need_mode; p.bypass = (const float*)ptr(op.bypass); }
                 e = launch_conv_umma(p, pl.tmA0[i], pl.tmA1[i], st);
             } else {
                 ConvSimtParams p{};
@@ -1178,7 +1208,8 @@ int flo_unet_set_mask(flo_unet_t* hh, const float* mask, int B, void* stream) {
     if (rc) return rc;
     MaskPrepParams mp{};
     mp.mask = mask; mp.n_levels = s.n_levels; mp.B = B; mp.ch = s.channels; mp.H = s.H; mp.W = s.W; mp.mode = pl->mask_mode;
-    for (int l = 0; l < s.n_levels; ++l) mp.out[l] = (float*)pl->buf_ptr[h->mask_buf[l]];
+    mp.out_bf16 = s.bf16;
+    for (int l = 0; l < s.n_levels; ++l) mp.out[l] = pl->buf_ptr[h->mask_buf[l]];
     CUDA_TRY(launch_mask_prep(mp, st));
     h->launches += mask ? 2 : 1;
     return FLO_OK;

@@ -1,13 +1,13 @@
 // Implicit-GEMM convolution on the 5th-generation tensor cores (tcgen05 / TMEM / TMA), sm_100a.
 //
-// GEMM view of a 1x1 / 3x3 (pad 1) convolution over blocked bf16 activations:
+// GEMM view of a k x k (k = 1, 3 or 5, pad k/2) convolution over blocked bf16 activations:
 //     D[pixel, cout] = sum_{tap, cin} A_tap[pixel, cin] * W[tap, cin, cout]
 // * A operand: ONE TMA tensor-tile load per source brings the zero-padded image tile of `nb`
-//   samples -- box {8ch, W+2, H+2, nb, C/8} at coordinates (0,-1,-1,b0,0), out-of-bounds = 0 --
-//   into shared memory as [C/8][nb][H+2][W+2][8ch].  That is exactly the tcgen05 no-swizzle
-//   K-major operand layout (16-byte rows, 8-row core matrices): the A tile of a 3x3 tap is the
-//   SAME bytes at a start address shifted by (dh*(W+2)+dw)*16 B, so im2col costs no data
-//   movement at all -- nine descriptors instead of nine copies.  torch.cat of two sources is two
+//   samples -- box {8ch, W+2p, H+2p, nb, C/8} at coordinates (0,-p,-p,b0,0), out-of-bounds = 0 --
+//   into shared memory as [C/8][nb][H+2p][W+2p][8ch].  That is exactly the tcgen05 no-swizzle
+//   K-major operand layout (16-byte rows, 8-row core matrices): the A tile of a tap is the
+//   SAME bytes at a start address shifted by (dh*(W+2p)+dw)*16 B, so im2col costs no data
+//   movement at all -- k*k descriptors instead of k*k copies.  torch.cat of two sources is two
 //   TMA loads into consecutive planes (two K segments).
 // * M tile = 128 output pixels = 16 groups of 8 consecutive padded pixels.  At 16x16 a tile is a
 //   16-row x 8-column strip (group stride = padded row pitch, every row useful); at lower
@@ -17,8 +17,11 @@
 //   through a ring of shared-memory stages by 1-D bulk TMA copies (cp.async.bulk, mbarrier tx).
 // * D: fp32 accumulators in TMEM (one 128 x n_tile block per M tile); tcgen05.mma issued by one thread;
 //   tcgen05.commit -> mbarrier hands stages back to the producer and the result to the epilogue.
-// * Epilogue: 4 warps tcgen05.ld their 32 TMEM lanes, add bias (+ fp32 residual), and write fp32
-//   and/or bf16 blocked outputs with 32-/16-byte vector stores.
+// * Epilogue: 4 warps tcgen05.ld their 32 TMEM lanes, add bias (then SiLU, then the fp32 residual), and write fp32
+//   and/or bf16 blocked outputs with 32-/16-byte vector stores, plus the pixel-unshuffled / nearest-x2 bf16 copies the
+//   inpainting mask fusions hand to the next Downsample / Upsample conv.
+// * Mask branches switched off at run time (*mask_mode < need_mode) do no MMA: the CTA copies the bypass tensor to every
+//   output, or returns when there is none.  The flag is uniform over the grid, so one captured graph serves every mode.
 //
 // Warp roles (192 threads): warps 0-3 epilogue, warp 4 TMA producer, warp 5 TMEM owner + MMA issuer.
 #include <cuda_fp16.h>
@@ -39,24 +42,85 @@ struct ConvGeom {
 };
 __device__ __forceinline__ int tile_row0(const ConvUmmaParams& p, int t) {
     if (p.sbo_px != 8) {            // strip mode: tile = 16 image rows x 8 columns
+        const int pad = p.ksize >> 1;
         const int tx_n = p.W >> 3;
         const int ty = t / tx_n, tx = t % tx_n;
-        return (ty * 16 + 1) * (p.W + 2) + 1 + 8 * tx;
+        return (ty * 16 + pad) * (p.W + 2 * pad) + pad + 8 * tx;
     }
     return p.row0 + t * p.tile_stride;
+}
+
+// Pixels of shared memory past the A planes that a tile may address: the last M tile's rows run up to 127 pixels past the
+// plane, and a tap shifts by up to pad*(Wp+1).  (1x1 keeps the 3x3 slack.)
+__host__ __device__ __forceinline__ uint32_t a_slack_px(int pad, int Wp) {
+    return 128u + (uint32_t)((pad > 1 ? pad : 1) * (Wp + 1) + 1);
+}
+
+// bf16 copies of one 8-channel pixel vector of a [cout/8][B][H][W][8] output: pixel-unshuffled ('b c (h p1) (w p2) ->
+// b (c p1 p2) h w' in our (p1 p2 c) channel order, as k_gn writes it) and nearest x2
+__device__ __forceinline__ void store_un_up(const ConvUmmaParams& p, int cb, int b, int h, int w, uint4 u) {
+    const int HW = p.H * p.W;
+    if (p.out_un) {
+        const int plane = ((h & 1) * 2 + (w & 1)) * (p.cout >> 3) + cb;
+        const int q = (h >> 1) * (p.W >> 1) + (w >> 1);
+        *reinterpret_cast<uint4*>(p.out_un + ((size_t)(plane * p.B + b) * (HW >> 2) + q) * 8) = u;
+    }
+    if (p.out_up) {
+        const int W2 = p.W * 2;
+#pragma unroll
+        for (int d = 0; d < 4; ++d) {
+            const int q = (2 * h + (d >> 1)) * W2 + 2 * w + (d & 1);
+            *reinterpret_cast<uint4*>(p.out_up + ((size_t)(cb * p.B + b) * (HW * 4) + q) * 8) = u;
+        }
+    }
+}
+__device__ __forceinline__ uint4 pack_bf16x8(const float* o) {
+    uint4 u;
+    __nv_bfloat162* h2 = reinterpret_cast<__nv_bfloat162*>(&u);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) h2[q] = __floats2bfloat162_rn(o[2 * q], o[2 * q + 1]);
+    return u;
+}
+
+// a mask branch switched off at run time: this CTA's samples and output channels are the bypass tensor
+__device__ __forceinline__ void conv_umma_bypass(const ConvUmmaParams& p) {
+    const int HW = p.H * p.W, ncb = p.n_tile >> 3;
+    const int b0 = blockIdx.x * p.nb, nbh = min(p.nb, p.B - b0);
+    const int cb0 = (blockIdx.y * p.n_tile) >> 3;
+    const int n = nbh * HW * ncb;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const int px = i % HW, r = i / HW, s = r % nbh, cb = cb0 + r / nbh, b = b0 + s;
+        const size_t off = ((size_t)(cb * p.B + b) * HW + px) * 8;
+        const float4 v0 = *reinterpret_cast<const float4*>(p.bypass + off);
+        const float4 v1 = *reinterpret_cast<const float4*>(p.bypass + off + 4);
+        if (p.out_m) {
+            *reinterpret_cast<float4*>(p.out_m + off) = v0;
+            *reinterpret_cast<float4*>(p.out_m + off + 4) = v1;
+        }
+        const float o[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
+        const uint4 u = pack_bf16x8(o);
+        if (p.out_o) *reinterpret_cast<uint4*>(p.out_o + off) = u;
+        const int h = px / p.W;
+        store_un_up(p, cb, b, h, px - h * p.W, u);
+    }
 }
 
 __global__ void __launch_bounds__(UMMA_THREADS) k_conv_umma(const __grid_constant__ CUtensorMap tmA0,
                                                             const __grid_constant__ CUtensorMap tmA1,
                                                             const ConvUmmaParams p) {
     extern __shared__ __align__(128) uint8_t smem[];
+    // run-time mask mode: read once, before any barrier or tensor memory exists (uniform over the grid)
+    if (p.mask_mode && *p.mask_mode < p.need_mode) {
+        if (p.bypass) conv_umma_bypass(p);
+        return;
+    }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int ncbT = p.ncb0 + p.ncb1;
     const int pad = p.ksize >> 1;
     const int Wp = p.W + 2 * pad, Hp = p.H + 2 * pad, PP = Wp * Hp;
     const uint32_t plane_bytes = (uint32_t)p.plane_px * 16u;
     const uint32_t a_bytes = (uint32_t)ncbT * plane_bytes;
-    const uint32_t a_region = (a_bytes + (uint32_t)(128 + Wp + 2) * 16u + 127u) & ~127u;
+    const uint32_t a_region = (a_bytes + a_slack_px(pad, Wp) * 16u + 127u) & ~127u;
     const uint32_t stage_bytes = (uint32_t)p.slices_per_stage * (uint32_t)p.n_tile * 32u;
     const uint32_t ring_off = a_region;
     const uint32_t bar_off = ring_off + (uint32_t)p.n_wstages * stage_bytes;
@@ -120,7 +184,7 @@ __global__ void __launch_bounds__(UMMA_THREADS) k_conv_umma(const __grid_constan
                 for (int s = 0; s < p.slices_per_stage; ++s) {
                     const int ks = i * p.slices_per_stage + s;
                     const int tap = ks / cpT, cp = ks - tap * cpT;
-                    const int shift = pad ? ((tap / 3 - 1) * Wp + (tap % 3 - 1)) : 0;
+                    const int shift = pad ? ((tap / p.ksize - pad) * Wp + (tap % p.ksize - pad)) : 0;
                     const uint64_t bdesc = make_smem_desc(bstage + (uint32_t)s * (uint32_t)p.n_tile * 32u, b_lbo, 128u);
                     for (int t = 0; t < p.n_mtiles; ++t) {
                         const uint32_t a_addr =
@@ -146,9 +210,9 @@ __global__ void __launch_bounds__(UMMA_THREADS) k_conv_umma(const __grid_constan
             bool valid;
             int px;
             if (pad) {
-                const int hh = rem / Wp, ww = rem - hh * Wp;
-                valid = (s < p.nb) && (hh >= 1) && (hh <= p.H) && (ww >= 1) && (ww <= p.W);
-                px = (hh - 1) * p.W + (ww - 1);
+                const int hh = rem / Wp - pad, ww = rem % Wp - pad;
+                valid = (s < p.nb) && (hh >= 0) && (hh < p.H) && (ww >= 0) && (ww < p.W);
+                px = hh * p.W + ww;
             } else {
                 valid = (s < p.nb);
                 px = rem;
@@ -171,6 +235,10 @@ __global__ void __launch_bounds__(UMMA_THREADS) k_conv_umma(const __grid_constan
                         o[0] += b0v.x; o[1] += b0v.y; o[2] += b0v.z; o[3] += b0v.w;
                         o[4] += b1v.x; o[5] += b1v.y; o[6] += b1v.z; o[7] += b1v.w;
                     }
+                    if (p.act_silu) {           // nn.SiLU of the mask-fusion convs, in k_conv_simt's IEEE form
+#pragma unroll
+                        for (int j = 0; j < 8; ++j) o[j] = o[j] / (1.0f + expf(-o[j]));
+                    }
                     const size_t off = ((size_t)((cc >> 3) * p.B + b) * HW + px) * 8;
                     if (p.res) {
                         const float4 r0 = *reinterpret_cast<const float4*>(p.res + off);
@@ -182,12 +250,13 @@ __global__ void __launch_bounds__(UMMA_THREADS) k_conv_umma(const __grid_constan
                         *reinterpret_cast<float4*>(p.out_m + off) = make_float4(o[0], o[1], o[2], o[3]);
                         *reinterpret_cast<float4*>(p.out_m + off + 4) = make_float4(o[4], o[5], o[6], o[7]);
                     }
-                    if (p.out_o) {
-                        uint4 u;
-                        __nv_bfloat162* h2 = reinterpret_cast<__nv_bfloat162*>(&u);
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) h2[q] = __floats2bfloat162_rn(o[2 * q], o[2 * q + 1]);
-                        *reinterpret_cast<uint4*>(p.out_o + off) = u;
+                    if (p.out_o || p.out_un || p.out_up) {
+                        const uint4 u = pack_bf16x8(o);
+                        if (p.out_o) *reinterpret_cast<uint4*>(p.out_o + off) = u;
+                        if (p.out_un || p.out_up) {
+                            const int h = px / p.W;
+                            store_un_up(p, cc >> 3, b, h, px - h * p.W, u);
+                        }
                     }
                 }
             }
@@ -213,7 +282,7 @@ int conv_umma_smem_bytes(const ConvUmmaParams& p) {
     const int pad = p.ksize >> 1, Wp = p.W + 2 * pad;
     const uint32_t plane_bytes = (uint32_t)p.plane_px * 16u;
     const uint32_t a_bytes = (uint32_t)(p.ncb0 + p.ncb1) * plane_bytes;
-    const uint32_t a_region = (a_bytes + (uint32_t)(128 + Wp + 2) * 16u + 127u) & ~127u;
+    const uint32_t a_region = (a_bytes + a_slack_px(pad, Wp) * 16u + 127u) & ~127u;
     const uint32_t stage_bytes = (uint32_t)p.slices_per_stage * (uint32_t)p.n_tile * 32u;
     return (int)(a_region + p.n_wstages * stage_bytes + 16 * MAX_WSTAGES + 16 + 16);
 }

@@ -96,12 +96,15 @@ struct ConvSimtParams {
     const float* bypass;                // ... else out = bypass (fp32 blocked, same shape), or nothing is written if null
 };
 
-// cond['mask_cond'] [B,ch,H,W] (NCHW fp32) -> one blocked 8-channel fp32 tensor per resolution level (bilinear,
-// F.interpolate(..., mode='bilinear'), unet.py:338,362) + the "mask in use" flag (unet.py:301 torch.allclose)
+// cond['mask_cond'] [B,ch,H,W] (NCHW fp32) -> one blocked mask tensor per resolution level (bilinear,
+// F.interpolate(..., mode='bilinear'), unet.py:338,362) + the "mask in use" flag (unet.py:301 torch.allclose).
+// fp32 path: 8 fp32 channels [1][B][h][w][8]; 16-bit path: 16 bf16 channels [2][B][h][w][8] whose second block is zero, so a
+// (dim + 16)-channel concatenation is a whole number of tcgen05 K16 slices.
 struct MaskPrepParams {
     const float* mask;
-    float* out[8];
+    void* out[8];
     int n_levels, B, ch, H, W;
+    int out_bf16;
     int* mode;
 };
 
@@ -165,7 +168,7 @@ struct ConvUmmaParams {
     int ncb0, ncb1;              // channel blocks of the two (concatenated) sources
     int cout;                    // total output channels
     int n_tile;                  // output channels per CTA (multiple of 16, <= 256)
-    int ksize;                   // 1 or 3
+    int ksize;                   // odd, <= 5 (pad = ksize / 2)
     int nb;                      // samples per CTA
     int n_mtiles;                // 128-row M tiles per CTA
     int row0;                    // flattened (padded) pixel index of row 0 of M tile 0
@@ -176,6 +179,14 @@ struct ConvUmmaParams {
     int n_wstages;               // ring depth
     int smem_bytes;
     int tmem_cols;
+    // inpainting mask branches, as in ConvSimtParams: out = res + SiLU(conv + bias), the pixel-unshuffled / nearest-x2
+    // bf16 copies, and the run-time bypass (all zero / null for every other conv)
+    int act_silu;
+    __nv_bfloat16* out_un;       // [4*cout/8][B][H/2][W/2][8] in (p1 p2 c) channel order, or null
+    __nv_bfloat16* out_up;       // [cout/8][B][2H][2W][8], or null
+    const int* mask_mode;        // device flag (0 no mask, 1 mask all ones, 2 mask in use), or null
+    int need_mode;               // the op runs when *mask_mode >= need_mode ...
+    const float* bypass;         // ... else every output is the bypass tensor (fp32 blocked), or nothing is written if null
 };
 
 // ---------------------------------------------------------------------------------------------

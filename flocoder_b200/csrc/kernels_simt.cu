@@ -805,12 +805,13 @@ cudaError_t launch_gn_any(const GnParams& p, cudaStream_t s) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// inpainting mask: NCHW fp32 [B,ch,H,W] -> per-level blocked 8-channel tensors (channels >= ch are zero) by the
-// bilinear rule of F.interpolate(mask, size=(h,w), mode='bilinear') (align_corners=False, no antialias; unet.py:338,362):
+// inpainting mask: NCHW fp32 [B,ch,H,W] -> per-level blocked tensors (channels >= ch are zero): 8 fp32 channels, or on the
+// 16-bit path 16 bf16 channels (the second 8-channel block all zero), rounded only at the store.  Bilinear rule of F.interpolate(mask, size=(h,w), mode='bilinear') (align_corners=False, no antialias; unet.py:338,362):
 // src = (dst + 0.5) * in/out - 0.5 clamped at 0, i1 = min(i0 + 1, in - 1).  Level 0 is a copy and also evaluates the
 // reference's bypass test torch.allclose(mask, 1) (unet.py:301: |m - 1| <= 1e-8 + 1e-5): *mode = 2 if any element fails.
 // ------------------------------------------------------------------------------------------------
 __global__ void k_mask_mode(int* mode, int value) { if (threadIdx.x == 0 && blockIdx.x == 0) *mode = value; }
+template <typename TO>
 __global__ void __launch_bounds__(128) k_mask_prep(MaskPrepParams p) {
     const int lvl = blockIdx.y, h = p.H >> lvl, w = p.W >> lvl, hw = h * w;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -840,14 +841,21 @@ __global__ void __launch_bounds__(128) k_mask_prep(MaskPrepParams p) {
             }
         }
     }
-    store8(p.out[lvl] + ((size_t)b * hw + px) * 8, o);
+    TO* out = reinterpret_cast<TO*>(p.out[lvl]);
+    store8(out + ((size_t)b * hw + px) * 8, o);
+    if (std::is_same<TO, __nv_bfloat16>::value) {            // zero block: channels 8..15 of the K16 slice
+#pragma unroll
+        for (int c = 0; c < 8; ++c) o[c] = 0.f;
+        store8(out + ((size_t)(p.B + b) * hw + px) * 8, o);
+    }
     if (not_ones) atomicMax(p.mode, 2);
 }
 cudaError_t launch_mask_prep(const MaskPrepParams& p, cudaStream_t s) {
     k_mask_mode<<<1, 32, 0, s>>>(p.mode, p.mask ? 1 : 0);
     if (p.mask) {
         dim3 grid((p.B * p.H * p.W + 127) / 128, p.n_levels);
-        k_mask_prep<<<grid, 128, 0, s>>>(p);
+        if (p.out_bf16) k_mask_prep<__nv_bfloat16><<<grid, 128, 0, s>>>(p);
+        else k_mask_prep<float><<<grid, 128, 0, s>>>(p);
     }
     return cudaGetLastError();
 }

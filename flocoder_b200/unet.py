@@ -85,7 +85,8 @@ class Unet(nn.Module):
     def __init__(self, dim, dim_mults=(1, 2, 4, 8), channels=3, resnet_block_groups=4,
                  n_classes=10, mask_cond=False, use_checkpoint=False, compute_dtype: Optional[str] = None):
         super().__init__()
-        self.mask_cond = bool(mask_cond)              # inpainting U-Net (unet.py:214-235): fp32 kernels only
+        self.mask_cond = bool(mask_cond)              # inpainting U-Net (unet.py:214-235): fp32 kernels, or bf16 with
+                                                      # engine_flags = FLO_FLAG_LAYERWISE
         self.use_checkpoint = use_checkpoint          # accepted for signature parity; inference only
         self.dim = dim
         self.dim_mults = tuple(int(m) for m in dim_mults)

@@ -44,7 +44,8 @@ extern "C" {
 typedef enum flo_status {
     FLO_OK = 0,
     FLO_ERR_INVALID = -1,     /* bad argument (ValueError in Python) */
-    FLO_ERR_UNSUPPORTED = -2, /* feature outside the built path, e.g. mask_cond with a 16-bit compute type (NotImplementedError) */
+    FLO_ERR_UNSUPPORTED = -2, /* feature outside the built path, e.g. mask_cond with FLO_F16, or with FLO_BF16 without
+                                 FLO_FLAG_LAYERWISE (NotImplementedError) */
     FLO_ERR_CUDA = -3,        /* CUDA runtime / driver failure (RuntimeError) */
     FLO_ERR_NOMEM = -4,
     FLO_ERR_STEP = -5         /* adaptive integrator: step size below the minimum step, or max_steps used up (RuntimeError) */
@@ -81,7 +82,8 @@ typedef struct flo_unet_cfg {
     int32_t compute_dtype; /* flo_dtype: FLO_F32 = fp32 CUDA-core path (<=1e-5 parity),
                               FLO_BF16 / FLO_F16 = 16-bit tcgen05 operands, fp32 accumulate */
     int32_t mask_cond;     /* Unet(mask_cond=...): 1 builds the inpainting U-Net with its mask-fusion branches
-                              (unet.py:214-235); FLO_F32 only */
+                              (unet.py:214-235); FLO_F32, or FLO_BF16 with FLO_FLAG_LAYERWISE and dim % 16 == 0
+                              (the fused stage kernels have no mask branches) */
     int32_t flags;         /* FLO_FLAG_*                            */
     int32_t device;        /* CUDA device ordinal                   */
 } flo_unet_cfg;

@@ -30,7 +30,8 @@ EXPORTS = (
     "flo_integrate_nfe", "flo_unet_num_ops", "flo_unet_op_name", "flo_unet_launches_per_forward",
     "flo_unet_launch_count", "flo_unet_read_activation", "flo_selftest_umma", "flo_describe_plan",
     "flo_unet_op_info", "flo_unet_profile_ops", "flo_unet_read_timeline", "flo_unet_set_mask",
-    "flo_integrate_rk45", "flo_integrate_rk45_timing", "flo_integrate_rk45_per_sample",
+    "flo_integrate_rk45", "flo_integrate_rk45_timing", "flo_integrate_rk45_per_sample", "flo_integrate_rk45_reverse",
+    "flo_integrate_rk45_per_sample_reverse",
 )
 
 
@@ -73,10 +74,12 @@ def lib() -> ctypes.CDLL:
     L.flo_unet_set_mask.argtypes = [c_void_p, c_void_p, c_int, c_void_p]
     L.flo_integrate_rk45.argtypes = [c_void_p, c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                                      ctypes.c_double, c_float, c_void_p, c_float, c_int, POINTER(c_int), c_int, c_void_p]
+    L.flo_integrate_rk45_reverse.argtypes = L.flo_integrate_rk45.argtypes
     L.flo_integrate_rk45_timing.argtypes = [c_void_p, POINTER(ctypes.c_double)]
     L.flo_integrate_rk45_per_sample.argtypes = [c_void_p, c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                                                 ctypes.c_double, c_float, c_void_p, c_float, c_int, POINTER(ctypes.c_int32),
                                                 c_int, c_void_p]
+    L.flo_integrate_rk45_per_sample_reverse.argtypes = L.flo_integrate_rk45_per_sample.argtypes
     L.flo_integrate_nfe.argtypes = [c_int, c_int]
     L.flo_unet_num_ops.argtypes = [c_void_p]
     L.flo_unet_op_name.argtypes = [c_void_p, c_int, c_char_p, c_int]
@@ -260,40 +263,45 @@ class Engine:
         return y
 
     def integrate_rk45(self, y: torch.Tensor, t0: float, t1: float = 1.0, rtol: float = 1e-5, atol: float = 1e-5,
-                       t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0, max_steps: int = 10000):
+                       t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0, max_steps: int = 10000,
+                       reverse: bool = False):
         """Adaptive Dormand-Prince 5(4) from ``t0`` to ``t1`` in place on ``y`` (``flo_integrate_rk45``: scipy's RK45 step
         control on the device, one host wait per attempt).  Returns ``(nfev, accepted, rejected)``; raises RuntimeError
-        when the step size collapses or ``max_steps`` attempts do not reach ``t1``."""
+        when the step size collapses or ``max_steps`` attempts do not reach ``t1``.  ``reverse=True`` integrates backwards
+        from ``t0`` down to ``t1 < t0`` (``flo_integrate_rk45_reverse``)."""
         assert y.dtype == torch.float32 and y.is_contiguous() and y.device == self.device
         b = y.shape[0]
         keep, cptr = self._cls_ptr(class_ids, b)
         counts = (c_int * 3)()
+        fn = "flo_integrate_rk45_reverse" if reverse else "flo_integrate_rk45"
         with torch.cuda.device(self.device):
-            check(self.L.flo_integrate_rk45(self.handle, y.data_ptr(), float(t0), float(t1), float(rtol), float(atol),
-                                            float(t_scale), cptr, float(cfg_strength), int(max_steps), counts, b,
-                                            _stream_ptr(self.device)), "flo_integrate_rk45")
+            check(getattr(self.L, fn)(self.handle, y.data_ptr(), float(t0), float(t1), float(rtol), float(atol),
+                                      float(t_scale), cptr, float(cfg_strength), int(max_steps), counts, b,
+                                      _stream_ptr(self.device)), fn)
         return counts[0], counts[1], counts[2]
 
     def integrate_rk45_per_sample(self, y: torch.Tensor, t0: float, t1: float = 1.0, rtol: float = 1e-5,
                                   atol: float = 1e-5, t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0,
-                                  max_steps: int = 10000) -> torch.Tensor:
+                                  max_steps: int = 10000, reverse: bool = False) -> torch.Tensor:
         """As :meth:`integrate_rk45`, but every sample is its own RK45 problem with its own step-size control
-        (``flo_integrate_rk45_per_sample``).  Returns the CPU int64 tensor ``[B, 3]`` of per-sample
-        ``(nfev, accepted, rejected)``; raises RuntimeError naming the sample when one fails."""
+        (``flo_integrate_rk45_per_sample``, or ``flo_integrate_rk45_per_sample_reverse`` with ``reverse=True``).
+        Returns the CPU int64 tensor ``[B, 3]`` of per-sample ``(nfev, accepted, rejected)``; raises RuntimeError naming
+        the sample when one fails."""
         assert y.dtype == torch.float32 and y.is_contiguous() and y.device == self.device
         b = y.shape[0]
         keep, cptr = self._cls_ptr(class_ids, b)
         counts = (ctypes.c_int32 * (3 * b))()
+        fn = "flo_integrate_rk45_per_sample_reverse" if reverse else "flo_integrate_rk45_per_sample"
         with torch.cuda.device(self.device):
-            check(self.L.flo_integrate_rk45_per_sample(self.handle, y.data_ptr(), float(t0), float(t1), float(rtol),
-                                                       float(atol), float(t_scale), cptr, float(cfg_strength),
-                                                       int(max_steps), counts, b, _stream_ptr(self.device)),
-                  "flo_integrate_rk45_per_sample")
+            check(getattr(self.L, fn)(self.handle, y.data_ptr(), float(t0), float(t1), float(rtol), float(atol),
+                                      float(t_scale), cptr, float(cfg_strength), int(max_steps), counts, b,
+                                      _stream_ptr(self.device)), fn)
         return torch.tensor(list(counts), dtype=torch.int64).reshape(b, 3)
 
     def rk45_timing(self):
         """(attempts, host wall ms, attempt-graph device ms) of the last :meth:`integrate_rk45` or
-        :meth:`integrate_rk45_per_sample` call (per-sample: attempts of the whole batch, the most any sample made)."""
+        :meth:`integrate_rk45_per_sample` call, either direction (per-sample: attempts of the whole batch, the most any
+        sample made)."""
         out = (ctypes.c_double * 3)()
         check(self.L.flo_integrate_rk45_timing(self.handle, out), "flo_integrate_rk45_timing")
         return int(out[0]), out[1], out[2]

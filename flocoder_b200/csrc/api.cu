@@ -1461,11 +1461,13 @@ static int ensure_rk45(Handle& h, Plan& fp, cudaStream_t st) {
     return FLO_OK;
 }
 
-// argument checks of both RK45 entry points: they need neither a handle nor a device
-static int rk45_check_args(double t0, double t1, double rtol, double atol, int max_steps) {
+// argument checks of the RK45 entry points: they need neither a handle nor a device.  direction = +1: the forward exports
+// (t0 < t1), -1: the _reverse ones (t1 < t0).
+static int rk45_check_args(double t0, double t1, double rtol, double atol, int max_steps, int direction) {
     if (!(rtol > 0)) { set_error("rtol must be > 0, got %g", rtol); return FLO_ERR_INVALID; }
     if (!(atol >= 0)) { set_error("atol must be >= 0, got %g", atol); return FLO_ERR_INVALID; }
-    if (!(t1 > t0) || !isfinite(t0) || !isfinite(t1)) { set_error("need finite t0 < t1, got t0=%g t1=%g", t0, t1); return FLO_ERR_INVALID; }
+    if (direction > 0 && (!(t1 > t0) || !isfinite(t0) || !isfinite(t1))) { set_error("need finite t0 < t1, got t0=%g t1=%g", t0, t1); return FLO_ERR_INVALID; }
+    if (direction < 0 && (!(t1 < t0) || !isfinite(t0) || !isfinite(t1))) { set_error("need finite t1 < t0, got t0=%g t1=%g", t0, t1); return FLO_ERR_INVALID; }
     if (max_steps < 1) { set_error("max_steps must be >= 1, got %d", max_steps); return FLO_ERR_INVALID; }
     return FLO_OK;
 }
@@ -1487,9 +1489,11 @@ static int rk45_route(Handle& h, int B, bool use_cfg, cudaStream_t st, Plan** fp
     return FLO_OK;
 }
 
-int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
-                       const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream) {
-    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps);
+// flo_integrate_rk45 (direction +1) and flo_integrate_rk45_reverse (-1)
+static int integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                          const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream,
+                          int direction) {
+    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps, direction);
     if (rc) return rc;
     Handle* h = reinterpret_cast<Handle*>(hh);
     if (!h || !y || !counts) { set_error("NULL argument"); return FLO_ERR_INVALID; }
@@ -1526,6 +1530,7 @@ int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rt
     CUDA_TRY(launch_setup_ctrl(fp->ctrl, c, nullptr, nullptr, st));
     Rk45Ctl r{};
     r.t = t0; r.t_new = t0; r.t1 = t1; r.rtol = rtol; r.atol = atol; r.max_step = INFINITY; r.interval = fabs(t1 - t0);
+    r.direction = direction;
     r.t_scale = t_scale; r.max_steps = max_steps; r.k0 = 0; r.two_pass = two_pass; r.flags = flags;
     r.status.state = RK_RUNNING; r.status.t = t0;
     CUDA_TRY(launch_rk45_setup(fp->rk_ctl, r, fp->ctrl, st));
@@ -1638,10 +1643,11 @@ static int ensure_rk45_per_sample(Handle& h, Plan& fp, cudaStream_t st) {
     return FLO_OK;
 }
 
-int flo_integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
-                                  const int64_t* class_ids, float cfg_strength, int max_steps, int32_t* counts, int B,
-                                  void* stream) {
-    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps);
+// flo_integrate_rk45_per_sample (direction +1) and flo_integrate_rk45_per_sample_reverse (-1)
+static int integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol,
+                                     float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps,
+                                     int32_t* counts, int B, void* stream, int direction) {
+    int rc = rk45_check_args(t0, t1, rtol, atol, max_steps, direction);
     if (rc) return rc;
     Handle* h = reinterpret_cast<Handle*>(hh);
     if (!h || !y || !counts) { set_error("NULL argument"); return FLO_ERR_INVALID; }
@@ -1684,6 +1690,7 @@ int flo_integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1
     CUDA_TRY(launch_setup_ctrl(fp->ctrl, c, nullptr, nullptr, st));
     Rk45Ctl r{};
     r.t = t0; r.t_new = t0; r.t1 = t1; r.rtol = rtol; r.atol = atol; r.max_step = INFINITY; r.interval = fabs(t1 - t0);
+    r.direction = direction;
     r.t_scale = t_scale; r.max_steps = max_steps; r.k0 = 0; r.two_pass = two_pass; r.flags = flags;
     r.status.state = RK_RUNNING; r.status.t = t0;
     CUDA_TRY(launch_rk45ps_setup(rp, r, st));
@@ -1782,6 +1789,31 @@ int flo_integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1
     CUDA_TRY(cudaMemcpyAsync(y, rp.ybuf, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return FLO_OK;
+}
+
+int flo_integrate_rk45(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                       const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream) {
+    return integrate_rk45(hh, y, t0, t1, rtol, atol, t_scale, class_ids, cfg_strength, max_steps, counts, B, stream, 1);
+}
+
+int flo_integrate_rk45_reverse(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                               const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B,
+                               void* stream) {
+    return integrate_rk45(hh, y, t0, t1, rtol, atol, t_scale, class_ids, cfg_strength, max_steps, counts, B, stream, -1);
+}
+
+int flo_integrate_rk45_per_sample(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol, float t_scale,
+                                  const int64_t* class_ids, float cfg_strength, int max_steps, int32_t* counts, int B,
+                                  void* stream) {
+    return integrate_rk45_per_sample(hh, y, t0, t1, rtol, atol, t_scale, class_ids, cfg_strength, max_steps, counts, B,
+                                     stream, 1);
+}
+
+int flo_integrate_rk45_per_sample_reverse(flo_unet_t* hh, float* y, double t0, double t1, double rtol, double atol,
+                                          float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps,
+                                          int32_t* counts, int B, void* stream) {
+    return integrate_rk45_per_sample(hh, y, t0, t1, rtol, atol, t_scale, class_ids, cfg_strength, max_steps, counts, B,
+                                     stream, -1);
 }
 
 int flo_integrate_rk45_timing(flo_unet_t* hh, double out[3]) {

@@ -352,6 +352,7 @@ struct Rk45Ctl {              // device-resident controller state (scipy RungeKu
     int k0;                   // physical K slot holding K[0] (0 or 6); K[6] is in 6 - k0
     int two_pass;             // 1: conditional + combining pass per evaluation (12 stage entries per attempt)
     int flags;                // Stage::flags of the evaluation's (last) pass: 0, SF_CFG_2B or SF_CFG_COMBINE
+    int direction;            // sign(t1 - t0): +1 integrates forward, -1 backward (scipy's OdeSolver.direction)
     unsigned arrive;          // k_rk45_end arrival counter (zero between launches)
     Rk45Status status;
 };

@@ -9,6 +9,10 @@
 //
 // One ODE system for the whole batch: the flattened [B,C,H,W] state has one step size and the RMS norm runs over all
 // B*C*H*W elements, so a sample's trajectory depends on the rest of its batch (as solve_ivp on y0.ravel()).
+//
+// Both directions: Rk45Ctl::direction = sign(t1 - t0) enters where scipy's OdeSolver.direction does (the signed step, the
+// clip to t1, min_step, the end test, the trial point of select_initial_step).  It is an int, +1 or -1: converted to double
+// it multiplies exactly, so the forward solve is bit-identical to a controller without it.
 #include <math.h>
 
 #include "umma_common.cuh"
@@ -35,14 +39,14 @@ constexpr double RK_ERR_EXP = -1.0 / (4 + 1);        // error_exponent = -1 / (e
 __host__ __device__ inline void rk45_begin_attempt(Rk45Ctl& c) {
     if (c.h_abs < c.min_step) { c.status.state = RK_TOO_SMALL; return; }
     if (c.attempts >= c.max_steps) { c.status.state = RK_TOO_MANY; return; }
-    double t_new = c.t + c.h_abs;                   // direction = +1 (t1 > t0)
-    if (t_new - c.t1 > 0) t_new = c.t1;
+    double t_new = c.t + c.h_abs * c.direction;     // h = h_abs * direction; exact for direction = +-1
+    if (c.direction * (t_new - c.t1) > 0) t_new = c.t1;
     c.h = t_new - c.t;
     c.h_abs = fabs(c.h);
     c.t_new = t_new;
 }
 __host__ __device__ inline void rk45_begin_step(Rk45Ctl& c) {
-    c.min_step = 10 * fabs(nextafter(c.t, INFINITY) - c.t);
+    c.min_step = 10 * fabs(nextafter(c.t, c.direction * INFINITY) - c.t);
     if (c.h_abs > c.max_step) c.h_abs = c.max_step;
     else if (c.h_abs < c.min_step) c.h_abs = c.min_step;
     c.step_rejected = 0;
@@ -75,7 +79,7 @@ __host__ __device__ inline void rk45_control(Rk45Ctl& c, int mode, double norm0,
             c.status.y_idx ^= 1;                    // y <- y_new
             c.k0 = 6 - c.k0;                        // K[0] <- K[6] (FSAL)
             c.status.accepted += 1;
-            if (c.t - c.t1 >= 0) c.status.state = RK_DONE;
+            if (c.direction * (c.t - c.t1) >= 0) c.status.state = RK_DONE;
             else rk45_begin_step(c);
         } else {
             // python's max(MIN_FACTOR, nan) is MIN_FACTOR, as fmax
@@ -133,7 +137,7 @@ __global__ void __launch_bounds__(256) k_rk45_stage(Rk45Params p, int stage) {
     const int yi = c.status.y_idx, k0 = c.k0;
     const float* y = p.ybuf + (size_t)yi * p.n;
     float* ynew = p.ybuf + (size_t)(yi ^ 1) * p.n;
-    const float h = stage < 0 ? (float)c.h0 : (float)c.h;
+    const float h = stage < 0 ? (float)(c.h0 * c.direction) : (float)c.h;       // c.h is signed already
     const float* ks[6];
 #pragma unroll
     for (int j = 0; j < 6; ++j) ks[j] = p.k + (size_t)rk_slot(k0, j) * p.n;
@@ -142,7 +146,7 @@ __global__ void __launch_bounds__(256) k_rk45_stage(Rk45Params p, int stage) {
         float x;
         if (stage == 0) {
             x = yv;
-        } else if (stage < 0) {                       // select_initial_step: y1 = y0 + h0 * f0
+        } else if (stage < 0) {                       // select_initial_step: y1 = y0 + h0 * direction * f0
             x = __fadd_rn(yv, __fmul_rn(h, ks[0][i]));
         } else {
             const float* a = stage < 6 ? RK_A[stage] : RK_B;
@@ -236,7 +240,8 @@ __global__ void __launch_bounds__(256) k_rk45_end(Rk45Params p, int mode) {
         c.arrive = 0;
         Stage* stages = const_cast<Stage*>(p.ctrl->stages);   // the stage table is written by this kernel and setup only
         if (mode == RK_END_NORM0) {
-            if (c.status.state == RK_RUNNING) rk45_write_eval(stages, c, 0, c.t + c.h0, 1);   // f1 = fun(t0 + h0, y1)
+            if (c.status.state == RK_RUNNING)             // f1 = fun(t0 + h0 * direction, y1)
+                rk45_write_eval(stages, c, 0, c.t + c.h0 * c.direction, 1);
         } else {
             rk45_write_attempt(stages, c);
         }
@@ -255,6 +260,7 @@ cudaError_t launch_rk45_end(const Rk45Params& p, int mode, cudaStream_t s) {
 //   k_rk45ps_setup  every controller <- the initial state; the stage entry of f0 (slot 0)
 //   k_rk45ps_stage  k_rk45_stage's arithmetic with the sample's own h (and h0), plus the sample's stage time
 //                   fl32(fl32(t + c_s*h) * t_scale) into tbuf for k_temb; a finished sample is frozen: xs = y at t1
+//                   (in either direction)
 //   k_rk45ps_end    one CTA per sample: k_rk45_end's norm over that sample's C*H*W elements, summed in the batched kernel's
 //                   partition (so B = 1 is bit-identical to the batched mode), the controller, and on accept the copies
 //                   K[6] -> K[0] and y_new -> y; the last CTA to arrive counts running / done / failed samples
@@ -264,7 +270,7 @@ __device__ void rk45ps_write_table(const Rk45PsParams& p, int mode) {
     Stage* stages = const_cast<Stage*>(p.ctrl->stages);
     Rk45Ctl c{};
     c.two_pass = p.two_pass; c.flags = p.flags;                                       // t_scaled is unused: k_temb reads tbuf
-    if (mode == RK_END_NORM0) rk45_write_eval(stages, c, 0, 0.0, 1);                   // f1 = fun(t0 + h0, y1)
+    if (mode == RK_END_NORM0) rk45_write_eval(stages, c, 0, 0.0, 1);                   // f1 = fun(t0 + h0 * direction, y1)
     else for (int e = 1; e <= 6; ++e) rk45_write_eval(stages, c, e - 1, 0.0, e);
 }
 
@@ -294,7 +300,7 @@ __global__ void __launch_bounds__(256) k_rk45ps_stage(Rk45PsParams p, int stage)
         double t;
         if (c.status.state != RK_RUNNING) t = c.t1;
         else if (stage == 0) t = c.t;
-        else if (stage < 0) t = c.t + c.h0;
+        else if (stage < 0) t = c.t + c.h0 * c.direction;
         else if (stage < 6) t = c.t + RK_C[stage] * c.h;
         else t = c.t + c.h;
         const float ts = __fmul_rn((float)t, c.t_scale);
@@ -312,8 +318,8 @@ __global__ void __launch_bounds__(256) k_rk45ps_stage(Rk45PsParams p, int stage)
         float x;
         if (stage == 0 || c.status.state != RK_RUNNING) {
             x = yv;
-        } else if (stage < 0) {                       // select_initial_step: y1 = y0 + h0 * f0
-            x = __fadd_rn(yv, __fmul_rn((float)c.h0, ks[0][i]));
+        } else if (stage < 0) {                       // select_initial_step: y1 = y0 + h0 * direction * f0
+            x = __fadd_rn(yv, __fmul_rn((float)(c.h0 * c.direction), ks[0][i]));
         } else {
             const float h = (float)c.h;
             const float* a = stage < 6 ? RK_A[stage] : RK_B;
@@ -380,13 +386,13 @@ __global__ void __launch_bounds__(256) k_rk45ps_end(Rk45PsParams p, int mode) {
             if (threadIdx.x == 0) { a0 += s0; a1 += s1; }
         }
         if (threadIdx.x == 0) {
-            Rk45Ctl c = *rc;
+            // the controller works on the record in place: a register copy of all of it spills under the 64-register cap
+            Rk45Ctl& c = *rc;
             const int acc0 = c.status.accepted;
             const double rn = sqrt((double)p.per);
             rk45_control(c, mode, sqrt(a0) / rn, sqrt(a1) / rn);           // norm(x) = ||x||_2 / sqrt(x.size)
             accepted = c.status.accepted != acc0;
             c.status.y_idx = 0; c.k0 = 0;             // fixed layout: the accepted step is copied below
-            *rc = c;
         }
         __syncthreads();
         if (accepted) {

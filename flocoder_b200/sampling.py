@@ -3,7 +3,8 @@
 Same function names, argument order, defaults and return values as the reference:
 ``warp_time``, ``rk4_step``, ``v_func_cfg``, ``generate_latents_rk4``, ``generate_latents``
 (+ the legacy ``euler_sampler``, ``legacy/train_sd_flowers.py:50-67``, and ``generate_latents_rk45``, the adaptive
-Dormand-Prince sampler the reference's ``method='rk45'`` dispatch names, with scipy's ``solve_ivp`` semantics).
+Dormand-Prince sampler the reference's ``method='rk45'`` dispatch names, with scipy's ``solve_ivp`` semantics), and
+``invert_latents``, which runs the same ODE backwards from data latents to noise.
 
 When ``model`` is a :class:`flocoder_b200.unet.Unet` the whole trajectory runs inside the
 C-ABI call ``flo_integrate``: stage times, the four U-Net evaluations per interval, the
@@ -28,7 +29,7 @@ from . import _lib
 from .unet import Unet
 
 __all__ = ["warp_time", "rk4_step", "v_func_cfg", "generate_latents_rk4", "generate_latents_rk45", "generate_latents",
-           "euler_sampler", "time_grid", "g2rgb", "decode_latents", "sampler"]
+           "invert_latents", "euler_sampler", "time_grid", "g2rgb", "decode_latents", "sampler"]
 
 
 def warp_time(t, dt=None, s=.5):
@@ -72,6 +73,18 @@ def time_grid(n_steps, start=0.0, device=None, dtype=torch.float32):
     return warp_time(torch.linspace(start, 1.0, n_steps, device=device, dtype=dtype))
 
 
+def _rk4_grid(n_steps, init_strength=None):
+    """``(warped fp32 CPU grid, interval count n_steps)`` of :func:`generate_latents_rk4`: ``linspace(0, 1, n_steps)``, or
+    with ``init_latents`` ``linspace(s, 1, max(1, int(n_steps * (1 - s))))`` for ``s = init_strength``
+    (``sampling.py:102-111``); :func:`invert_latents` runs the same grid backwards."""
+    if init_strength is None:
+        ts = torch.linspace(0, 1, n_steps, device="cpu", dtype=torch.float32)
+    else:
+        n_steps = max(1, int(n_steps * (1.0 - init_strength)))
+        ts = torch.linspace(init_strength, 1.0, n_steps, device="cpu", dtype=torch.float32)
+    return warp_time(ts), n_steps
+
+
 def _device_dtype(model):
     p = next(model.parameters())
     return p.device, p.dtype
@@ -92,13 +105,11 @@ def generate_latents_rk4(model, shape, n_steps=50, cond=None, cfg_strength=3.0, 
     device, dtype = _device_dtype(model)
     y = source if source is not None else torch.randn(shape, device=device, dtype=dtype)
     if init_latents is None:
-        ts = torch.linspace(0, 1, n_steps, device="cpu", dtype=torch.float32)
+        ts, n_steps = _rk4_grid(n_steps)
         jitter_strength = 0
     else:
         y = (1 - init_strength) * y + init_strength * init_latents
-        n_steps = max(1, int(n_steps * (1.0 - init_strength)))
-        ts = torch.linspace(init_strength, 1.0, n_steps, device="cpu", dtype=torch.float32)
-    ts = warp_time(ts)
+        ts, n_steps = _rk4_grid(n_steps, init_strength)
     nfe = n_steps * 4
 
     if not isinstance(model, Unet):
@@ -143,9 +154,10 @@ def _rk45_t0(init_latents, init_strength):
     return float(warp_time(torch.tensor(float(init_strength), dtype=torch.float32)))
 
 
-def _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps, what=""):
-    """The legacy composition for a foreign model: ``solve_ivp`` on the host over ``y.ravel()``, one model call per stage.
-    Returns ``(state at t1, nfev)``; ``what`` names the problem in the errors (e.g. ``"sample 3 "``)."""
+def _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps, what="", t1=1.0):
+    """The legacy composition for a foreign model: ``solve_ivp`` on the host over ``y.ravel()``, one model call per stage,
+    from ``t0`` to ``t1`` (either direction).  Returns ``(state at t1, nfev)``; ``what`` names the problem in the errors
+    (e.g. ``"sample 3 "``)."""
     import numpy as np
     from scipy.integrate import solve_ivp
     t_vec = torch.zeros(y.shape[0], device=y.device, dtype=y.dtype)
@@ -158,10 +170,19 @@ def _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps, wha
         x = torch.from_numpy(np.ascontiguousarray(yf)).to(device=y.device, dtype=y.dtype).reshape(y.shape)
         return v_func_cfg(model, cond, cfg_strength, t_vec, x, t).double().cpu().numpy().ravel()
 
-    sol = solve_ivp(fun, (t0, 1.0), y.double().cpu().numpy().ravel(), method="RK45", rtol=rtol, atol=atol)
+    sol = solve_ivp(fun, (t0, t1), y.double().cpu().numpy().ravel(), method="RK45", rtol=rtol, atol=atol)
     if sol.status != 0:
         raise RuntimeError(f"RK45 {what}failed at t={sol.t[-1]}: {sol.message}")
     return torch.from_numpy(sol.y[:, -1]).reshape(y.shape).to(device=y.device, dtype=y.dtype), int(sol.nfev)
+
+
+def _check_rk45_args(rtol, atol, max_steps):
+    if not rtol > 0:
+        raise ValueError(f"rtol must be > 0, got {rtol}")
+    if not atol >= 0:
+        raise ValueError(f"atol must be >= 0, got {atol}")
+    if int(max_steps) != max_steps or max_steps < 1:
+        raise ValueError(f"max_steps must be a positive integer, got {max_steps}")
 
 
 def _sample_cond(cond, i):
@@ -201,12 +222,7 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
     other callable keeps the legacy composition: ``solve_ivp`` on the host, calling the model once per stage (per sample,
     on ``x[i:i+1]`` with ``cond`` cut to that sample).  A step size below scipy's minimum step, or more than ``max_steps``
     attempts, raises RuntimeError (naming the sample with ``per_sample``)."""
-    if not rtol > 0:
-        raise ValueError(f"rtol must be > 0, got {rtol}")
-    if not atol >= 0:
-        raise ValueError(f"atol must be >= 0, got {atol}")
-    if int(max_steps) != max_steps or max_steps < 1:
-        raise ValueError(f"max_steps must be a positive integer, got {max_steps}")
+    _check_rk45_args(rtol, atol, max_steps)
     if init_latents is not None and not 0.0 <= init_strength < 1.0:
         raise ValueError(f"init_strength must be in [0, 1) with init_latents (t0 = warp_time(init_strength) < 1), "
                          f"got {init_strength}")
@@ -218,14 +234,7 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
 
     if not isinstance(model, Unet):
         # foreign model: the legacy composition -- scipy on the host, one model call per stage
-        if not per_sample:
-            return _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps)
-        outs, nfe = [], torch.zeros(y.shape[0], dtype=torch.int64)
-        for i in range(y.shape[0]):
-            out_i, nfe[i] = _solve_ivp_rk45(model, y[i:i + 1], _sample_cond(cond, i), cfg_strength, t0, rtol, atol,
-                                            max_steps, what=f"sample {i} ")
-            outs.append(out_i)
-        return torch.cat(outs, dim=0) if outs else y.clone(), nfe
+        return _rk45_foreign(model, y, cond, cfg_strength, t0, 1.0, rtol, atol, max_steps, per_sample)
 
     b, c, h, w = y.shape
     eng = model.engine(h, w)
@@ -242,6 +251,86 @@ def generate_latents_rk45(model, shape, cond=None, cfg_strength=3.0, source=None
         return state.to(out_dtype), counts[:, 0].clone()
     nfe, _, _ = eng.integrate_rk45(state, t0, 1.0, rtol=rtol, atol=atol, class_ids=cls, cfg_strength=cfg,
                                    max_steps=int(max_steps))
+    return state.to(out_dtype), nfe
+
+
+def _rk45_foreign(model, y, cond, cfg_strength, t0, t1, rtol, atol, max_steps, per_sample):
+    """:func:`_solve_ivp_rk45` on the whole batch, or with ``per_sample`` on every sample alone (``nfe`` a CPU int64 ``[B]``)."""
+    if not per_sample:
+        return _solve_ivp_rk45(model, y, cond, cfg_strength, t0, rtol, atol, max_steps, t1=t1)
+    outs, nfe = [], torch.zeros(y.shape[0], dtype=torch.int64)
+    for i in range(y.shape[0]):
+        out_i, nfe[i] = _solve_ivp_rk45(model, y[i:i + 1], _sample_cond(cond, i), cfg_strength, t0, rtol, atol,
+                                        max_steps, what=f"sample {i} ", t1=t1)
+        outs.append(out_i)
+    return torch.cat(outs, dim=0) if outs else y.clone(), nfe
+
+
+@torch.no_grad()
+def invert_latents(model, latents, n_steps=50, cond=None, cfg_strength=3.0, method="rk4", init_strength=0.0, rtol=1e-5,
+                   atol=1e-5, max_steps=10000, per_sample=False):
+    """Integrate data latents back towards noise: the sampling ODE run backwards from ``t = 1`` down to
+    ``t0 = warp_time(init_strength)`` (``t0 = 0`` by default, where the sampler draws its noise).  Returns
+    ``(state at t0, nfe)``.
+
+    Uses: encode a real latent (e.g. from ``codec.encode``) to the noise that generates it; measure a model's round-trip
+    error (generate, invert, compare); or invert partway, to ``t0 > 0``, and integrate forward again from there with other
+    conditioning -- the deterministic counterpart of the ``init_latents`` mixing of the forward samplers.
+
+    * ``method="rk4"``: classic RK4 over the grid :func:`generate_latents_rk4` uses with ``init_latents`` and this
+      ``init_strength`` (at 0 the plain sampling grid of ``n_steps`` points), traversed from 1 down to ``t0``: negative
+      ``dt`` in every step.  ``nfe`` is the true count ``4 * (len(grid) - 1)``, NOT the ``n_steps * 4`` the forward
+      sampler reports after the reference.
+    * ``method="rk45"``: adaptive Dormand-Prince with scipy's step-size control, ``solve_ivp(fun, (1, t0), y.ravel(),
+      method='RK45', rtol=rtol, atol=atol)``; ``nfe`` as :func:`generate_latents_rk45` reports it (an int, or with
+      ``per_sample=True`` a CPU int64 ``[B]`` of each sample's own ``solve_ivp`` count).  ``n_steps`` is then ignored.
+    * Classifier-free guidance and the inpainting mask (``cond``) apply to every evaluation, as in the forward samplers.
+
+    For a :class:`~flocoder_b200.unet.Unet` the whole inversion runs on the device (``flo_integrate`` over the descending
+    grid, ``flo_integrate_rk45_reverse`` / ``flo_integrate_rk45_per_sample_reverse``).  Any other callable gets the
+    generic composition: :func:`rk4_step` with negative ``dt``, or ``solve_ivp`` on the host (per sample with
+    ``per_sample``).  Argument errors raise ValueError before the model is called."""
+    if method not in ("rk4", "rk45"):
+        raise ValueError(f"method must be 'rk4' or 'rk45', got {method!r}")
+    _check_rk45_args(rtol, atol, max_steps)
+    if not 0.0 <= init_strength < 1.0:
+        raise ValueError(f"init_strength must be in [0, 1) (t0 = warp_time(init_strength) < 1), got {init_strength}")
+    if method == "rk4" and (int(n_steps) != n_steps or n_steps < 1):
+        raise ValueError(f"n_steps must be a positive integer, got {n_steps}")
+    y = latents
+    if method == "rk4":                               # RK45 ignores n_steps
+        grid = _rk4_grid(int(n_steps), init_strength)[0].flip(0)     # 1 -> warp_time(init_strength)
+    t0 = float(warp_time(torch.tensor(float(init_strength), dtype=torch.float32)))   # generate_latents_rk45's t0
+
+    if not isinstance(model, Unet):
+        if method == "rk45":
+            return _rk45_foreign(model, y, cond, cfg_strength, 1.0, t0, rtol, atol, max_steps, per_sample)
+        device, dtype = _device_dtype(model)
+        ts_d = grid.to(device=device, dtype=dtype)
+        t_vec = torch.zeros(y.shape[0], device=device, dtype=dtype)
+        v_func = partial(v_func_cfg, model, cond, cfg_strength, t_vec)
+        for i in range(len(ts_d) - 1):
+            y = rk4_step(v_func, y, ts_d[i], ts_d[i + 1] - ts_d[i])
+        return y, 4 * (len(grid) - 1)
+
+    b, c, h, w = y.shape
+    eng = model.engine(h, w)
+    out_dtype = y.dtype
+    state = y.to(device=eng.device, dtype=torch.float32).contiguous()
+    if state.data_ptr() == y.data_ptr():
+        state = state.clone()                      # never integrate in place on the caller's tensor
+    cls = _class_ids(model, cond)
+    cfg = float(cfg_strength) if (cls is not None and cfg_strength) else 0.0
+    eng.set_mask(model.mask_of(cond), b)
+    if method == "rk4":
+        if len(grid) >= 2:
+            eng.integrate(state, grid.tolist(), _lib.FLO_RK4, class_ids=cls, cfg_strength=cfg)
+        return state.to(out_dtype), 4 * (len(grid) - 1)
+    kw = dict(rtol=rtol, atol=atol, class_ids=cls, cfg_strength=cfg, max_steps=int(max_steps), reverse=True)
+    if per_sample:
+        counts = eng.integrate_rk45_per_sample(state, 1.0, t0, **kw)
+        return state.to(out_dtype), counts[:, 0].clone()
+    nfe, _, _ = eng.integrate_rk45(state, 1.0, t0, **kw)
     return state.to(out_dtype), nfe
 
 

@@ -55,7 +55,9 @@ typedef enum flo_dtype { FLO_F32 = 0, FLO_BF16 = 1, FLO_F16 = 2 } flo_dtype;
 
 /* Integrators.  Stage times are formed in fp32 exactly as the reference forms them on 0-d
  * tensors (sampling.py:44-47,117): dt = ts[i+1]-ts[i];  t, t+dt/2, t+dt;  time fed to the
- * U-Net is fl32(t)*t_scale (sampling.py:63). */
+ * U-Net is fl32(t)*t_scale (sampling.py:63).  The grid of FLO_RK4 / FLO_EULER_GRID need not be ascending: over a
+ * descending grid every dt is negative and the call integrates backwards in time (e.g. from data at t = 1 back to
+ * noise at t = 0, the inversion of a sampled trajectory). */
 typedef enum flo_method {
     FLO_RK4 = 0,          /* ts = time grid with n_ts points -> n_ts-1 classic RK4 intervals (sampling.py:37-48) */
     FLO_EULER_LEGACY = 1, /* ts = the n_ts evaluation times t_i, fixed dt: x += v(x, t_i*t_scale)*dt
@@ -158,6 +160,14 @@ FLO_API int flo_integrate_host(flo_unet_t* h, const float* x0, float* x1, const 
 FLO_API int flo_integrate_rk45(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol, float t_scale,
                        const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B, void* stream);
 
+/* flo_integrate_rk45 backwards in time: from t0 down to t1 < t0, with scipy's direction = -1 (signed steps h = -h_abs,
+ * the last step clipped to land on t1, min_step = 10*|nextafter(t, -inf) - t|, the trial point of select_initial_step at
+ * t0 - h0), as solve_ivp(fun, (t0, t1), ...) with t1 < t0 does.  Arguments, routes, counts and error codes are those of
+ * flo_integrate_rk45, except that it requires finite t1 < t0 (FLO_ERR_INVALID otherwise, no device needed). */
+FLO_API int flo_integrate_rk45_reverse(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol,
+                       float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps, int counts[3], int B,
+                       void* stream);
+
 /* Per-sample adaptive Dormand-Prince 5(4): every sample is its own solve_ivp(fun_i, (t0, t1), y0[i].ravel(), 'RK45') with
  * its own t, step size, accept / reject decisions and nfev; the error norm of sample i is the RMS over its C*H*W elements,
  * so a sample's result does not depend on the rest of its batch.  The batch still shares every U-Net evaluation: a sample
@@ -170,6 +180,12 @@ FLO_API int flo_integrate_rk45(flo_unet_t* h, float* y, double t0, double t1, do
 FLO_API int flo_integrate_rk45_per_sample(flo_unet_t* h, float* y, double t0, double t1, double rtol, double atol,
                        float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps, int32_t* counts, int B,
                        void* stream);
+
+/* flo_integrate_rk45_per_sample backwards in time, from t0 down to t1 < t0 (direction -1 as flo_integrate_rk45_reverse);
+ * a sample that reached t1 stays frozen there.  Requires finite t1 < t0; everything else as the forward call. */
+FLO_API int flo_integrate_rk45_per_sample_reverse(flo_unet_t* h, float* y, double t0, double t1, double rtol,
+                       double atol, float t_scale, const int64_t* class_ids, float cfg_strength, int max_steps,
+                       int32_t* counts, int B, void* stream);
 
 /* Number of function evaluations flo_integrate performs for (method, n_ts) -- the honest count,
  * not the reference's n_steps*4 over-count (sampling.py:121). */
@@ -193,8 +209,9 @@ FLO_API int flo_unet_profile_ops(flo_unet_t* h, int B, int reps, float* ms_per_o
 /* Debug: SM-clock timeline (clock64) of CTA 0 of fused stage `stage` from the last forward at batch B; needs the
  * environment variable FLO_TIMELINE=1 when the batch plan is created.  out128: HOST array of 128 int64. */
 FLO_API int flo_unet_read_timeline(flo_unet_t* h, int B, int stage, long long* out128);
-/* Last flo_integrate_rk45 or flo_integrate_rk45_per_sample call: out = {attempts (per-sample: of the whole batch), host wall ms over the attempts, device ms of the attempt graphs (CUDA
- * events)}; wall - device is the host round trip the per-attempt wait costs. */
+/* Last flo_integrate_rk45, flo_integrate_rk45_per_sample or _reverse call: out = {attempts (per-sample: of the whole batch),
+ * host wall ms over the attempts, device ms of the attempt graphs (CUDA events)}; wall - device is the host round trip the
+ * per-attempt wait costs. */
 FLO_API int flo_integrate_rk45_timing(flo_unet_t* h, double out[3]);
 /* Kernel launches issued per forward pass (graph nodes) and total since creation. */
 FLO_API int flo_unet_launches_per_forward(flo_unet_t* h, int B);

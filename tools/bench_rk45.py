@@ -6,6 +6,10 @@ Per configuration: samples/s of the adaptive solve (rtol = atol = 1e-5), its nfe
 CUDA events (flo_integrate_rk45_timing); and samples/s of RK4-50 (200 evaluations) from the same run.  Prints one JSON line
 per configuration, with the card name and power limit, and writes them to --out when given.
 
+Reverse rows: invert_latents of the RK4-50 result back to t = 0, with RK4-50 over the reversed grid (the same graphs as the
+forward RK4, so the same rate is expected) and with the adaptive solve (rtol = atol = 1e-5), alternating with the forward
+integrators.
+
 With --per-sample the per-sample RK45 (every sample its own step-size control) runs as a third arm, alternating with the
 other two on the same inputs.  Besides samples/s, attempts (the batch's, = the most any sample made) and the host gap it
 reports each sample's nfe (min / median / max) and the share of evaluated sample-forwards spent on samples that had already
@@ -71,10 +75,19 @@ def main():
             def rk4():
                 return sampling.generate_latents_rk4(m, (b, 4, 16, 16), n_steps=50, source=x0)   # the reference's RK4-50: 49 intervals
 
-            rk45(); rk4(); torch.cuda.synchronize()                  # warm-up: plans, graphs, modules
+            rk45(); x1, _ = rk4(); torch.cuda.synchronize()          # warm-up: plans, graphs, modules
+
+            def rk45_rev():
+                return sampling.invert_latents(m, x1, method="rk45")
+
+            def rk4_rev():
+                return sampling.invert_latents(m, x1, n_steps=50)
+
+            rk45_rev(); rk4_rev(); torch.cuda.synchronize()
             if args.per_sample:
                 rk45ps(); torch.cuda.synchronize()
             best45, best4, timing, nfe = float("inf"), float("inf"), None, 0
+            best45r, best4r, timing_r, nfe_r = float("inf"), float("inf"), None, 0
             best_ps, timing_ps, nfe_ps = float("inf"), None, None
             for _ in range(args.reps):                               # alternate the integrators
                 torch.cuda.synchronize()
@@ -88,6 +101,16 @@ def main():
                 rk4()
                 torch.cuda.synchronize()
                 best4 = min(best4, time.perf_counter() - t0)
+                t0 = time.perf_counter()
+                _, nfe_r = rk45_rev()
+                torch.cuda.synchronize()
+                dt45r = time.perf_counter() - t0
+                if dt45r < best45r:
+                    best45r, timing_r = dt45r, eng.rk45_timing()
+                t0 = time.perf_counter()
+                rk4_rev()
+                torch.cuda.synchronize()
+                best4r = min(best4r, time.perf_counter() - t0)
                 if args.per_sample:
                     t0 = time.perf_counter()
                     _, nfe_ps = rk45ps()
@@ -101,7 +124,12 @@ def main():
                             "ms_per_attempt_wall": wall_ms / attempts, "ms_per_attempt_graph": graph_ms / attempts,
                             "host_gap_ms_per_attempt": (wall_ms - graph_ms) / attempts,
                             "host_gap_share": (wall_ms - graph_ms) / wall_ms},
-                   "rk4_50": {"samples_per_s": b / best4, "nfe": 200}, "reps": args.reps, "timing": "best of reps, wall clock"}
+                   "rk4_50": {"samples_per_s": b / best4, "nfe": 200},
+                   "rk45_reverse": {"rtol": 1e-5, "atol": 1e-5, "samples_per_s": b / best45r, "nfe": nfe_r,
+                                    "attempts": timing_r[0], "ms_per_attempt_graph": timing_r[2] / timing_r[0],
+                                    "host_gap_share": (timing_r[1] - timing_r[2]) / timing_r[1]},
+                   "rk4_50_reverse": {"samples_per_s": b / best4r, "nfe": 196},
+                   "reps": args.reps, "timing": "best of reps, wall clock"}
             if args.per_sample:
                 a_ps, wall_ps, graph_ps = timing_ps
                 evaluated = b * (2 + 6 * a_ps)                       # sample-forwards the batch ran, finished samples included

@@ -31,7 +31,7 @@ EXPORTS = (
     "flo_unet_launch_count", "flo_unet_read_activation", "flo_selftest_umma", "flo_describe_plan",
     "flo_unet_op_info", "flo_unet_profile_ops", "flo_unet_read_timeline", "flo_unet_set_mask",
     "flo_integrate_rk45", "flo_integrate_rk45_timing", "flo_integrate_rk45_per_sample", "flo_integrate_rk45_reverse",
-    "flo_integrate_rk45_per_sample_reverse",
+    "flo_integrate_rk45_per_sample_reverse", "flo_unet_jvp", "flo_integrate_divergence",
 )
 
 
@@ -80,6 +80,9 @@ def lib() -> ctypes.CDLL:
                                                 ctypes.c_double, c_float, c_void_p, c_float, c_int, POINTER(ctypes.c_int32),
                                                 c_int, c_void_p]
     L.flo_integrate_rk45_per_sample_reverse.argtypes = L.flo_integrate_rk45_per_sample.argtypes
+    L.flo_unet_jvp.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p]
+    L.flo_integrate_divergence.argtypes = [c_void_p, c_void_p, POINTER(c_float), c_int, c_float, c_void_p, c_void_p, c_int,
+                                           c_void_p, c_int, c_void_p]
     L.flo_integrate_nfe.argtypes = [c_int, c_int]
     L.flo_unet_num_ops.argtypes = [c_void_p]
     L.flo_unet_op_name.argtypes = [c_void_p, c_int, c_char_p, c_int]
@@ -246,6 +249,36 @@ class Engine:
             check(self.L.flo_unet_forward(self.handle, x.data_ptr(), time.data_ptr(), cptr, v.data_ptr(), b,
                                           _stream_ptr(self.device)), "flo_unet_forward")
         return v
+
+    def jvp(self, x: torch.Tensor, time: torch.Tensor, class_ids: Optional[torch.Tensor], dx: torch.Tensor):
+        """``(v, dv)``: the velocity at ``x`` and the Jacobian-vector products ``dv[p] = J_x v . dx[p]`` (``flo_unet_jvp``,
+        exact forward mode on the fp32 path).  ``x`` [B,C,H,W], ``dx`` [P,B,C,H,W], fp32 contiguous on the engine's device."""
+        assert x.dtype == torch.float32 and x.is_contiguous() and x.device == self.device
+        assert dx.dtype == torch.float32 and dx.is_contiguous() and dx.device == self.device and dx.dim() == 5
+        b, n_tan = x.shape[0], dx.shape[0]
+        v, dv = torch.empty_like(x), torch.empty_like(dx)
+        keep, cptr = self._cls_ptr(class_ids, b)
+        with torch.cuda.device(self.device):
+            check(self.L.flo_unet_jvp(self.handle, x.data_ptr(), time.data_ptr(), cptr, dx.data_ptr(), n_tan, v.data_ptr(),
+                                      dv.data_ptr(), b, _stream_ptr(self.device)), "flo_unet_jvp")
+        return v, dv
+
+    def integrate_divergence(self, y: torch.Tensor, ts: Sequence[float], probes: torch.Tensor, t_scale: float = 999.0,
+                             class_ids=None) -> torch.Tensor:
+        """RK4 over ``ts`` in place on ``y`` with the Hutchinson divergence of the fixed ``probes`` [P,B,C,H,W] at every
+        stage (``flo_integrate_divergence``).  Returns ``div`` [B] fp64 on the device: sum over the intervals of
+        ``dt/6 (d1 + 2 d2 + 2 d3 + d4)``, ``d = mean_p probe_p . (J v probe_p)``."""
+        assert y.dtype == torch.float32 and y.is_contiguous() and y.device == self.device
+        assert probes.dtype == torch.float32 and probes.is_contiguous() and probes.device == self.device
+        b = y.shape[0]
+        ts_arr = (c_float * len(ts))(*[float(t) for t in ts])
+        div = torch.empty(b, dtype=torch.float64, device=self.device)
+        keep, cptr = self._cls_ptr(class_ids, b)
+        with torch.cuda.device(self.device):
+            check(self.L.flo_integrate_divergence(self.handle, y.data_ptr(), ts_arr, len(ts), float(t_scale), cptr,
+                                                  probes.data_ptr(), probes.shape[0], div.data_ptr(), b,
+                                                  _stream_ptr(self.device)), "flo_integrate_divergence")
+        return div
 
     def integrate(self, y: torch.Tensor, ts: Sequence[float], method: int, dt: float = 0.0,
                   t_scale: float = 999.0, class_ids=None, cfg_strength: float = 0.0,

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB = os.path.join(OUT_DIR, "libflocoder_b200.so")
-SOURCES = ["api.cu", "kernels_simt.cu", "conv_umma.cu", "fused.cu", "fused_attn.cu", "selftest.cu", "rk45.cu"]
+SOURCES = ["api.cu", "kernels_simt.cu", "conv_umma.cu", "fused.cu", "fused_attn.cu", "selftest.cu", "rk45.cu", "jvp.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",

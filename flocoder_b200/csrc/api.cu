@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <climits>
 #include <float.h>
 #include <map>
 #include <memory>
@@ -264,6 +265,9 @@ struct FStage {
 struct Handle;
 struct Plan {
     int B = 0;
+    int P = 0;                         // JVP plans: tangents per sample (the program runs over (1+P)*B rows, jvp.cu); 0: plain
+    float* prod = nullptr;             // JVP plans: [P,B,C,H,W] eps * dv of the current stage (ctrl.vtan of flo_integrate_divergence)
+    double* jdiv = nullptr;            // JVP plans: [B] running divergence integral
     uint8_t* arena = nullptr;          // activations
     size_t arena_bytes = 0;
     float *y = nullptr, *acc = nullptr, *xs = nullptr, *vcond = nullptr, *film_ps = nullptr;
@@ -335,7 +339,7 @@ struct Handle {
     // temb constants (offsets into blob_f32)
     size_t o_freqs, o_w1t, o_b1, o_w2t, o_b2, o_emb = NONE, o_wc1t = NONE, o_bc1 = NONE, o_wc3t = NONE, o_bc3 = NONE,
            o_wft, o_bf, o_init_w, o_init_b, o_final_w, o_final_b;
-    std::map<int, std::unique_ptr<Plan>> plans;
+    std::map<int64_t, std::unique_ptr<Plan>> plans;      // key: B for plain plans, plan_key(B, P) for JVP plans
     uint64_t use_ctr = 0;
     cudaStream_t last_stream = nullptr;     // a handle serves one stream at a time: calls on another stream first wait for this one
     bool has_last_stream = false;
@@ -829,13 +833,17 @@ static int launch_op(Handle& h, Plan& pl, int i, cudaStream_t st) {
     const Spec& s = h.spec;
     auto ptr = [&](int b) -> void* { return b >= 0 ? pl.buf_ptr[b] : nullptr; };
     auto f32c = [&](size_t off) -> const float* { return off == NONE ? nullptr : h.d_f32 + off; };
+    // a JVP plan runs every op over R rows: the linear ops as they are, without bias on the tangent rows; the nonlinear ones
+    // on their JVP kernels
+    const int R = pl.B * (1 + pl.P), bias_rows = pl.P ? pl.B : 0;
     cudaError_t e = cudaSuccess;
     switch (op.kind) {
         case OP_INIT: {
             InitConvParams p{};
             p.ctrl = pl.ctrl; p.w = f32c(h.o_init_w); p.bias = f32c(h.o_init_b);
             p.out_m = (float*)ptr(op.out_m); p.out_o = ptr(op.out_o);
-            p.B = pl.B; p.HW = s.H * s.W; p.cin = s.channels; p.dim = s.dim; p.o_is_bf16 = s.bf16;
+            p.n_bias_rows = bias_rows;
+            p.B = R; p.HW = s.H * s.W; p.cin = s.channels; p.dim = s.dim; p.o_is_bf16 = s.bf16;
             e = launch_init_conv(p, st);
         } break;
         case OP_CONV: {
@@ -851,7 +859,7 @@ static int launch_op(Handle& h, Plan& pl, int i, cudaStream_t st) {
                 p.in0 = ptr(op.in0); p.in1 = ptr(op.in1); p.ncb0 = op.ncb0; p.ncb1 = op.ncb1; p.in_is_bf16 = 0;
                 p.w = f32c(op.w_simt); p.bias = f32c(op.bias); p.res = (const float*)ptr(op.res);
                 p.out_m = (float*)ptr(op.out_m); p.out_o = nullptr; p.o_is_bf16 = 0;
-                p.B = pl.B; p.H = op.H; p.W = op.W; p.cout = op.cout; p.ksize = op.ksize;
+                p.B = R; p.n_bias_rows = bias_rows; p.H = op.H; p.W = op.W; p.cout = op.cout; p.ksize = op.ksize;
                 p.act_silu = op.act_silu; p.out_unshuf = ptr(op.out_un); p.out_up = ptr(op.out_up);
                 if (op.need_mode) { p.mask_mode = pl.mask_mode; p.need_mode = op.need_mode; p.bypass = (const float*)ptr(op.bypass); }
                 e = launch_conv_simt(p, st);
@@ -864,18 +872,19 @@ static int launch_op(Handle& h, Plan& pl, int i, cudaStream_t st) {
             p.out_m = (float*)ptr(op.out_m); p.out_o = ptr(op.out_o); p.out_unshuf = ptr(op.out_un); p.out_up = ptr(op.out_up);
             p.o_is_bf16 = s.bf16; p.B = pl.B; p.C = op.C; p.H = op.H; p.W = op.W; p.groups = op.groups;
             p.film_off = op.film_off; p.film_dim = h.film_dim; p.silu = op.silu;
-            e = launch_gn(p, st);
+            e = pl.P ? launch_gn_jvp(p, R, st) : launch_gn(p, st);
         } break;
         case OP_LINATTN:
         case OP_MIDATTN: {
             AttnParams p{};
             p.qkv = ptr(op.qkv); p.out = ptr(op.attn_out); p.is_bf16 = s.bf16; p.B = pl.B; p.n = op.n;
-            e = op.kind == OP_LINATTN ? launch_linattn(p, st) : launch_midattn(p, st);
+            if (pl.P) e = op.kind == OP_LINATTN ? launch_linattn_jvp(p, R, st) : launch_midattn_jvp(p, R, st);
+            else e = op.kind == OP_LINATTN ? launch_linattn(p, st) : launch_midattn(p, st);
         } break;
         case OP_FINAL: {
             FinalParams p{};
             p.ctrl = pl.ctrl; p.in = (const float*)ptr(op.gn_in); p.w = f32c(h.o_final_w); p.bias = f32c(h.o_final_b);
-            p.B = pl.B; p.HW = s.H * s.W; p.dim = s.dim; p.channels = s.channels;
+            p.B = R; p.n_bias_rows = bias_rows; p.HW = s.H * s.W; p.dim = s.dim; p.channels = s.channels;
             e = launch_final(p, st);
         } break;
     }
@@ -890,6 +899,23 @@ static int launch_unit(Handle& h, Plan& pl, int i, cudaStream_t st) {
     return h.spec.fused ? launch_fused_stage(h, pl, i, st) : launch_op(h, pl, i, st);
 }
 
+// One U-Net evaluation: the units of the program, and in a JVP plan the divergence reduction of the stage it evaluated (which
+// does nothing after a plain JVP).
+static int launch_program(Handle& h, Plan& pl, cudaStream_t st) {
+    for (int i = 0; i < n_units(h); ++i) {
+        int rc = launch_unit(h, pl, i, st);
+        if (rc) return rc;
+    }
+    if (pl.P) {
+        const Spec& s = h.spec;
+        cudaError_t e = launch_div_reduce(pl.ctrl, pl.jdiv, pl.B, pl.P, s.channels * s.H * s.W, st);
+        if (e != cudaSuccess) { set_error("launch of k_div_reduce failed: %s", cudaGetErrorString(e)); return FLO_ERR_CUDA; }
+    }
+    return FLO_OK;
+}
+
+static int64_t plan_key(int B, int P) { return P ? -((int64_t)B * ((int64_t)1 << 31) + P) : B; }
+
 static void destroy_plan(Plan&) {}          // resources are released by ~Plan when the owning unique_ptr goes away
 
 // One stream at a time per handle (the stage table, the control block and the workspaces are per handle / per plan):
@@ -900,10 +926,14 @@ static int enter_stream(Handle& h, cudaStream_t st) {
     return FLO_OK;
 }
 
-static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
-    auto it = h.plans.find(B);
+// P > 0: the JVP plan of B samples with P tangents each (fp32 path; the callers refuse the rest first)
+static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st, int P = 0) {
+    const int64_t key = plan_key(B, P);
+    auto it = h.plans.find(key);
     if (it != h.plans.end()) { it->second->last_use = ++h.use_ctr; *out = it->second.get(); return FLO_OK; }
     if (B <= 0) { set_error("batch size must be positive, got %d", B); return FLO_ERR_INVALID; }
+    if (P < 0 || (int64_t)B * (1 + P) > INT_MAX) { set_error("%d samples with %d tangents each are too many rows", B, P); return FLO_ERR_INVALID; }
+    const int R = B * (1 + P);
     if (h.plans.size() >= MAX_PLANS) {
         // ragged last batches / uneven shards would otherwise grow the cache without bound: drop the least recently used plan
         // (its workspace may still be in use by enqueued work: wait for the device first; plan creation is a slow path anyway)
@@ -915,15 +945,17 @@ static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
     }
     const Spec& s = h.spec;
     std::unique_ptr<Plan> pl(new Plan());
-    pl->B = B;
+    pl->B = B; pl->P = P;
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t state_bytes = al((size_t)B * s.channels * s.H * s.W * 4);
+    const size_t state_bytes = al((size_t)R * s.channels * s.H * s.W * 4);     // xs holds the tangent inputs in rows >= B
     const size_t film_bytes = al((size_t)B * h.film_dim * 4);
     const size_t cls_bytes = al((size_t)B * 8);
-    pl->arena_bytes = s.fused ? 256 : al(h.arena_ps * (size_t)B);     // layer-by-layer activations
+    pl->arena_bytes = s.fused ? 256 : al(h.arena_ps * (size_t)R);     // layer-by-layer activations
     const size_t farena_bytes = s.fused ? al(h.farena_ps * (size_t)B) : 0;   // stage-boundary tensors of the fused path
     const size_t flag_bytes = al((size_t)B * 4);
-    pl->total_bytes = pl->arena_bytes + farena_bytes + 4 * state_bytes + film_bytes + cls_bytes + flag_bytes + 512;
+    const size_t prod_bytes = P ? al((size_t)P * B * s.channels * s.H * s.W * 4) : 0, div_bytes = P ? al((size_t)B * 8) : 0;
+    pl->total_bytes = pl->arena_bytes + farena_bytes + 4 * state_bytes + film_bytes + cls_bytes + flag_bytes + 512 + prod_bytes +
+                      div_bytes;
     cudaError_t e = cudaMalloc((void**)&pl->base, pl->total_bytes);
     if (e != cudaSuccess) { set_error("cudaMalloc of %zu workspace bytes for B=%d failed: %s", pl->total_bytes, B, cudaGetErrorString(e)); cudaGetLastError(); return FLO_ERR_NOMEM; }
     uint8_t* q = pl->base;
@@ -937,9 +969,10 @@ static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
     pl->cls = (int64_t*)q; q += cls_bytes;
     pl->pair_flags = (int*)q; q += flag_bytes;
     pl->ctrl = (Ctrl*)q; q += 256;
-    pl->mask_mode = (int*)q;
+    pl->mask_mode = (int*)q; q += 256;
+    if (P) { pl->prod = (float*)q; q += prod_bytes; pl->jdiv = (double*)q; }
     pl->buf_ptr.resize(h.bufs.size());
-    for (size_t i = 0; i < h.bufs.size(); ++i) pl->buf_ptr[i] = s.fused ? nullptr : pl->arena + h.bufs[i].off_ps * (size_t)B;
+    for (size_t i = 0; i < h.bufs.size(); ++i) pl->buf_ptr[i] = s.fused ? nullptr : pl->arena + h.bufs[i].off_ps * (size_t)R;
     // halo / padding rows of the arena are never read as data, but keep everything finite.  On the CALLER's stream: the
     // first kernels of this plan are enqueued there right after this call, and a non-blocking stream is not ordered after
     // the legacy default stream.
@@ -968,8 +1001,7 @@ static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
     if (!(s.flags & FLO_FLAG_NO_GRAPH)) {
         cudaGraph_t g = nullptr;
         CUDA_TRY(cudaStreamBeginCapture(h.capture_stream, cudaStreamCaptureModeThreadLocal));
-        int rc = FLO_OK;
-        for (int i = 0; i < n_units(h) && rc == FLO_OK; ++i) rc = launch_unit(h, *pl, i, h.capture_stream);
+        int rc = launch_program(h, *pl, h.capture_stream);
         cudaError_t ce = cudaStreamEndCapture(h.capture_stream, &g);
         if (rc) { if (g) cudaGraphDestroy(g); destroy_plan(*pl); return rc; }
         if (ce != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(ce)); destroy_plan(*pl); return FLO_ERR_CUDA; }
@@ -989,7 +1021,7 @@ static int get_plan(Handle& h, int B, Plan** out, cudaStream_t st) {
     }
     pl->last_use = ++h.use_ctr;
     *out = pl.get();
-    h.plans[B] = std::move(pl);
+    h.plans[key] = std::move(pl);
     return FLO_OK;
 }
 
@@ -997,12 +1029,10 @@ static int run_forward(Handle& h, Plan& pl, cudaStream_t st) {
     if (pl.graph) {
         CUDA_TRY(cudaGraphLaunch(pl.graph, st));
     } else {
-        for (int i = 0; i < n_units(h); ++i) {
-            int rc = launch_unit(h, pl, i, st);
-            if (rc) return rc;
-        }
+        int rc = launch_program(h, pl, st);
+        if (rc) return rc;
     }
-    h.launches += (int64_t)n_units(h);
+    h.launches += (int64_t)n_units(h) + (pl.P ? 1 : 0);
     return FLO_OK;
 }
 
@@ -1144,6 +1174,7 @@ int flo_unet_create(flo_unet_t** out, const flo_unet_cfg* cfg, const void* const
         CUDA_TRY(conv_umma_configure());
     }
     CUDA_TRY(simt_configure());
+    if (!h->spec.bf16) CUDA_TRY(jvp_configure());
     if (h->spec.fused) CUDA_TRY(fused_configure());
     CUDA_TRY(cudaStreamCreateWithFlags(&h->capture_stream, cudaStreamNonBlocking));
     *out = reinterpret_cast<flo_unet_t*>(h.release());
@@ -1371,7 +1402,7 @@ static int integrate_impl(Handle* h, Plan* pl, float* y, const float* ts, int n_
     Ctrl c{};
     c.step = 0; c.done_ctr = 0; c.film_per_sample = 0; c.n_stages = n_pass; c.cfg = cfg_strength;
     c.y = y; c.acc = pl->acc; c.xs = pl->xs; c.vcond = pl->vcond; c.vout = nullptr; c.vtrace = v_trace;
-    c.film = h->d_film_u; c.stages = h->d_stages;
+    c.film = h->d_film_u; c.stages = h->d_stages; c.vtan = pl->prod;
     // film_per_sample is a per-pass property: encode it by pointing ctrl at the right table per pass
     for (int p = 0; p < n_pass; ++p) {
         if (pass_per_sample[p]) {
@@ -1437,6 +1468,90 @@ int flo_integrate_host(flo_unet_t* hh, const float* x0, float* x1, const float* 
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(x1, pl->y, bytes, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
+    return FLO_OK;
+}
+
+// ---- forward-mode JVPs (jvp.cu): the fp32 program over (1+P)*B rows
+// Refused before anything is allocated: the 16-bit paths have no tangent kernels, the inpainting net's mask-fusion convolutions
+// apply SiLU (not linear), and k_linattn_jvp holds at most LINATTN_JVP_MAX_N pixels.
+static int check_jvp(const Handle& h) {
+    const Spec& s = h.spec;
+    if (s.bf16) {
+        set_error("JVPs run on the fp32 path only (compute_dtype fp32): the 16-bit paths have no tangent kernels");
+        return FLO_ERR_UNSUPPORTED;
+    }
+    if (s.mask_cond) {
+        set_error("JVPs of the inpainting U-Net (mask_cond=1) are not supported: its mask-fusion convolutions apply SiLU");
+        return FLO_ERR_UNSUPPORTED;
+    }
+    for (const Op& op : h.ops)
+        if (op.kind == OP_LINATTN && op.n > LINATTN_JVP_MAX_N) {
+            set_error("linear attention '%s' at %dx%d (n=%d) has no JVP kernel: it holds at most %d pixels", op.name.c_str(), op.H,
+                      op.W, op.n, LINATTN_JVP_MAX_N);
+            return FLO_ERR_UNSUPPORTED;
+        }
+    return FLO_OK;
+}
+
+int flo_unet_jvp(flo_unet_t* hh, const float* x, const float* time, const int64_t* class_ids, const float* dx, int P,
+                 float* v, float* dv, int B, void* stream) {
+    if (P < 1 || P > JVP_MAX_TANGENTS) { set_error("need 1 to %d tangents, got P=%d", JVP_MAX_TANGENTS, P); return FLO_ERR_INVALID; }
+    if (B < 1) { set_error("batch size must be positive, got %d", B); return FLO_ERR_INVALID; }
+    Handle* h = reinterpret_cast<Handle*>(hh);
+    if (!h || !x || !time || !dx || !v || !dv) { set_error("NULL argument"); return FLO_ERR_INVALID; }
+    int rc = check_jvp(*h);
+    if (rc) return rc;
+    CUDA_TRY(cudaSetDevice(h->spec.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = enter_stream(*h, st);
+    if (rc) return rc;
+    Plan* pl = nullptr;
+    rc = get_plan(*h, B, &pl, st, P);
+    if (rc) return rc;
+    const Spec& s = h->spec;
+    const size_t n = (size_t)B * s.channels * s.H * s.W;
+    CUDA_TRY(cudaMemcpyAsync(pl->xs, x, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(pl->xs + n, dx, (size_t)P * n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    TembParams tp = temb_params(*h);
+    tp.t = time; tp.t_stride = 1; tp.cls = (s.n_classes > 0) ? class_ids : nullptr; tp.n_rows = B; tp.film = pl->film_ps;
+    CUDA_TRY(launch_temb(tp, st));
+    rc = ensure_stage_capacity(*h, 1);
+    if (rc) return rc;
+    Ctrl c{};
+    c.step = 0; c.done_ctr = 0; c.film_per_sample = 1; c.n_stages = 1; c.cfg = 0.f;
+    c.y = pl->y; c.acc = pl->acc; c.xs = pl->xs; c.vcond = pl->vcond; c.vout = v; c.vtrace = nullptr; c.vtan = dv;
+    c.film = pl->film_ps; c.stages = h->d_stages;
+    Stage s0{};
+    s0.kind = ST_PLAIN; s0.eval_idx = -1;
+    CUDA_TRY(launch_setup_ctrl(pl->ctrl, c, h->d_stages, &s0, st));
+    h->launches += 2;
+    return run_forward(*h, *pl, st);
+}
+
+int flo_integrate_divergence(flo_unet_t* hh, float* y, const float* ts, int n_ts, float t_scale, const int64_t* class_ids,
+                             const float* probes, int P, double* div, int B, void* stream) {
+    if (P < 1 || P > JVP_MAX_TANGENTS) { set_error("need 1 to %d probes, got P=%d", JVP_MAX_TANGENTS, P); return FLO_ERR_INVALID; }
+    if (n_ts < 2) { set_error("need at least two time points, got n_ts=%d", n_ts); return FLO_ERR_INVALID; }
+    if (B < 1) { set_error("batch size must be positive, got %d", B); return FLO_ERR_INVALID; }
+    Handle* h = reinterpret_cast<Handle*>(hh);
+    if (!h || !y || !ts || !probes || !div) { set_error("NULL argument"); return FLO_ERR_INVALID; }
+    int rc = check_jvp(*h);
+    if (rc) return rc;
+    CUDA_TRY(cudaSetDevice(h->spec.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = enter_stream(*h, st);
+    if (rc) return rc;
+    Plan* pl = nullptr;
+    rc = get_plan(*h, B, &pl, st, P);
+    if (rc) return rc;
+    const Spec& s = h->spec;
+    const size_t n = (size_t)B * s.channels * s.H * s.W;
+    // the probes sit in the tangent rows of the stage input for the whole trajectory: k_final writes only rows < B of xs
+    CUDA_TRY(cudaMemcpyAsync(pl->xs + n, probes, (size_t)P * n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(pl->jdiv, 0, (size_t)B * sizeof(double), st));
+    rc = integrate_impl(h, pl, y, ts, n_ts, FLO_RK4, 0.f, t_scale, class_ids, 0.f, nullptr, st);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(div, pl->jdiv, (size_t)B * sizeof(double), cudaMemcpyDeviceToDevice, st));
     return FLO_OK;
 }
 

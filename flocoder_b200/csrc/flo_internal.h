@@ -63,6 +63,7 @@ struct Ctrl {
     const float* film;    // FiLM table [rows][film_dim]
     const Stage* stages;
     int* pair_flags;      // SF_CFG_2B: [B] arrival counters of the sample halves (zero between passes)
+    float* vtan;          // JVP plans: [P,B,C,H,W] destination of the tangent rows of k_final: dv (ST_PLAIN), else eps * dv
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -75,6 +76,7 @@ struct InitConvParams {
     float* out_m;         // fp32 blocked or null
     void* out_o;          // operand blocked (bf16 or fp32) or null
     int B, HW, cin, dim, o_is_bf16;
+    int n_bias_rows;      // rows >= n_bias_rows (JVP tangent rows) get no bias; 0 = all rows
 };
 
 struct ConvSimtParams {
@@ -94,6 +96,7 @@ struct ConvSimtParams {
     const int* mask_mode;               // device flag (0 no mask, 1 mask all ones, 2 mask in use), or null
     int need_mode;                      // the op runs when *mask_mode >= need_mode ...
     const float* bypass;                // ... else out = bypass (fp32 blocked, same shape), or nothing is written if null
+    int n_bias_rows;                    // rows >= n_bias_rows (JVP tangent rows) get no bias; 0 = all rows
 };
 
 // cond['mask_cond'] [B,ch,H,W] (NCHW fp32) -> one blocked mask tensor per resolution level (bilinear,
@@ -155,6 +158,8 @@ struct FinalParams {
     const float* w;       // [channels][dim]
     const float* bias;
     int B, HW, dim, channels;
+    int n_bias_rows;      // JVP plans: the B samples (rows below get bias and the stage epilogue, rows at and above are
+                          // tangents written to ctrl.vtan); 0 = all B rows are samples
 };
 
 // tcgen05 convolution (conv_umma.cu)
@@ -203,6 +208,18 @@ cudaError_t launch_temb(const TembParams& p, cudaStream_t s);
 cudaError_t launch_final(const FinalParams& p, cudaStream_t s);
 cudaError_t launch_mask_prep(const MaskPrepParams& p, cudaStream_t s);   // p.mask == null: *mode = 0 only
 cudaError_t launch_gn_any(const GnParams& p, cudaStream_t s);            // any channels-per-group (fp32 path)
+
+// forward-mode JVP of the fp32 program (jvp.cu).  Rows of a JVP plan with P tangents at B samples: [0, B) primal, B*(1+p) + b
+// tangent p of sample b; R = (1+P)*B is the row stride of every blocked tensor, p.B the sample count.
+cudaError_t launch_gn_jvp(const GnParams& p, int R, cudaStream_t s);
+cudaError_t launch_linattn_jvp(const AttnParams& p, int R, cudaStream_t s);   // n <= 256
+cudaError_t launch_midattn_jvp(const AttnParams& p, int R, cudaStream_t s);   // n <= 64
+// div[b] += dt/6 * w * (1/P) sum_p sum_chw ctrl.vtan[p][b][chw] for the RK stage k_final just finished (w = 1, 2, 2, 1), in fp64
+// and a fixed order that depends on chw and P only
+cudaError_t launch_div_reduce(const Ctrl* ctrl, double* div, int B, int P, int chw, cudaStream_t s);
+constexpr int LINATTN_JVP_MAX_N = 256;
+constexpr int JVP_MAX_TANGENTS = 65534;      // the JVP kernels put 1 + P on gridDim.y (at most 65535)
+cudaError_t jvp_configure();
 
 // Host-side kernel choices of the layer-by-layer program: the launchers above follow them, and the planner refuses an op
 // they give no kernel for before anything is launched.

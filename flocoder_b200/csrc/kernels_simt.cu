@@ -111,6 +111,7 @@ __global__ void __launch_bounds__(128) k_init_conv(InitConvParams p) {
 #pragma unroll 4
     for (int ci = 0; ci < p.cin; ++ci) xin[ci] = x[((size_t)b * p.cin + ci) * p.HW + px];
     const int ncb = p.dim >> 3;
+    const bool bias = !p.n_bias_rows || b < p.n_bias_rows;
     for (int cb = 0; cb < ncb; ++cb) {
         float o[8];
 #pragma unroll
@@ -118,7 +119,7 @@ __global__ void __launch_bounds__(128) k_init_conv(InitConvParams p) {
             const int co = cb * 8 + j;
             float a = 0.f;
             for (int ci = 0; ci < p.cin; ++ci) a = fmaf(xin[ci], p.w[co * p.cin + ci], a);
-            o[j] = a + p.bias[co];
+            o[j] = bias ? a + p.bias[co] : a;
         }
         const size_t off = ((size_t)(cb * p.B + b) * p.HW + px) * 8;
         if (p.out_m) store8(p.out_m + off, o);
@@ -174,7 +175,7 @@ __global__ void __launch_bounds__(128) k_conv_simt(ConvSimtParams p) {
                 }
             }
         }
-        if (p.bias) {
+        if (p.bias && (!p.n_bias_rows || b < p.n_bias_rows)) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) acc[j] += p.bias[co0 + j];
         }
@@ -1234,17 +1235,22 @@ __global__ void __launch_bounds__(128) k_final(FinalParams p) {
     const int step = c->step;
     const Stage st = c->stages[step];
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    const int ns = p.n_bias_rows ? p.n_bias_rows : p.B;      // samples; rows from ns on are JVP tangents
     if (idx < p.B * p.HW) {
         const int b = idx / p.HW, px = idx % p.HW;
         float x[64];
         const int ncb = p.dim >> 3;
         for (int cb = 0; cb < ncb; ++cb) load8(p.in + ((size_t)(cb * p.B + b) * p.HW + px) * 8, x + cb * 8);
-        const size_t plane = (size_t)p.B * p.channels * p.HW;
+        const size_t plane = (size_t)ns * p.channels * p.HW;
         for (int co = 0; co < p.channels; ++co) {
             float k = 0.f;
             for (int i = 0; i < p.dim; ++i) k = fmaf(x[i], p.w[co * p.dim + i], k);
-            k += p.bias[co];
             const size_t o = ((size_t)b * p.channels + co) * p.HW + px;
+            if (b >= ns) {                          // tangent row: dv, or eps * dv with the probe eps held in xs
+                c->vtan[o - plane] = st.kind == ST_PLAIN ? k : k * c->xs[o];
+                continue;
+            }
+            k += p.bias[co];
             if (st.flags & SF_CFG_COMBINE) {        // v = v_nc + cfg*(v_c - v_nc)   (sampling.py:74)
                 const float vc = c->vcond[o];
                 k = __fadd_rn(k, __fmul_rn(c->cfg, __fsub_rn(vc, k)));

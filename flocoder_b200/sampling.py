@@ -4,7 +4,8 @@ Same function names, argument order, defaults and return values as the reference
 ``warp_time``, ``rk4_step``, ``v_func_cfg``, ``generate_latents_rk4``, ``generate_latents``
 (+ the legacy ``euler_sampler``, ``legacy/train_sd_flowers.py:50-67``, and ``generate_latents_rk45``, the adaptive
 Dormand-Prince sampler the reference's ``method='rk45'`` dispatch names, with scipy's ``solve_ivp`` semantics), and
-``invert_latents``, which runs the same ODE backwards from data latents to noise.
+``invert_latents``, which runs the same ODE backwards from data latents to noise, and ``log_likelihood``, the model's
+density of data latents by the instantaneous change of variables along that inversion.
 
 When ``model`` is a :class:`flocoder_b200.unet.Unet` the whole trajectory runs inside the
 C-ABI call ``flo_integrate``: stage times, the four U-Net evaluations per interval, the
@@ -20,6 +21,7 @@ behaviour for foreign models, not a fallback for ours.
 """
 from __future__ import annotations
 
+import math
 import random
 from functools import partial
 
@@ -29,7 +31,7 @@ from . import _lib
 from .unet import Unet
 
 __all__ = ["warp_time", "rk4_step", "v_func_cfg", "generate_latents_rk4", "generate_latents_rk45", "generate_latents",
-           "invert_latents", "euler_sampler", "time_grid", "g2rgb", "decode_latents", "sampler"]
+           "invert_latents", "log_likelihood", "euler_sampler", "time_grid", "g2rgb", "decode_latents", "sampler"]
 
 
 def warp_time(t, dt=None, s=.5):
@@ -332,6 +334,99 @@ def invert_latents(model, latents, n_steps=50, cond=None, cfg_strength=3.0, meth
         return state.to(out_dtype), counts[:, 0].clone()
     nfe, _, _ = eng.integrate_rk45(state, 1.0, t0, **kw)
     return state.to(out_dtype), nfe
+
+
+def _check_likelihood_args(latents, n_steps, n_probes, probes):
+    """The probe count ``P`` of :func:`log_likelihood`; ValueError for anything it cannot run."""
+    if latents.dim() != 4:
+        raise ValueError(f"latents must be [B,C,H,W], got {tuple(latents.shape)}")
+    if int(n_steps) != n_steps or n_steps < 2:
+        raise ValueError(f"n_steps must be an integer >= 2, got {n_steps}")
+    if n_probes is not None and (int(n_probes) != n_probes or n_probes < 1):
+        raise ValueError(f"n_probes must be a positive integer, got {n_probes}")
+    if probes is None:
+        return 1 if n_probes is None else int(n_probes)
+    if probes.dim() != 5 or tuple(probes.shape[1:]) != tuple(latents.shape) or probes.shape[0] < 1:
+        raise ValueError(f"probes must be [P,{','.join(map(str, latents.shape))}], got {tuple(probes.shape)}")
+    if n_probes is not None and int(n_probes) != probes.shape[0]:
+        raise ValueError(f"n_probes={n_probes} disagrees with the {probes.shape[0]} probes given")
+    return probes.shape[0]
+
+
+def _divergence_foreign(model, y, grid, cond, probes):
+    """The generic composition for any callable: RK4 over ``grid`` (the arithmetic of :func:`rk4_step`) with, at every
+    stage, ``d = mean_p probe_p . (J v probe_p)`` from ``torch.func.jvp`` of ``model(x, t * 999, cond)``, accumulated with
+    the same RK4 weights in fp64.  Returns ``(state at grid[-1], div)``."""
+    device, dtype = _device_dtype(model)
+    ts = grid.to(device=device, dtype=dtype)
+    t_vec = torch.zeros(y.shape[0], device=device, dtype=dtype)
+    div = torch.zeros(y.shape[0], dtype=torch.float64, device=device)
+    eps = probes.to(device=device, dtype=dtype)
+
+    def f(x, t):
+        t_vec.fill_(float(t))
+        fn = lambda xx: model(xx, t_vec * 999, cond=cond)            # noqa: E731
+        v, d = None, torch.zeros(y.shape[0], dtype=torch.float64, device=device)
+        for e in eps:
+            v, jv = torch.func.jvp(fn, (x,), (e,))
+            d += (e * jv).double().flatten(1).sum(1)
+        return v, d / eps.shape[0]
+
+    for i in range(len(ts) - 1):
+        t, dt = ts[i], ts[i + 1] - ts[i]
+        k1, d1 = f(y, t)
+        t_mid = t + dt / 2
+        k2, d2 = f(y + dt * k1 / 2, t_mid)
+        k3, d3 = f(y + dt * k2 / 2, t_mid)
+        k4, d4 = f(y + dt * k3, t + dt)
+        y = y + (dt / 6) * (k1 + 2 * k2 + 2 * k3 + k4)
+        div += float(dt) / 6 * (d1 + 2 * d2 + 2 * d3 + d4)
+    return y, div
+
+
+@torch.no_grad()
+def log_likelihood(model, latents, n_steps=50, cond=None, n_probes=None, probes=None, generator=None):
+    """Log-density ``log p(x)`` of data latents under the flow, in nats, by the instantaneous change of variables
+    ``d/dt log p_t(x_t) = -div v(x_t, t)``.  Returns ``(logp, noise, nfe)``.
+
+    * The latents are integrated back to ``noise`` with the RK4 of :func:`invert_latents` (``init_strength = 0``: the
+      warped sampling grid of ``n_steps >= 2`` points from 1 down to 0), and ``div v`` is integrated alongside with the same
+      RK4 weights, estimated at every stage by Hutchinson's ``mean_p probe_p . (J_x v probe_p)`` with exact Jacobian-vector
+      products.
+    * ``logp = -|noise|^2 / 2 - (D/2) ln(2 pi) + div`` per sample, ``D = C*H*W`` and ``div`` the integral from 1 to 0 of
+      ``div v dt``: fp64 ``[B]`` on ``latents.device``.  Bits per dimension are ``-logp / (D ln 2)``.
+    * Probes are fixed over the whole trajectory: ``probes`` ``[P,B,C,H,W]``, or ``n_probes`` (default 1) Rademacher +-1
+      draws from ``generator``.  Given both, ``n_probes`` must equal ``P``.  More probes lower the estimator's variance;
+      the ``D`` basis vectors scaled by ``sqrt(D)`` give the exact trace.
+    * ``cond={'class_cond': ids}`` gives ``log p(x | class)``; there is no guidance.  ``nfe = 4 * (n_steps - 1)`` velocity
+      evaluations, each carrying ``P`` Jacobian-vector products.
+
+    For a :class:`~flocoder_b200.unet.Unet` the whole trajectory runs on the device (``flo_integrate_divergence``: the fp32
+    path; NotImplementedError for 16-bit models, ``mask_cond`` and more than 256 pixels).  Any other callable gets the
+    generic composition with ``torch.func.jvp`` in the model's dtype.  Argument errors raise ValueError before the model is
+    called."""
+    n_tan = _check_likelihood_args(latents, n_steps, n_probes, probes)
+    b, c, h, w = latents.shape
+    if probes is None:
+        gen_device = generator.device if generator is not None else torch.device("cpu")
+        probes = torch.randint(0, 2, (n_tan, b, c, h, w), generator=generator, device=gen_device).mul_(2).sub_(1)
+    grid = _rk4_grid(int(n_steps), 0.0)[0].flip(0)                  # invert_latents' grid: 1 -> 0
+    nfe = 4 * (len(grid) - 1)
+    if not isinstance(model, Unet):
+        noise, div = _divergence_foreign(model, latents, grid, cond, probes)
+    else:
+        model.check_jvp_supported(h, w)
+        eng = model.engine(h, w)
+        state = latents.to(device=eng.device, dtype=torch.float32).contiguous()
+        if state.data_ptr() == latents.data_ptr():
+            state = state.clone()                      # never integrate in place on the caller's tensor
+        eps = probes.to(device=eng.device, dtype=torch.float32).contiguous()
+        div = eng.integrate_divergence(state, grid.tolist(), eps, class_ids=_class_ids(model, cond))
+        noise = state.to(latents.dtype)
+    z = noise.double().flatten(1)
+    d = c * h * w
+    logp = -0.5 * (z * z).sum(1) - 0.5 * d * math.log(2 * math.pi) + div.to(z.device)
+    return logp.to(latents.device), noise, nfe
 
 
 @torch.no_grad()

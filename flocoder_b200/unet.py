@@ -253,6 +253,41 @@ class Unet(nn.Module):
         v = eng.forward(x.to(torch.float32).contiguous(), time.contiguous(), cls)
         return v.to(x.dtype)
 
+    def check_jvp_supported(self, height: int, width: int) -> None:
+        """NotImplementedError unless :meth:`jvp` has kernels for this module at ``height x width``: the fp32 path only,
+        no inpainting mask branches (their convolutions apply SiLU), at most 256 pixels (linear attention)."""
+        if self._resolved_compute_dtype() != "fp32":
+            raise NotImplementedError(f"JVPs run on the fp32 path only, this model computes in {self._resolved_compute_dtype()}")
+        if self.mask_cond:
+            raise NotImplementedError("JVPs of the inpainting U-Net (mask_cond=True) are not supported")
+        if height * width > 256:
+            raise NotImplementedError(f"JVPs need at most 256 latent pixels (linear attention), got {height}x{width}")
+
+    @torch.no_grad()
+    def jvp(self, x: torch.Tensor, time: torch.Tensor, tangents: torch.Tensor, cond=None):
+        """``(v, dv)`` with ``v = forward(x, time, cond)`` and ``dv = J_x v . tangents``: exact forward-mode Jacobian-vector
+        products, several tangents per sample in one pass.  ``tangents`` is ``[B,C,H,W]`` or ``[P,B,C,H,W]``; ``dv`` has its
+        shape.  fp32 path only (NotImplementedError for 16-bit models, ``mask_cond`` and more than 256 pixels)."""
+        if x.dim() != 4 or x.shape[1] != self.channels:
+            raise ValueError(f"x must be [B,{self.channels},H,W], got {tuple(x.shape)}")
+        single = tangents.dim() == 4
+        dx = tangents.unsqueeze(0) if single else tangents
+        if dx.dim() != 5 or tuple(dx.shape[1:]) != tuple(x.shape) or dx.shape[0] < 1:
+            raise ValueError(f"tangents must be {tuple(x.shape)} or [P,{','.join(map(str, x.shape))}], got {tuple(tangents.shape)}")
+        cls = self.split_cond(cond)
+        if cls is not None and not self.class_condition:
+            cls = None
+        b, _, h, w = x.shape
+        self.check_jvp_supported(h, w)
+        eng = self.engine(h, w)
+        if x.device != eng.device or dx.device != eng.device:
+            raise RuntimeError(f"x / tangents are on {x.device} / {dx.device} but the model is on {eng.device}")
+        time = time.to(device=x.device, dtype=torch.float32).reshape(-1)
+        if time.numel() != b:
+            raise ValueError(f"time must have {b} elements, got {time.numel()}")
+        v, dv = eng.jvp(x.to(torch.float32).contiguous(), time.contiguous(), cls, dx.to(torch.float32).contiguous())
+        return v.to(x.dtype), (dv[0] if single else dv).to(tangents.dtype)
+
 
 def infer_unet_config(state_dict) -> dict:
     """U-Net constructor arguments recoverable from a reference ``state_dict`` (``generate_samples.py:91-101`` infers only

@@ -145,6 +145,23 @@ FLO_API int flo_integrate_host(flo_unet_t* h, const float* x0, float* x1, const 
                        float dt, float t_scale, const int64_t* class_ids, float cfg_strength, int B,
                        void* stream);
 
+/* v = Unet.forward(x, time, cond) and dv[p] = J_x v · dx[p] for P tangents: exact forward mode, fp32 handles only.
+ * x, v: [B,C,H,W]; dx, dv: [P,B,C,H,W] fp32 device; time, class_ids as flo_unet_forward.  Asynchronous.
+ * FLO_ERR_INVALID for P outside 1..65534, B < 1 or a NULL pointer (checked first, no device needed);
+ * FLO_ERR_UNSUPPORTED, before anything is allocated, for 16-bit handles, mask_cond handles and linear attention over
+ * more than 256 pixels. */
+FLO_API int flo_unet_jvp(flo_unet_t* h, const float* x, const float* time, const int64_t* class_ids,
+                         const float* dx, int P, float* v, float* dv, int B, void* stream);
+
+/* FLO_RK4 over ts (either direction, stage times exactly as flo_integrate forms them) with, at every stage input, the
+ * Hutchinson divergence of the fixed probes [P,B,C,H,W]; div: [B] fp64 device, out = Σ_intervals dt/6·(d1+2d2+2d3+d4)
+ * with d = (1/P) Σ_p probe_p · (J_x v · probe_p), summed in fp64 in an order that depends on C*H*W and P only.
+ * y as flo_integrate.  Whole trajectory on the device, no host synchronisation, one graph replay per evaluation.
+ * FLO_ERR_INVALID for P outside 1..65534, n_ts < 2, B < 1 or a NULL y / ts / probes / div (checked first, no device
+ * needed); FLO_ERR_UNSUPPORTED as flo_unet_jvp. */
+FLO_API int flo_integrate_divergence(flo_unet_t* h, float* y, const float* ts, int n_ts, float t_scale,
+                         const int64_t* class_ids, const float* probes, int P, double* div, int B, void* stream);
+
 /* Adaptive Dormand-Prince 5(4) from t0 to t1 with scipy.integrate.solve_ivp(method='RK45')'s step-size control
  * (scipy/integrate/_ivp/rk.py, common.py): select_initial_step, SAFETY 0.9, factors in [0.2, 10], exponent -1/5,
  * min_step = 10*|nextafter(t, inf) - t|, the last step clipped to land on t1, max_step = inf.
